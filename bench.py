@@ -3,6 +3,7 @@
 bench.py — output Mpix/s of IMP's fused decoded-pixel chain on B200 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference] [--extras all|none|cfg1,cfg5]
+                  [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic frames. The headline workload is BASELINE.json
 configs[1] (cfg2): 256 requests of a 3840x2160 BGRA frame -> crop 3600x2025 -> INTER_AREA to 800x450 -> 256x64 watermark
@@ -292,10 +293,38 @@ def lpt_assign(costs, n):
     return owner
 
 
-def measure(cx: Ctx, name: str, steps: int, warmup: int, e2e_steps: int, shard: str = "weak", seed_off: int = 0):
+DUMP_BYTES = 60 << 20          # --dump-outputs: float32 pixels written in all, under 64 MB with the .npy headers
+
+
+def dump_sample(n_jobs: int, job_shape, budget: int = DUMP_BYTES):
+    """The frames --dump-outputs writes: [(job, rows)] in submission order. Jobs are taken in a fixed seeded permutation while
+    their float32 frames fit the budget; rows is None for a whole frame. When the first job's frame alone is over the budget,
+    it is the only one, cut to a fixed seeded sample of its rows (sorted). The same workload always gives the same sample."""
+    rng = np.random.default_rng(2024)
+    pick, total = [], 0
+    for j in rng.permutation(n_jobs).tolist():
+        h, w, c = job_shape(j)
+        if total + 4 * h * w * c <= budget:
+            pick.append((j, None)); total += 4 * h * w * c
+            continue
+        if not pick:
+            pick.append((j, np.sort(rng.choice(h, max(1, budget // (4 * w * c)), replace=False))))
+        break
+    return sorted(pick, key=lambda p: p[0])
+
+
+def write_dump(path: str, name: str, frames) -> None:
+    """frames: [(job index, HxWxC uint8 array)] -> <path>/<name>_job<index>.npy as float32 (exact for bytes)."""
+    os.makedirs(path, exist_ok=True)
+    for j, f in frames:
+        np.save(os.path.join(path, f"{name}_job{j:05d}.npy"), f.astype(np.float32))
+
+
+def measure(cx: Ctx, name: str, steps: int, warmup: int, e2e_steps: int, shard: str = "weak", seed_off: int = 0, dump: bool = False):
     """Device-resident batch (CUDA events) + end-to-end host batch of one workload on this rank.
     shard: "weak" = every rank runs the whole workload on its own frames; "mod" / "lpt" = the workload's jobs are split
-    over the ranks (strong scaling): job i on GPU i mod N, or largest-first by algorithmic bytes."""
+    over the ranks (strong scaling): job i on GPU i mod N, or largest-first by algorithmic bytes.
+    dump: keep a sample of the frames the last timed step wrote (res["_dump"], see dump_sample) for --dump-outputs."""
     torch, api, L, dev = cx.torch, cx.api, cx.L, cx.dev
     wl = workload(name, cx.a.scale)
     cfg = api.Config(**wl["cfg"])
@@ -325,12 +354,14 @@ def measure(cx: Ctx, name: str, steps: int, warmup: int, e2e_steps: int, shard: 
     batch = api.Batch(L)
     used = {si: 0 for si in per_shape}
     out_pix = 0
+    slots = []
     for j in mine:
         si = order[j]
         p = plans[si]
         k = used[si]; used[si] += 1
         s = srcs[si]
         batch.add(p, s[k % s.shape[0]].data_ptr(), s.shape[2], dsts[si][k].data_ptr(), dsts[si].shape[2])
+        slots.append((j, si, k))
         out_pix += p.out_w * p.out_h
     torch.cuda.synchronize()
     torch.cuda.set_stream(cx.tstream)
@@ -368,6 +399,19 @@ def measure(cx: Ctx, name: str, steps: int, warmup: int, e2e_steps: int, shard: 
                        "frac_of_nominal_8000": achieved / 8000.0,      # SURVEY §8d asks for both denominators
                        "peak_source": cx.peak_src, "algorithmic_bytes_per_step": int(algo_bytes), "kernel_launches_per_step": batch.launches_per_run,
                        "ms_per_launch_group": float(np.mean(step_ms)), "ms_min": float(np.min(step_ms)), "rank": cx.rank}
+    if dump:
+        def frame(i, rows):
+            j, si, k = slots[i]
+            p = plans[si]
+            t = dsts[si][k, :, :p.out_w * p.out_c]
+            if rows is not None:
+                t = t[torch.as_tensor(rows, device=dev)]
+            return j, t.reshape(-1, p.out_w, p.out_c).cpu().numpy()
+
+        def job_shape(i):
+            p = plans[slots[i][1]]
+            return p.out_h, p.out_w, p.out_c
+        res["_dump"] = [frame(i, rows) for i, rows in dump_sample(len(slots), job_shape)]
     batch.close()
     del srcs, dsts
     torch.cuda.empty_cache()
@@ -581,7 +625,12 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--extras", default="all", help="all | none | comma list of cfg1,cfg3,cfg3nn,cfg4,cfg5 (other BASELINE configs measured in the same run)")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of the frames the headline's last "
+                    "step produced as DIR/<config>_job<index>.npy (float32 HxWxC; a seeded sample of the rows of a frame too large on its "
+                    "own, the rows bench.dump_sample picks, in order; under 64 MB in all; rank 0), to compare two builds")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     wl = workload(a.config, a.scale)
@@ -615,8 +664,10 @@ def main():
     stop, samples = threading.Event(), []
     th = threading.Thread(target=sample_clocks, args=(stop, samples), daemon=True)
     th.start()
-    head = measure(cx, a.config, a.steps, a.warmup, a.e2e_steps, shard="weak")
+    head = measure(cx, a.config, a.steps, a.warmup, a.e2e_steps, shard="weak", dump=bool(a.dump_outputs))
     stop.set(); th.join(timeout=2)            # clocks were sampled across the device-timed and the end-to-end regions of the headline
+    if a.dump_outputs and rank == 0:
+        write_dump(a.dump_outputs, a.config, head.pop("_dump"))
     ceiling = h2d_ceiling(cx)
     lat = {}
     if rank == 0:

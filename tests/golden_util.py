@@ -1,4 +1,5 @@
 """Loads tests/golden/golden_v1.npz (made by tests/golden/make_golden.py from the compiled reference + cv2)."""
+import hashlib
 import json
 import os
 from urllib.parse import unquote
@@ -53,6 +54,56 @@ def load_io():
     packs = [dict(img=z[f"p{pi}_in"], fi24=z[f"p{pi}_fi24"], fi32=z[f"p{pi}_fi32"]) for pi in range(len(meta["packs"]))]
     jobs = [dict(j, out=z[f"j{ji}_out"]) for ji, j in enumerate(meta["jobs"])]
     return dict(gifs=gifs, packs=packs, jobs=jobs)
+
+
+CV2_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_cv2_v1.json")
+
+
+def digest(a):
+    """SHA-256 of an array's shape and bytes: what golden_cv2_v1.json stores instead of the arrays themselves."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(repr(a.shape).encode() + a.tobytes()).hexdigest()
+
+
+def load_cv2():
+    """tests/golden/golden_cv2_v1.json (made by tests/golden/make_golden_cv2.py with cv2 4.13, IPP off):
+    {case key: {"in": digest of the input, "out": digest of cv2's result}} for the cases below."""
+    with open(CV2_PATH) as f:
+        return json.load(f)["cases"]
+
+
+def _rnd(seed, h, w, c):
+    return np.random.default_rng(seed).integers(0, 256, (h, w, c), dtype=np.uint8)
+
+
+def cv2_resize_cases():
+    """Random sizes, channel counts and the four interpolations (0 NN, 1 LINEAR, 2 CUBIC, 3 AREA shrink only):
+    yields (key, img, dw, dh, mode)."""
+    rng = np.random.default_rng(42)
+    for it in range(120):
+        sw, sh = int(rng.integers(1, 90)), int(rng.integers(1, 70))
+        dw, dh = int(rng.integers(1, 120)), int(rng.integers(1, 100))
+        c = int(rng.choice([1, 3, 4]))
+        img = rng.integers(0, 256, (sh, sw, c), dtype=np.uint8)
+        for mode in (0, 1, 2, 3):
+            if mode == 3 and (dw > sw or dh > sh):
+                continue
+            yield f"resize/{it}/{mode}", img, dw, dh, mode
+
+
+GAUSS_SIGMAS = [0.3, 0.5, 0.8, 1.0, 1.5, 2.0, 2.3, 3.0, 4.7, 6.0, 12.0]
+
+
+def cv2_gaussian_cases():
+    """cvSmooth's Gaussian (BORDER_REPLICATE, sigma as the reference's float): yields (key, img, sigma)."""
+    for sigma in GAUSS_SIGMAS:
+        for (w, h, c) in [(64, 48, 3), (33, 17, 4), (5, 4, 3), (1, 1, 4)]:
+            yield f"gaussian/{sigma}/{w}x{h}x{c}", _rnd(int(sigma * 100) + w, h, w, c), sigma
+
+
+def cv2_orient_image():
+    """The input of the flip / transpose / rotate cases: keys flip/0, flip/1, flip/-1, transpose, rotate90."""
+    return _rnd(3, 13, 9, 3)
 
 
 def fi_page(frame):

@@ -1,6 +1,6 @@
 """CPU tests of the oracle: the C restatement against (1) SURVEY App. B known answers, (2) the golden
-vectors generated from the compiled reference + cv2, (3) live, the compiled reference and cv2 when they
-are present (this container)."""
+vectors generated from the compiled reference + cv2 and the stored cv2 4.13 results (tests/golden/), (3) live,
+the compiled reference (oracle/_ref, built from the reference's sources by oracle/Makefile) when it is present."""
 import numpy as np
 import pytest
 
@@ -137,42 +137,36 @@ def test_restatement_vs_compiled_reference_filters(orc, c):
         assert orc.Ref.filter(img, rq, False)[0] == orc.apply_filter(img, rq, False)[0] == 52
 
 
+def _same_as_cv2(want, key, img, got):
+    """got equals what cv2 4.13 returned for this input (tests/golden/golden_cv2_v1.json)."""
+    assert G.digest(img) == want[key]["in"], (key, "the seeded input is not the one the golden results were made from")
+    assert G.digest(got) == want[key]["out"], (key, img.shape, got.shape, "differs from cv2 4.13: compare pixel by pixel with cv2 "
+                                               "on the same case (tests/golden/make_golden_cv2.py) to see where")
+
+
 def test_restatement_vs_cv2_resize_fuzz(orc):
-    if not _have_cv2():
-        pytest.skip("cv2 not available")
-    import cv2
-    cv2.ipp.setUseIPP(False)
+    want = G.load_cv2()
     o = orc.orc()
-    rng = np.random.default_rng(42)
-    for it in range(120):
-        sw, sh = int(rng.integers(1, 90)), int(rng.integers(1, 70))
-        dw, dh = int(rng.integers(1, 120)), int(rng.integers(1, 100))
-        c = int(rng.choice([1, 3, 4]))
-        img = rng.integers(0, 256, (sh, sw, c), dtype=np.uint8)
-        for mode in (0, 1, 2, 3):
-            if mode == 3 and (dw > sw or dh > sh):
-                continue
-            ref = cv2.resize(img, (dw, dh), interpolation=mode).reshape(dh, dw, c)
-            got = o.resize(img, dw, dh, mode)
-            assert np.array_equal(ref, got), (sw, sh, dw, dh, c, mode)
+    keys = set()
+    for key, img, dw, dh, mode in G.cv2_resize_cases():
+        _same_as_cv2(want, key, img, o.resize(img, dw, dh, mode))
+        keys.add(key)
+    assert keys == {k for k in want if k.startswith("resize/")}
 
 
 def test_restatement_vs_cv2_gaussian_and_index_maps(orc):
-    if not _have_cv2():
-        pytest.skip("cv2 not available")
-    import cv2
-    cv2.ipp.setUseIPP(False)
+    want = G.load_cv2()
     o = orc.orc()
-    for sigma in [0.3, 0.5, 0.8, 1.0, 1.5, 2.0, 2.3, 3.0, 4.7, 6.0, 12.0]:
-        for (w, h, c) in [(64, 48, 3), (33, 17, 4), (5, 4, 3), (1, 1, 4)]:
-            img = rnd_image(int(sigma * 100) + w, h, w, c)
-            ref = cv2.GaussianBlur(img, (0, 0), float(np.float32(sigma)), sigmaY=0, borderType=cv2.BORDER_REPLICATE).reshape(h, w, c)
-            assert np.array_equal(ref, o.gaussian(img, sigma)), (sigma, w, h, c)
-    img = rnd_image(3, 13, 9, 3)
+    keys = set()
+    for key, img, sigma in G.cv2_gaussian_cases():
+        _same_as_cv2(want, key, img, o.gaussian(img, sigma))
+        keys.add(key)
+    assert keys == {k for k in want if k.startswith("gaussian/")}
+    img = G.cv2_orient_image()
     for m in (0, 1, -1):
-        assert np.array_equal(o.flip(img, m), cv2.flip(img, m))
-    assert np.array_equal(o.transpose(img), cv2.transpose(img))
-    assert np.array_equal(o.flip(o.transpose(img), 1), cv2.rotate(img, cv2.ROTATE_90_CLOCKWISE))
+        _same_as_cv2(want, f"flip/{m}", img, o.flip(img, m))
+    _same_as_cv2(want, "transpose", img, o.transpose(img))
+    _same_as_cv2(want, "rotate90", img, o.flip(o.transpose(img), 1))
 
 
 QUERIES = ["resize=30,20", "crop=1,1", "crop=16,9,l,t", "crop=40px,20px,6px,0px", "crop=40px,20", "crop=5000px,10px", "crop=0px,10px",

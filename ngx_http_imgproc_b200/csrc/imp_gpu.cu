@@ -21,6 +21,7 @@
 #include <mutex>
 #include <new>
 #include <thread>
+#include <tuple>
 #include <unordered_map>
 
 namespace {
@@ -85,12 +86,13 @@ struct imp_gpu_batch {
     cudaEvent_t up_ev = nullptr; bool up_pending = false;
     bool table_needed = false;                   // false when every launch group holds one job (passed by value)
     Buf scratch;
-    struct Step { bool generic_blur; ImpLaunchGroup g; int job; ImpPass hdr; size_t scratch_off; int smem; };
+    struct Step { ImpLaunchGroup g; ImpPass hdr; uint16_t* plane; };     // hdr, plane: BlurGeneric only (its u16 plane)
     std::vector<Step> steps;
     unsigned long long algo_bytes = 0;
     int launches = 0;
     // tensor maps are encoded once per (buffer, geometry): the staging lanes present the same addresses again and again
-    std::unordered_map<ImpTmKey, ImpTmap, ImpTmKeyHash> tmaps;
+    using TmCache = std::unordered_map<ImpTmKey, ImpTmap, ImpTmKeyHash>;
+    TmCache tmaps;
 };
 
 namespace {
@@ -307,54 +309,8 @@ void cache_clear() {
     parked_release(true);
 }
 
-int ops_smem(const ImpPass& h) { return std::max(16, h.nops * (int)sizeof(ImpOp) + h.lut_bytes); }
-
 int pass_pitch(const ImpHostPass& hp) { return align16(hp.out_w * hp.out_c); }
 
-// Scratch a plan needs on the device: intermediates between passes + the u16 plane of each generic blur.
-// off[k] = offset of pass k's output (non-final passes); blur_off[k] = offset of pass k's u16 plane.
-int pick_variant(const ImpPass& h, const ImpJob& j);
-int variant_param(const ImpPass& h, int variant);
-int variant_smem(const ImpPass& h, int variant, int param);
-constexpr int kTileSmemLimit = 200 * 1024;     // cudaFuncAttributeMaxDynamicSharedMemorySize of every tile kernel (imp_kernels.cu)
-
-// `src`/`sp`: the job's source (null = one of the library's own aligned buffers). The u16 plane is only reserved for a
-// blur that cannot take the fused tile kernel (radius > 12, or a pass-0 source whose rows are not 16-byte addressable).
-size_t plan_scratch_layout(const imp_gpu_plan* p, size_t base, std::vector<size_t>& off, std::vector<size_t>& blur_off,
-                           const uint8_t* src = nullptr, int sp = 0) {
-    size_t cur = base;
-    auto take = [&](size_t bytes) { size_t o = cur; cur += (bytes + 255) & ~size_t(255); return o; };
-    off.assign(p->passes.size(), 0); blur_off.assign(p->passes.size(), 0);
-    for (size_t k = 0; k < p->passes.size(); k++) {
-        const ImpHostPass& hp = p->passes[k];
-        if (k + 1 < p->passes.size()) off[k] = take((size_t)pass_pitch(hp) * hp.out_h);
-        if (hp.hdr.kind == IMP_G_BLUR) {
-            ImpJob probe{};
-            probe.src = (k == 0 && src) ? src : reinterpret_cast<const uint8_t*>(uintptr_t(256));
-            probe.src_pitch = (k == 0 && src) ? sp : 16;
-            if (pick_variant(hp.hdr, probe) == 0) blur_off[k] = take((size_t)hp.hdr.sw * hp.hdr.sh * hp.hdr.sc * 2);
-        }
-    }
-    return cur;
-}
-
-ImpJob make_job(const imp_gpu_plan* p, int d, size_t k, const uint8_t* src, int sp, uint8_t* dst, int dp,
-                uint8_t* scratch, const std::vector<size_t>& off) {
-    const imp_gpu_plan::Dev& pd = p->dev[d];
-    ImpJob j{};
-    j.pass = pd.pass_blobs[k];
-    if (p->wm) { j.wm = p->wm->dev[d].d; j.wm_pitch = p->wm->dev[d].pitch; j.wm_c = p->wm->c; }
-    if (k == 0) { j.src = src; j.src_pitch = sp; }
-    else { j.src = scratch + off[k - 1]; j.src_pitch = pass_pitch(p->passes[k - 1]); }
-    if (k + 1 == p->passes.size()) { j.dst = dst; j.dst_pitch = dp; }
-    else { j.dst = scratch + off[k]; j.dst_pitch = pass_pitch(p->passes[k]); }
-    return j;
-}
-
-int pass_tiles(const ImpPass& h) { return ((h.bw + 31) / 32) * ((h.bh + 31) / 32); }      // imp_pass_kernel: 32 x (8 x PASS_PPT) pixels per CTA
-
-// Tile (shared-memory, TMA-staged) variant: needs 16-byte addressable source rows — pitch % 16 == 0 and
-// either the image rows or the window rows start 16-byte aligned (imp_tiles.cuh) — and a footprint that fits.
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda link dependency).
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -372,7 +328,7 @@ EncodeTiledFn encode_tiled() {
 // Tensor map over the job's source window for the strip kernels: 8-byte elements, rows = window rows, origin =
 // the window's first byte aligned down to 16; box = tile_rs bytes x tile_rows rows. Out-of-range box parts are
 // zero-filled by the TMA unit, so edge tiles never touch memory outside the window's rows.
-int encode_job_tmap(const ImpPass& h, ImpJob& j, std::unordered_map<ImpTmKey, ImpTmap, ImpTmKeyHash>* cache = nullptr) {
+int encode_job_tmap(const ImpPass& h, ImpJob& j, imp_gpu_batch::TmCache* cache) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail_msg("cuTensorMapEncodeTiled is unavailable in this driver");
     const uintptr_t win = (uintptr_t)j.src + (size_t)h.sy0 * j.src_pitch + (size_t)h.sx0 * h.sc;
@@ -401,144 +357,129 @@ int encode_job_tmap(const ImpPass& h, ImpJob& j, std::unordered_map<ImpTmKey, Im
     return IMP_OK;
 }
 
-int pick_variant(const ImpPass& h, const ImpJob& j) {
-    // IMP_GPU_FORCE_DIRECT=1 routes everything through the general direct-from-global kernels (used by the tests to keep
-    // the fallback paths — unaligned pitches, oversized footprints, large sigma — covered on the GPU).
+// Which of its pass's launches a job takes: `tiled` when the job's source rows are 16-byte addressable — pitch % 16 == 0
+// and either the image rows or the window rows start 16-byte aligned (imp_tiles.cuh) — and tensor maps can be encoded,
+// `fallback` otherwise. IMP_GPU_FORCE_DIRECT=1 routes every job through imp_pass_kernel (INTER_CUBIC included) or the
+// two-launch Gaussian (used by the tests to keep the general paths — unaligned pitches, oversized footprints, large
+// sigma — covered on the GPU).
+ImpLaunch pick_launch(const ImpHostPass& hp, const uint8_t* src, int sp) {
     static const bool force_direct = [] { const char* e = getenv("IMP_GPU_FORCE_DIRECT"); return e && *e == '1'; }();
-    if (force_direct) return 0;
-    const int fallback = h.kind == IMP_G_CUBIC ? 3 : 0;              // cubic: the column-run kernel has no alignment requirements
-    if (h.tile_smem <= 0 || !encode_tiled()) return fallback;
-    if (j.src_pitch % 16) return fallback;
-    const uintptr_t img = (uintptr_t)j.src;
-    const uintptr_t win = img + (size_t)h.sy0 * j.src_pitch + (size_t)h.sx0 * h.sc;
-    if (img % 16 && win % 16) return fallback;
-    int variant = 1;                                                 // strip kernels: INTER_AREA (and INTER_LINEAR as an A/B candidate)
-    if (h.kind == IMP_G_BLUR) variant = h.blur_r > 0 ? 2 : 0;        // fused blur tile kernel
-    if (h.kind == IMP_G_CUBIC) variant = 4;                          // cubic tile kernel
-    if (h.gt > 0 && h.kind != IMP_G_CUBIC) variant = 5;              // gather tile kernel: index map, INTER_NN, INTER_LINEAR
-    else if (h.kind == IMP_G_COPY || h.kind == IMP_G_NN) return fallback;
-    // the launch must fit the opt-in shared-memory limit the kernels are configured with (many LUT filters can push a
-    // pass over it: ADVICE r1); the direct kernels stage only the ops
-    if (variant && variant_smem(h, variant, variant_param(h, variant)) > kTileSmemLimit) return fallback;
-    return variant;
+    const ImpPass& h = hp.hdr;
+    if (force_direct) return imp_pass_launch(h, h.kind == IMP_G_BLUR ? ImpKernel::BlurGeneric : ImpKernel::Direct);
+    const uintptr_t img = (uintptr_t)src, win = img + (size_t)h.sy0 * sp + (size_t)h.sx0 * h.sc;
+    return encode_tiled() && sp % 16 == 0 && (img % 16 == 0 || win % 16 == 0) ? hp.tiled : hp.fallback;
 }
-int blur_smem_bytes(const ImpPass& h) {
-    const int ops = (h.nops * (int)sizeof(ImpOp) + h.lut_bytes + 15) & ~15;
-    return imp_blur_dyn_smem(h.sc, h.blur_r, ops, h.tile_rs);
-}
-int variant_tiles(const ImpPass& h, int variant);
-int tile_stage_bytes(const ImpPass& h) {
-    const int extra = h.kind == IMP_G_AREA_FRAC ? (((h.tile_ytaps * 8 + 15) & ~15) + 128) : 0;    // staged y taps + the 8 rows' int4 descriptors
-    return (h.tile_smem + extra + 127) & ~127;
-}
-// Ring depth: as many stages as fit 72 KB (three CTAs of 72 KB + ops still share an SM's 227 KB), between 2 and 8.
-// Small tiles (cfg1: 7 KB) need the depth to keep enough bytes in flight; cfg2's 23.7 KB stage gets 3 (1.5 % over 2).
-int tile_stages(const ImpPass& h) {
-    static const int forced = [] { const char* e = getenv("IMP_GPU_STAGES"); return e ? atoi(e) : 0; }();     // tuning knob
-    if (forced >= 2 && forced <= 8) return forced;
-    // the table-ops-only instantiation runs four CTAs per SM (56 registers): 54 KB of ring each instead of 72
-    const bool four = (h.light & 1) && h.kind != IMP_G_AREA_FRAC;
-    return std::max(2, std::min(8, ((four ? 54 : 72) * 1024) / tile_stage_bytes(h)));
-}
-int tile_smem_bytes(const ImpPass& h, int stages) {
-    const int ops = (h.nops * (int)sizeof(ImpOp) + h.lut_bytes + 15) & ~15;
-    return 128 + ((ops + 127) & ~127) + stages * tile_stage_bytes(h) + 64;      // +64: padded taps past the last row
+bool uses_tmap(ImpKernel k) { return k == ImpKernel::Strip || k == ImpKernel::BlurTile || k == ImpKernel::CubicTile || k == ImpKernel::GatherTile; }
+
+// Scratch a plan needs on the device: intermediates between passes + the u16 plane of each generic blur.
+// off[k] = offset of pass k's output (non-final passes); blur_off[k] = offset of pass k's u16 plane.
+// `src`/`sp`: the job's source (null = one of the library's own aligned buffers). The u16 plane is only reserved for a
+// blur that takes the generic kernels (radius > 12, or a pass-0 source whose rows are not 16-byte addressable).
+size_t plan_scratch_layout(const imp_gpu_plan* p, size_t base, std::vector<size_t>& off, std::vector<size_t>& blur_off,
+                           const uint8_t* src = nullptr, int sp = 0) {
+    size_t cur = base;
+    auto take = [&](size_t bytes) { size_t o = cur; cur += (bytes + 255) & ~size_t(255); return o; };
+    off.assign(p->passes.size(), 0); blur_off.assign(p->passes.size(), 0);
+    for (size_t k = 0; k < p->passes.size(); k++) {
+        const ImpHostPass& hp = p->passes[k];
+        if (k + 1 < p->passes.size()) off[k] = take((size_t)pass_pitch(hp) * hp.out_h);
+        if (hp.hdr.kind == IMP_G_BLUR && pick_launch(hp, k == 0 ? src : nullptr, k == 0 ? sp : 0).kernel == ImpKernel::BlurGeneric)
+            blur_off[k] = take((size_t)hp.hdr.sw * hp.hdr.sh * hp.hdr.sc * 2);
+    }
+    return cur;
 }
 
-int variant_param(const ImpPass& h, int variant) { return variant == 1 ? tile_stages(h) : variant == 2 ? h.blur_r : (variant == 5 || variant == 4) ? h.gt : 0; }
-int variant_smem(const ImpPass& h, int variant, int param) {
-    if (variant == 4) return imp_cubic_dyn_smem(h.sc, (h.nops * (int)sizeof(ImpOp) + h.lut_bytes + 15) & ~15, h.tile_rs, h.tile_rows, h.gt, h.dc);
-    if (variant == 5) return imp_gather_dyn_smem(h.gt, (h.nops * (int)sizeof(ImpOp) + h.lut_bytes + 15) & ~15, h.tile_rs, h.tile_rows, h.dc);
-    return variant == 1 ? tile_smem_bytes(h, param) : variant == 2 ? blur_smem_bytes(h) : ops_smem(h);
+ImpJob make_job(const imp_gpu_plan* p, int d, size_t k, const uint8_t* src, int sp, uint8_t* dst, int dp,
+                uint8_t* scratch, const std::vector<size_t>& off) {
+    const imp_gpu_plan::Dev& pd = p->dev[d];
+    ImpJob j{};
+    j.pass = pd.pass_blobs[k];
+    if (p->wm) { j.wm = p->wm->dev[d].d; j.wm_pitch = p->wm->dev[d].pitch; j.wm_c = p->wm->c; }
+    if (k == 0) { j.src = src; j.src_pitch = sp; }
+    else { j.src = scratch + off[k - 1]; j.src_pitch = pass_pitch(p->passes[k - 1]); }
+    if (k + 1 == p->passes.size()) { j.dst = dst; j.dst_pitch = dp; }
+    else { j.dst = scratch + off[k]; j.dst_pitch = pass_pitch(p->passes[k]); }
+    return j;
 }
-int variant_tiles(const ImpPass& h, int variant) {
-    if (variant == 1) return (h.bw + 31) / 32;
-    if (variant == 2) return ((h.bw + IMP_BLUR_TW - 1) / IMP_BLUR_TW) * ((h.bh + IMP_BLUR_TH - 1) / IMP_BLUR_TH);   // same count in destination space
-    if (variant == 3) return ((h.bw + 31) / 32) * ((h.bh + 8 * IMP_CUBIC_RUN - 1) / (8 * IMP_CUBIC_RUN));
-    if (variant == 5) return (((h.bw + h.gt - 1) / h.gt) * ((h.bh + h.gt - 1) / h.gt) + IMP_GATHER_TPC - 1) / IMP_GATHER_TPC;     // CTAs: IMP_GATHER_TPC tiles each
-    if (variant == 4) return ((h.bw + h.gt - 1) / h.gt) * ((h.bh + h.gt - 1) / h.gt);                  // same count in destination space
-    return pass_tiles(h);
+
+// Turns `items` into launch steps and the jobs they cover (in device-table order), pass by pass. Within a pass the jobs are
+// grouped by (kind, sc, kernel, param, flavour, ctas_per_sm), one launch per group in that order; a generic blur is a step
+// of its own. alloc(bytes, &p): where the items' scratch lives (plan_scratch_layout, item after item).
+template <class Alloc>
+int build_steps(const std::vector<imp_gpu_batch::Item>& items, Alloc alloc, imp_gpu_batch::TmCache* tmaps,
+                std::vector<imp_gpu_batch::Step>& steps, std::vector<ImpJob>& jobs) {
+    steps.clear(); jobs.clear();
+    std::vector<std::vector<size_t>> off(items.size()), boff(items.size());
+    size_t bytes = 0;
+    size_t max_passes = 0;
+    for (size_t i = 0; i < items.size(); i++) {
+        bytes = plan_scratch_layout(items[i].plan, bytes, off[i], boff[i], items[i].src, items[i].sp);
+        max_passes = std::max(max_passes, items[i].plan->passes.size());
+    }
+    uint8_t* scratch = nullptr;
+    if (int rc = alloc(bytes, &scratch)) return rc;
+    struct Pending {
+        const ImpPass* hdr; ImpLaunch l; ImpJob job; uint16_t* plane;
+        auto key() const { return std::make_tuple(hdr->kind, hdr->sc, l.kernel, l.param, l.flavour, l.ctas_per_sm); }
+    };
+    std::vector<Pending> pend;
+    for (size_t k = 0; k < max_passes; k++) {
+        pend.clear();
+        for (size_t i = 0; i < items.size(); i++) {
+            const auto& it = items[i];
+            if (it.plan->passes.size() <= k) continue;
+            const ImpHostPass& hp = it.plan->passes[k];
+            ImpJob jb = make_job(it.plan, t_dev, k, it.src, it.sp, it.dst, it.dp, scratch, off[i]);
+            const ImpLaunch l = pick_launch(hp, jb.src, jb.src_pitch);
+            if (uses_tmap(l.kernel)) { int rc = encode_job_tmap(hp.hdr, jb, tmaps); if (rc) return rc; }
+            pend.push_back(Pending{&hp.hdr, l, jb, reinterpret_cast<uint16_t*>(scratch + boff[i][k])});
+        }
+        std::stable_sort(pend.begin(), pend.end(), [](const Pending& a, const Pending& c) { return a.key() < c.key(); });
+        for (size_t s = 0, e; s < pend.size(); s = e) {
+            const bool generic = pend[s].l.kernel == ImpKernel::BlurGeneric;
+            for (e = s + 1; e < pend.size() && !generic && pend[e].key() == pend[s].key(); e++) {}
+            imp_gpu_batch::Step st{};
+            st.g = ImpLaunchGroup{pend[s].hdr->kind, pend[s].hdr->sc, pend[s].l.kernel, pend[s].l.param, pend[s].l.flavour, (int)jobs.size(), (int)(e - s), 0, 0};
+            if (generic) { st.hdr = *pend[s].hdr; st.plane = pend[s].plane; }
+            for (size_t j = s; j < e; j++) {
+                st.g.ctas = std::max(st.g.ctas, pend[j].l.ctas_per_job);
+                st.g.smem_bytes = std::max(st.g.smem_bytes, pend[j].l.smem_bytes);
+                jobs.push_back(pend[j].job);
+            }
+            steps.push_back(st);
+        }
+    }
+    return IMP_OK;
+}
+
+// d_jobs: the device copy of `jobs`; a group of one job takes it by value instead (kernel parameter).
+int launch_steps(const std::vector<imp_gpu_batch::Step>& steps, const std::vector<ImpJob>& jobs, const ImpJob* d_jobs, cudaStream_t st) {
+    for (const auto& s : steps) {
+        if (s.g.kernel == ImpKernel::BlurGeneric) CK(imp_launch_blur_generic(jobs[s.g.first], s.hdr, s.plane, s.g.smem_bytes, st));
+        else if (s.g.count == 1) { ImpLaunchGroup g = s.g; g.first = 0; CK(imp_launch_group(g, nullptr, &jobs[s.g.first], st)); }
+        else CK(imp_launch_group(s.g, d_jobs, nullptr, st));
+    }
+    return IMP_OK;
 }
 
 // `up`: the stream the job table is uploaded on (the stream the launches follow on). Nothing here blocks unless a buffer
 // has to grow or the previous table of this batch is still being copied out of the pinned staging.
 int batch_compile(imp_gpu_batch* b, cudaStream_t up) {
-    const int d = t_dev;
-    b->dev = d;
-    b->steps.clear(); b->h_jobs.clear(); b->algo_bytes = 0; b->launches = 0;
-    size_t scratch = 0;
-    int max_passes = 0;
-    std::vector<std::vector<size_t>> off(b->items.size()), boff(b->items.size());
-    for (size_t i = 0; i < b->items.size(); i++) {
-        imp_gpu_plan* p = b->items[i].plan;
-        int rc = plan_to_device(p);
+    b->dev = t_dev;
+    b->algo_bytes = 0; b->launches = 0;
+    for (const auto& it : b->items) {
+        int rc = plan_to_device(it.plan);
         if (rc) return rc;
-        if ((rc = plan_wait_ready(p, up))) return rc;
-        max_passes = std::max(max_passes, (int)p->passes.size());
-        b->algo_bytes += p->algo_bytes;
-        scratch = plan_scratch_layout(p, scratch, off[i], boff[i], b->items[i].src, b->items[i].sp);
+        if ((rc = plan_wait_ready(it.plan, up))) return rc;
+        b->algo_bytes += it.plan->algo_bytes;
     }
-    { int rc = b->scratch.grow(scratch, false); if (rc) return rc; }
-    // `occ`: how many CTAs of the job's shared-memory footprint fit an SM (capped at the 3 the register budget allows).
-    // A launch takes the largest footprint of its group, so strip jobs are grouped by this class as well: a few big
-    // tiles must not drag thousands of small ones down to two CTAs per SM.
-    struct Pending { int kind, sc, variant, tmax, occ; ImpJob job; ImpPass hdr; size_t boff; };
-    auto occ_class = [](const ImpPass& h, int variant, int param) {
-        if (variant == 4 || variant == 5) return h.light & 1;          // these group by the op-interpreter flavour instead
-        if (variant == 2) return (h.light >> 1) & 1;
-        if (variant != 1) return 0;
-        const bool four = (h.light & 1) && h.kind != IMP_G_AREA_FRAC;
-        return std::max(1, std::min(four ? 4 : 3, (227 * 1024) / (variant_smem(h, variant, param) + 1024))) + ((h.light & 1) ? 8 : (h.light & 4) ? 16 : 0);
-    };
-    for (int k = 0; k < max_passes; k++) {
-        std::vector<Pending> pend;
-        for (size_t i = 0; i < b->items.size(); i++) {
-            const auto& it = b->items[i];
-            if ((int)it.plan->passes.size() <= k) continue;
-            const ImpHostPass& hp = it.plan->passes[k];
-            ImpJob jb = make_job(it.plan, d, k, it.src, it.sp, it.dst, it.dp, b->scratch.p, off[i]);
-            const int variant = pick_variant(hp.hdr, jb);
-            if (variant == 1 || variant == 2 || variant == 4 || variant == 5) { int rc = encode_job_tmap(hp.hdr, jb, &b->tmaps); if (rc) return rc; }
-            const int param = variant_param(hp.hdr, variant);
-            pend.push_back(Pending{hp.hdr.kind, hp.hdr.sc, variant, param, occ_class(hp.hdr, variant, param), jb, hp.hdr, boff[i][k]});
-        }
-        std::stable_sort(pend.begin(), pend.end(), [](const Pending& a, const Pending& c) {
-            if (a.kind != c.kind) return a.kind < c.kind;
-            if (a.sc != c.sc) return a.sc < c.sc;
-            if (a.variant != c.variant) return a.variant < c.variant;
-            if (a.tmax != c.tmax) return a.tmax < c.tmax;
-            return a.occ < c.occ; });
-        size_t s = 0;
-        while (s < pend.size()) {
-            size_t e = s;
-            while (e < pend.size() && pend[e].kind == pend[s].kind && pend[e].sc == pend[s].sc && pend[e].variant == pend[s].variant && pend[e].tmax == pend[s].tmax && pend[e].occ == pend[s].occ) e++;
-            if (pend[s].kind == IMP_G_BLUR && pend[s].variant == 0) {
-                for (size_t j = s; j < e; j++) {
-                    imp_gpu_batch::Step st{};
-                    st.generic_blur = true; st.job = (int)b->h_jobs.size(); st.hdr = pend[j].hdr; st.smem = ops_smem(pend[j].hdr);
-                    st.scratch_off = pend[j].boff;
-                    b->h_jobs.push_back(pend[j].job);
-                    b->steps.push_back(st); b->launches += 2;
-                }
-            } else {
-                imp_gpu_batch::Step st{};
-                st.generic_blur = false;
-                st.g.kind = pend[s].kind; st.g.sc = pend[s].sc; st.g.first = (int)b->h_jobs.size(); st.g.count = (int)(e - s);
-                st.g.max_tiles = 0; st.g.smem_bytes = 16; st.g.variant = pend[s].variant; st.g.tmax = pend[s].tmax;
-                st.g.light = (pend[s].variant == 2 || pend[s].variant == 4 || pend[s].variant == 5) ? pend[s].occ : (pend[s].variant == 1 ? (pend[s].occ >= 16 ? 2 : pend[s].occ >= 8 ? 1 : 0) : 0);
-                for (size_t j = s; j < e; j++) {
-                    st.g.max_tiles = std::max(st.g.max_tiles, variant_tiles(pend[j].hdr, pend[s].variant));
-                    st.g.smem_bytes = std::max(st.g.smem_bytes, variant_smem(pend[j].hdr, pend[s].variant, pend[s].tmax));
-                    b->h_jobs.push_back(pend[j].job);
-                }
-                b->steps.push_back(st); b->launches += 1;
-            }
-            s = e;
-        }
-    }
-    // a launch group of one job takes it by value (kernel parameter): the device table is only needed for real groups
+    auto grow = [b](size_t bytes, uint8_t** p) { int rc = b->scratch.grow(bytes, false); *p = b->scratch.p; return rc; };
+    if (int rc = build_steps(b->items, grow, &b->tmaps, b->steps, b->h_jobs)) return rc;
     b->table_needed = false;
-    for (const auto& st : b->steps) if (!st.generic_blur && st.g.count > 1) b->table_needed = true;
+    for (const auto& st : b->steps) {
+        b->launches += st.g.kernel == ImpKernel::BlurGeneric ? 2 : 1;
+        if (st.g.count > 1) b->table_needed = true;
+    }
     if (b->table_needed) {
         if (b->h_jobs.size() > b->jobs_cap) {
             if (b->d_jobs) CK(cudaFree(b->d_jobs));
@@ -560,15 +501,6 @@ int batch_compile(imp_gpu_batch* b, cudaStream_t up) {
     return IMP_OK;
 }
 
-int batch_launch_steps(imp_gpu_batch* b, cudaStream_t st) {
-    for (const auto& s : b->steps) {
-        if (s.generic_blur) CK(imp_launch_blur_generic(b->h_jobs[s.job], s.hdr, (uint16_t*)(b->scratch.p + s.scratch_off), s.smem, st));
-        else if (s.g.count == 1) { ImpLaunchGroup g = s.g; g.first = 0; CK(imp_launch_group(g, nullptr, &b->h_jobs[s.g.first], st)); }
-        else CK(imp_launch_group(s.g, b->d_jobs, nullptr, st));
-    }
-    return IMP_OK;
-}
-
 void batch_release(imp_gpu_batch* b) {          // device/pinned memory of a batch (its device must be current)
     if (b->d_jobs) cudaFree(b->d_jobs);
     b->d_jobs = nullptr; b->jobs_cap = 0;
@@ -577,33 +509,10 @@ void batch_release(imp_gpu_batch* b) {          // device/pinned memory of a bat
     b->up_ev = nullptr; b->up_pending = false;
 }
 
-// One frame with by-value job descriptors: no device job table, nothing to free afterwards.
-// `scratch` must hold plan_scratch_layout(plan) bytes (or be null when the plan needs none).
-int launch_single(imp_gpu_plan* p, const uint8_t* src, int sp, uint8_t* dst, int dp, uint8_t* scratch, cudaStream_t st) {
-    std::vector<size_t> off, boff;
-    plan_scratch_layout(p, 0, off, boff, src, sp);
-    for (size_t k = 0; k < p->passes.size(); k++) {
-        const ImpHostPass& hp = p->passes[k];
-        ImpJob j = make_job(p, t_dev, k, src, sp, dst, dp, scratch, off);
-        const int variant = pick_variant(hp.hdr, j);
-        if (variant == 1 || variant == 2 || variant == 4 || variant == 5) { int rc = encode_job_tmap(hp.hdr, j, nullptr); if (rc) return rc; }
-        if (hp.hdr.kind == IMP_G_BLUR && variant == 0) {
-            CK(imp_launch_blur_generic(j, hp.hdr, (uint16_t*)(scratch + boff[k]), ops_smem(hp.hdr), st));
-        } else {
-            const int param = variant_param(hp.hdr, variant);
-            ImpLaunchGroup g{hp.hdr.kind, hp.hdr.sc, 0, 1, variant_tiles(hp.hdr, variant), variant_smem(hp.hdr, variant, param), variant, param, variant == 2 ? ((hp.hdr.light >> 1) & 1) : (hp.hdr.light & 1) ? 1 : (variant == 1 && (hp.hdr.light & 4)) ? 2 : 0};
-            CK(imp_launch_group(g, nullptr, &j, st));
-        }
-    }
-    return IMP_OK;
-}
-
-size_t plan_scratch_bytes(const imp_gpu_plan* p, const uint8_t* src = nullptr, int sp = 0) { std::vector<size_t> a, b; return plan_scratch_layout(p, 0, a, b, src, sp); }
-
 
 // ---- the chunked end-to-end path over host buffers ---------------------------------------------------------------------
 // Requests are cut into CHUNKS of consecutive jobs (up to kChunkJobs jobs / kChunkBytes of crop windows); a chunk owns one
-// lane (stream + staging) while it is in flight: H2D of every window, ONE grouped launch per kernel variant over the whole
+// lane (stream + staging) while it is in flight: H2D of every window, ONE launch per (pass, kernel choice) over the whole
 // chunk through a device job table (the path the device-resident batches take), D2H of every result. Lanes rotate, so the
 // copies of chunk k+1 overlap the kernels of chunk k and the D2H of chunk k-1 (PCIe is full duplex).
 constexpr int kChunkJobs = 256;
@@ -860,7 +769,7 @@ int lane_issue(Lane& L, const HostJobs& J, int first, int last) {
     if (L.up_done) CK(cudaEventRecord(L.up_done, L.st));
     for (const Repitch& q : repitch) CK(imp_launch_repitch(q.src, q.sp, q.dst, q.dp, q.row_bytes, q.rows, L.st));
     if ((r = batch_compile(&B, L.st))) return r;
-    if ((r = batch_launch_steps(&B, L.st))) return r;
+    if ((r = launch_steps(B.steps, B.h_jobs, B.d_jobs, L.st))) return r;
     for (int k = 0; k < m; k++) {
         const int i = first + k;
         const imp_gpu_plan* p = J.plans[i];
@@ -1158,7 +1067,7 @@ int imp_gpu_batch_launch(imp_gpu_batch* b, void* stream) {
         try { rc = batch_compile(b, st); } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
         if (rc) return rc;
     }
-    return batch_launch_steps(b, st);
+    return launch_steps(b->steps, b->h_jobs, b->d_jobs, st);
 }
 
 // ---- one frame -----------------------------------------------------------------------------------------
@@ -1171,10 +1080,18 @@ int imp_gpu_run_device(imp_gpu_plan* plan, const void* d_src, int sp, void* d_ds
     if ((rc = plan_to_device(plan))) return rc;
     cudaStream_t st = pick_stream(stream);
     if ((rc = plan_wait_ready(plan, st))) return rc;
-    const size_t need = plan_scratch_bytes(plan, (const uint8_t*)d_src, sp);
+    // the batch's steps over this one frame: every group holds one job, passed by value (no device job table)
     uint8_t* scratch = nullptr;
-    if (need) CK(cudaMallocAsync((void**)&scratch, need, st));        // stream-ordered: stays asynchronous
-    rc = launch_single(plan, (const uint8_t*)d_src, sp, (uint8_t*)d_dst, dp, scratch, st);
+    auto alloc = [&](size_t bytes, uint8_t** p) {
+        if (bytes) CK(cudaMallocAsync((void**)&scratch, bytes, st));      // stream-ordered: stays asynchronous
+        *p = scratch;
+        return IMP_OK;
+    };
+    std::vector<imp_gpu_batch::Step> steps;
+    std::vector<ImpJob> jobs;
+    try { rc = build_steps({imp_gpu_batch::Item{plan, (const uint8_t*)d_src, sp, (uint8_t*)d_dst, dp}}, alloc, nullptr, steps, jobs); }
+    catch (const std::bad_alloc&) { rc = IMP_ERROR_MALLOC_FAILED; }
+    if (!rc) rc = launch_steps(steps, jobs, nullptr, st);
     if (scratch) CK(cudaFreeAsync(scratch, st));
     return rc;
 }

@@ -9,6 +9,35 @@
 #include "imp_plan.h"
 #include "../../include/imp_gpu.h"
 
+// ---- launch choice --------------------------------------------------------------------------------
+// The kernel that runs a pass. The values order a pass's launch groups (batch_compile sorts by them); BlurGeneric sorts
+// before BlurTile, where the two-launch Gaussian has always stood.
+enum class ImpKernel : int {
+    BlurGeneric = -1,    // imp_blur_h_kernel + imp_blur_v_kernel through a u16 plane, one job per launch pair (any sigma)
+    Direct = 0,          // imp_pass_kernel<KIND, C> (imp_kernels.cu): any pitch, alignment and footprint
+    Strip = 1,           // imp_strip_kernel<C, MODE, FL> (imp_tiles.cuh): INTER_AREA, shrinking INTER_LINEAR
+    BlurTile = 2,        // imp_blur_tile_kernel<C, R, NOCOMP> (imp_blur.cuh): tap radius <= 12
+    CubicRun = 3,        // imp_cubic_run_kernel<C> (imp_kernels.cu): INTER_CUBIC, any pitch and alignment
+    CubicTile = 4,       // imp_cubic_tile_kernel<C, LIGHT> (imp_cubic.cuh)
+    GatherTile = 5,      // imp_gather_tile_kernel<C, KIND, LIGHT> (imp_gathertile.cuh): index map, NN, enlarging INTER_LINEAR
+};
+// Dynamic shared memory the tile kernels are configured for (cudaFuncAttributeMaxDynamicSharedMemorySize); a tile launch
+// whose footprint exceeds it (many LUT filters can push a pass over) takes the pass's fallback kernel instead.
+constexpr int IMP_SMEM_OPTIN = 200 * 1024;
+// How one job of a pass is launched.
+struct ImpLaunch {
+    ImpKernel kernel;
+    int param;           // Strip: ring stages; BlurTile: tap radius; CubicTile, GatherTile: tile edge; otherwise 0
+    int flavour;         // op interpreter: 0 general, 1 fused tables only, 2 (Strip) compositing + tables; BlurTile: 1 = NOCOMP
+    int smem_bytes;      // dynamic shared memory
+    int ctas_per_job;    // grid.x (BlurGeneric: 0, its launches size their own 2-D grid)
+    int ctas_per_sm;     // Strip: CTAs of this footprint an SM holds, the occupancy class strip jobs are grouped by; otherwise 0
+};
+// imp_planner.cpp: the launch of pass `h` on kernel `k` (one that serves the pass's kind), and the pass's two choices
+// (ImpHostPass::tiled, ::fallback below).
+ImpLaunch imp_pass_launch(const ImpPass& h, ImpKernel k);
+void imp_pass_launches(const ImpPass& h, ImpLaunch* tiled, ImpLaunch* fallback);
+
 // ---- planner output (host) ------------------------------------------------------------------------
 struct ImpHostPass {
     ImpPass hdr;                       // offsets filled by finalize()
@@ -17,6 +46,10 @@ struct ImpHostPass {
     int out_w, out_h, out_c;           // stored image
     int uses_watermark;
     double sigma;                      // BLUR only
+    // Jobs whose source rows are 16-byte addressable take `tiled` (a shared-memory tile kernel when the pass has one and
+    // its footprint fits IMP_SMEM_OPTIN, else the same as `fallback`); every other job takes `fallback`: Direct, CubicRun
+    // or BlurGeneric by kind.
+    ImpLaunch tiled, fallback;
 };
 
 // A decoded overlay (what PrepareWatermark leaves in the conf pool, bridge.c:199-237). The reference decodes it ONCE at
@@ -62,21 +95,42 @@ int imp_build_plan(const imp_gpu_request* req, const imp_gpu_config* cfg, int w,
 
 // imp_kernels.cu
 #define IMP_CUBIC_RUN 8           // imp_cubic_run_kernel: output rows per thread; a CTA covers 32 x (8 * IMP_CUBIC_RUN) pixels
+unsigned long long imp_launches();
+void imp_count_launches(int n);
+// One launch over jobs that share kind, source channels and the launch choice (kernel, param, flavour).
 struct ImpLaunchGroup {
-    int kind, sc;                // kernel variant
+    int kind, sc;                // ImpGather and source channels of every job
+    ImpKernel kernel;            // never BlurGeneric (imp_launch_blur_generic)
+    int param, flavour;          // as in ImpLaunch
     int first, count;            // jobs [first, first+count) of the device job table
-    int max_tiles;               // largest tile count of any job in the group (grid.x)
-    int smem_bytes;              // ops + LUT staging (+ source tile for tile variants)
-    int variant;                 // 0 = direct-from-global kernel, 1 = shared-memory tile kernel (imp_tiles.cuh)
-    int tmax;                    // tile variant: number of ring stages (2..8)
-    int light;                   // gather / cubic tile kernels: the table-ops-only instantiation (ImpPass::light of every job)
+    int ctas;                    // grid.x: the largest ctas_per_job of the group
+    int smem_bytes;              // the largest smem_bytes of the group
 };
 // d_jobs == nullptr: a single job passed by value (`one`), no device job table needed.
 cudaError_t imp_launch_group(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st);
+#if defined(__CUDACC__)
+// Launches Kernel(jobs, first, count, one, extra...) over a group: grid.x = g.ctas, the jobs over grid.y (and z beyond
+// 65535). OptIn: the kernel is configured for IMP_SMEM_OPTIN bytes of dynamic shared memory, once per device.
+template <auto Kernel, bool OptIn = true, class... Extra>
+cudaError_t imp_launch_jobs(const ImpLaunchGroup& g, dim3 block, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st, Extra... extra) {
+    if (OptIn) {
+        static std::atomic<bool> attr_set[16];             // per device; setting the attribute twice is harmless
+        int dev = 0; cudaGetDevice(&dev);
+        if (!attr_set[dev & 15]) {
+            cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, IMP_SMEM_OPTIN);
+            if (e != cudaSuccess) return e;
+            attr_set[dev & 15] = true;
+        }
+    }
+    const ImpJob dummy{};
+    dim3 grid(g.ctas, g.count < 65535 ? g.count : 65535, (g.count + 65534) / 65535);
+    Kernel<<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, one ? *one : dummy, extra...);
+    imp_count_launches(1);
+    return cudaGetLastError();
+}
+#endif
 // Two-kernel Gaussian through a u16 scratch (any sigma). One job, passed by value.
 cudaError_t imp_launch_blur_generic(const ImpJob& job, const ImpPass& hdr, uint16_t* d_scratch, int smem_bytes, cudaStream_t st);
-unsigned long long imp_launches();
-void imp_count_launches(int n);
 cudaError_t imp_upload_tables();
 // one translation unit per kernel family (each with its own copy of the per-byte division tables, imp_pixel.cuh)
 cudaError_t imp_upload_tables_strip();

@@ -1,43 +1,31 @@
 // imp_k_blur.cu — translation unit of the fused Gaussian blur tile kernel (imp_blur.cuh).
 #include "imp_internal.h"
-#include <atomic>
 #include "imp_blur.cuh"
 
 cudaError_t imp_upload_tables_blur() { return imp_upload_tables_tu(); }
 unsigned imp_debug_flags_blur() { return imp_debug_flags_tu(); }
 
-template <int SC, int R, bool NOCOMP>
-static cudaError_t launch_blur_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob& o, cudaStream_t st) {
-    static std::atomic<bool> attr_set[16];                 // per device; setting the attribute twice is harmless
-    int dev = 0; cudaGetDevice(&dev);
-    auto kern = imp_tiles::imp_blur_tile_kernel<SC, R, NOCOMP>;
-    if (!attr_set[dev & 15]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev & 15] = true;
-    }
-    dim3 block(imp_tiles::BLUR_THREADS);
-    dim3 grid(g.max_tiles, g.count < 65535 ? g.count : 65535, (g.count + 65534) / 65535);      // max_tiles = tiles of a job
-    kern<<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o);
-    imp_count_launches(1);
-    return cudaGetLastError();
+template <int SC, int R>
+static cudaError_t launch_blur_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
+    using imp_tiles::imp_blur_tile_kernel;
+    const dim3 block(imp_tiles::BLUR_THREADS);
+    return g.flavour ? imp_launch_jobs<imp_blur_tile_kernel<SC, R, true>>(g, block, d_jobs, one, st)
+                     : imp_launch_jobs<imp_blur_tile_kernel<SC, R, false>>(g, block, d_jobs, one, st);
 }
 
 template <int SC>
-static cudaError_t launch_blur_tile_r(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob& o, cudaStream_t st) {
-    switch (g.tmax) {
-        case 3:  return g.light ? launch_blur_tile<SC, 3, true>(g, d_jobs, o, st) : launch_blur_tile<SC, 3, false>(g, d_jobs, o, st);
-        case 6:  return g.light ? launch_blur_tile<SC, 6, true>(g, d_jobs, o, st) : launch_blur_tile<SC, 6, false>(g, d_jobs, o, st);
-        case 9:  return g.light ? launch_blur_tile<SC, 9, true>(g, d_jobs, o, st) : launch_blur_tile<SC, 9, false>(g, d_jobs, o, st);
-        case 12: return g.light ? launch_blur_tile<SC, 12, true>(g, d_jobs, o, st) : launch_blur_tile<SC, 12, false>(g, d_jobs, o, st);
+static cudaError_t launch_blur_tile_r(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
+    switch (g.param) {                                     // tap radius
+        case 3:  return launch_blur_tile<SC, 3>(g, d_jobs, one, st);
+        case 6:  return launch_blur_tile<SC, 6>(g, d_jobs, one, st);
+        case 9:  return launch_blur_tile<SC, 9>(g, d_jobs, one, st);
+        case 12: return launch_blur_tile<SC, 12>(g, d_jobs, one, st);
     }
     return cudaErrorInvalidValue;
 }
 
 cudaError_t imp_launch_blur_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
-    const ImpJob dummy{};
-    const ImpJob& o = one ? *one : dummy;
-    if (g.sc == 3) return launch_blur_tile_r<3>(g, d_jobs, o, st);
-    if (g.sc == 4) return launch_blur_tile_r<4>(g, d_jobs, o, st);
+    if (g.sc == 3) return launch_blur_tile_r<3>(g, d_jobs, one, st);
+    if (g.sc == 4) return launch_blur_tile_r<4>(g, d_jobs, one, st);
     return cudaErrorInvalidValue;
 }

@@ -1,35 +1,17 @@
 // imp_k_cubic.cu — translation unit of the INTER_CUBIC tile kernel (imp_cubic.cuh).
 #include "imp_internal.h"
-#include <atomic>
 #include "imp_cubic.cuh"
 
 cudaError_t imp_upload_tables_cubic() { return imp_upload_tables_tu(); }
 unsigned imp_debug_flags_cubic() { return imp_debug_flags_tu(); }
 
-template <int SC, bool LIGHT>
-static cudaError_t launch_cubic_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob& o, cudaStream_t st) {
-    static std::atomic<bool> attr_set[16];
-    int dev = 0; cudaGetDevice(&dev);
-    auto kern = imp_tiles::imp_cubic_tile_kernel<SC, LIGHT>;
-    if (!attr_set[dev & 15]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev & 15] = true;
-    }
-    dim3 block(imp_tiles::CUBIC_THREADS);
-    dim3 grid(g.max_tiles, g.count < 65535 ? g.count : 65535, (g.count + 65534) / 65535);      // max_tiles = output tiles of a job
-    kern<<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o);
-    imp_count_launches(1);
-    return cudaGetLastError();
-}
-
 cudaError_t imp_launch_cubic_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
-    const ImpJob dummy{};
-    const ImpJob& o = one ? *one : dummy;
+    using imp_tiles::imp_cubic_tile_kernel;
+    const dim3 block(imp_tiles::CUBIC_THREADS);
     switch (g.sc) {
-        case 1: return g.light ? launch_cubic_tile<1, true>(g, d_jobs, o, st) : launch_cubic_tile<1, false>(g, d_jobs, o, st);
-        case 3: return g.light ? launch_cubic_tile<3, true>(g, d_jobs, o, st) : launch_cubic_tile<3, false>(g, d_jobs, o, st);
-        case 4: return g.light ? launch_cubic_tile<4, true>(g, d_jobs, o, st) : launch_cubic_tile<4, false>(g, d_jobs, o, st);
+        case 1: return g.flavour ? imp_launch_jobs<imp_cubic_tile_kernel<1, true>>(g, block, d_jobs, one, st) : imp_launch_jobs<imp_cubic_tile_kernel<1, false>>(g, block, d_jobs, one, st);
+        case 3: return g.flavour ? imp_launch_jobs<imp_cubic_tile_kernel<3, true>>(g, block, d_jobs, one, st) : imp_launch_jobs<imp_cubic_tile_kernel<3, false>>(g, block, d_jobs, one, st);
+        case 4: return g.flavour ? imp_launch_jobs<imp_cubic_tile_kernel<4, true>>(g, block, d_jobs, one, st) : imp_launch_jobs<imp_cubic_tile_kernel<4, false>>(g, block, d_jobs, one, st);
     }
     return cudaErrorInvalidValue;
 }

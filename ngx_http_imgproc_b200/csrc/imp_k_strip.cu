@@ -1,43 +1,37 @@
 // imp_k_strip.cu — translation unit of the persistent TMA strip kernels (imp_tiles.cuh): INTER_AREA fractional / integer.
 #include "imp_internal.h"
-#include <atomic>
 #include "imp_tiles.cuh"
 
 cudaError_t imp_upload_tables_strip() { return imp_upload_tables_tu(); }
 unsigned imp_debug_flags_strip() { return imp_debug_flags_tu(); }
 
-template <int SC, int MODE, int FL>
-static cudaError_t launch_strip(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob& o, cudaStream_t st) {
-    static std::atomic<bool> attr_set[16];                 // per device; setting the attribute twice is harmless
-    int dev = 0; cudaGetDevice(&dev);
-    auto kern = imp_tiles::imp_strip_kernel<SC, MODE, FL>;
-    if (!attr_set[dev & 15]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev & 15] = true;
+template <int SC, int MODE>
+static cudaError_t launch_strip(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
+    using imp_tiles::imp_strip_kernel;
+    const dim3 block(imp_tiles::STRIP_THREADS);
+    switch (g.flavour) {
+        case 1:  return imp_launch_jobs<imp_strip_kernel<SC, MODE, 1>>(g, block, d_jobs, one, st, g.param);
+        case 2:  return imp_launch_jobs<imp_strip_kernel<SC, MODE, 2>>(g, block, d_jobs, one, st, g.param);
+        default: return imp_launch_jobs<imp_strip_kernel<SC, MODE, 0>>(g, block, d_jobs, one, st, g.param);
     }
-    dim3 block(imp_tiles::STRIP_THREADS);
-    dim3 grid(g.max_tiles, g.count < 65535 ? g.count : 65535, (g.count + 65534) / 65535);      // max_tiles = strips (tile columns)
-    kern<<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o, g.tmax);
-    imp_count_launches(1);
-    return cudaGetLastError();
 }
 
+template <int MODE>
+static cudaError_t launch_strip_sc(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
+    switch (g.sc) {
+        case 1: return launch_strip<1, MODE>(g, d_jobs, one, st);
+        case 3: return launch_strip<3, MODE>(g, d_jobs, one, st);
+        case 4: return launch_strip<4, MODE>(g, d_jobs, one, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+// strip kernel modes (imp_tiles.cuh): 0 fractional INTER_AREA, 1 integer INTER_AREA, 3 INTER_LINEAR
 cudaError_t imp_launch_strip(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
-    const ImpJob dummy{};
-    const ImpJob& o = one ? *one : dummy;
-    // strip kernel modes (imp_tiles.cuh): 0 fractional INTER_AREA, 1 integer INTER_AREA, 3 INTER_LINEAR
-    const int mode = g.kind == IMP_G_AREA_FRAC ? 0 : g.kind == IMP_G_AREA_INT ? 1 : g.kind == IMP_G_LINEAR ? 3 : -1;
-    switch (mode * 8 + g.sc) {
-        case 0 * 8 + 1: return g.light == 1 ? launch_strip<1, 0, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<1, 0, 2>(g, d_jobs, o, st) : launch_strip<1, 0, 0>(g, d_jobs, o, st);
-        case 0 * 8 + 3: return g.light == 1 ? launch_strip<3, 0, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<3, 0, 2>(g, d_jobs, o, st) : launch_strip<3, 0, 0>(g, d_jobs, o, st);
-        case 0 * 8 + 4: return g.light == 1 ? launch_strip<4, 0, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<4, 0, 2>(g, d_jobs, o, st) : launch_strip<4, 0, 0>(g, d_jobs, o, st);
-        case 1 * 8 + 1: return g.light == 1 ? launch_strip<1, 1, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<1, 1, 2>(g, d_jobs, o, st) : launch_strip<1, 1, 0>(g, d_jobs, o, st);
-        case 1 * 8 + 3: return g.light == 1 ? launch_strip<3, 1, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<3, 1, 2>(g, d_jobs, o, st) : launch_strip<3, 1, 0>(g, d_jobs, o, st);
-        case 1 * 8 + 4: return g.light == 1 ? launch_strip<4, 1, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<4, 1, 2>(g, d_jobs, o, st) : launch_strip<4, 1, 0>(g, d_jobs, o, st);
-        case 3 * 8 + 1: return g.light == 1 ? launch_strip<1, 3, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<1, 3, 2>(g, d_jobs, o, st) : launch_strip<1, 3, 0>(g, d_jobs, o, st);
-        case 3 * 8 + 3: return g.light == 1 ? launch_strip<3, 3, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<3, 3, 2>(g, d_jobs, o, st) : launch_strip<3, 3, 0>(g, d_jobs, o, st);
-        case 3 * 8 + 4: return g.light == 1 ? launch_strip<4, 3, 1>(g, d_jobs, o, st) : g.light == 2 ? launch_strip<4, 3, 2>(g, d_jobs, o, st) : launch_strip<4, 3, 0>(g, d_jobs, o, st);
+    switch (g.kind) {
+        case IMP_G_AREA_FRAC: return launch_strip_sc<0>(g, d_jobs, one, st);
+        case IMP_G_AREA_INT:  return launch_strip_sc<1>(g, d_jobs, one, st);
+        case IMP_G_LINEAR:    return launch_strip_sc<3>(g, d_jobs, one, st);
     }
     return cudaErrorInvalidValue;
 }

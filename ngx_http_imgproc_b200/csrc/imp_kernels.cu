@@ -472,54 +472,51 @@ __global__ void __launch_bounds__(256) imp_blur_v_kernel(const ImpJob job, const
 }
 
 template <int KIND>
-cudaError_t launch_kind(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
-    const int tiles = g.max_tiles;
-    const ImpJob dummy{};
-    const ImpJob& o = one ? *one : dummy;
-    dim3 block(TILE_W, TILE_H);
-    dim3 grid(tiles, g.count < 65535 ? g.count : 65535, (g.count + 65534) / 65535);
+cudaError_t launch_direct_sc(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
+    const dim3 block(TILE_W, TILE_H);                  // grid.x: 32 x (8 * PASS_PPT) tiles
     switch (g.sc) {
-        case 1: imp_pass_kernel<KIND, 1><<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o); break;
-        case 3: imp_pass_kernel<KIND, 3><<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o); break;
-        case 4: imp_pass_kernel<KIND, 4><<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o); break;
-        default: return cudaErrorInvalidValue;
+        case 1: return imp_launch_jobs<imp_pass_kernel<KIND, 1>, false>(g, block, d_jobs, one, st);
+        case 3: return imp_launch_jobs<imp_pass_kernel<KIND, 3>, false>(g, block, d_jobs, one, st);
+        case 4: return imp_launch_jobs<imp_pass_kernel<KIND, 4>, false>(g, block, d_jobs, one, st);
     }
-    g_imp_launches++;
-    return cudaGetLastError();
+    return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_direct(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
+    switch (g.kind) {
+        case IMP_G_COPY:      return launch_direct_sc<IMP_G_COPY>(g, d_jobs, one, st);
+        case IMP_G_NN:        return launch_direct_sc<IMP_G_NN>(g, d_jobs, one, st);
+        case IMP_G_AREA_INT:  return launch_direct_sc<IMP_G_AREA_INT>(g, d_jobs, one, st);
+        case IMP_G_AREA_FRAC: return launch_direct_sc<IMP_G_AREA_FRAC>(g, d_jobs, one, st);
+        case IMP_G_CUBIC:     return launch_direct_sc<IMP_G_CUBIC>(g, d_jobs, one, st);
+        case IMP_G_LINEAR:    return launch_direct_sc<IMP_G_LINEAR>(g, d_jobs, one, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_cubic_run(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
+    const dim3 block(TILE_W, TILE_H);                  // grid.x: 32 x (8 * CUBIC_RUN) tiles
+    switch (g.sc) {
+        case 1: return imp_launch_jobs<imp_cubic_run_kernel<1>, false>(g, block, d_jobs, one, st);
+        case 3: return imp_launch_jobs<imp_cubic_run_kernel<3>, false>(g, block, d_jobs, one, st);
+        case 4: return imp_launch_jobs<imp_cubic_run_kernel<4>, false>(g, block, d_jobs, one, st);
+    }
+    return cudaErrorInvalidValue;
 }
 
 }  // namespace
 
-cudaError_t launch_cubic_run(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
-    const ImpJob dummy{};
-    const ImpJob& o = one ? *one : dummy;
-    dim3 block(TILE_W, TILE_H);
-    dim3 grid(g.max_tiles, g.count < 65535 ? g.count : 65535, (g.count + 65534) / 65535);     // max_tiles = 32 x (8*CUBIC_RUN) tiles
-    switch (g.sc) {
-        case 1: imp_cubic_run_kernel<1><<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o); break;
-        case 3: imp_cubic_run_kernel<3><<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o); break;
-        case 4: imp_cubic_run_kernel<4><<<grid, block, g.smem_bytes, st>>>(d_jobs, g.first, g.count, o); break;
-        default: return cudaErrorInvalidValue;
-    }
-    g_imp_launches++;
-    return cudaGetLastError();
-}
-
 cudaError_t imp_launch_group(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
-    if (g.variant == 3 && g.kind == IMP_G_CUBIC) return launch_cubic_run(g, d_jobs, one, st);
-    if (g.variant == 2 && g.kind == IMP_G_BLUR) return imp_launch_blur_tile(g, d_jobs, one, st);       // imp_k_blur.cu
-    if (g.variant == 4 && g.kind == IMP_G_CUBIC) return imp_launch_cubic_tile(g, d_jobs, one, st);     // imp_k_cubic.cu
-    if (g.variant == 5) return imp_launch_gather_tile(g, d_jobs, one, st);                             // imp_k_gather.cu
-    if (g.variant == 1) return imp_launch_strip(g, d_jobs, one, st);                                   // imp_k_strip.cu
-    switch (g.kind) {
-        case IMP_G_COPY:      return launch_kind<IMP_G_COPY>(g, d_jobs, one, st);
-        case IMP_G_NN:        return launch_kind<IMP_G_NN>(g, d_jobs, one, st);
-        case IMP_G_AREA_INT:  return launch_kind<IMP_G_AREA_INT>(g, d_jobs, one, st);
-        case IMP_G_AREA_FRAC: return launch_kind<IMP_G_AREA_FRAC>(g, d_jobs, one, st);
-        case IMP_G_CUBIC:     return launch_kind<IMP_G_CUBIC>(g, d_jobs, one, st);
-        case IMP_G_LINEAR:    return launch_kind<IMP_G_LINEAR>(g, d_jobs, one, st);
-        default: return cudaErrorInvalidValue;
+    switch (g.kernel) {
+        case ImpKernel::Direct:     return launch_direct(g, d_jobs, one, st);
+        case ImpKernel::Strip:      return imp_launch_strip(g, d_jobs, one, st);          // imp_k_strip.cu
+        case ImpKernel::BlurTile:   return imp_launch_blur_tile(g, d_jobs, one, st);      // imp_k_blur.cu
+        case ImpKernel::CubicRun:   return launch_cubic_run(g, d_jobs, one, st);
+        case ImpKernel::CubicTile:  return imp_launch_cubic_tile(g, d_jobs, one, st);     // imp_k_cubic.cu
+        case ImpKernel::GatherTile: return imp_launch_gather_tile(g, d_jobs, one, st);    // imp_k_gather.cu
+        case ImpKernel::BlurGeneric: break;                                               // imp_launch_blur_generic
     }
+    return cudaErrorInvalidValue;
 }
 
 cudaError_t imp_launch_blur_generic(const ImpJob& job, const ImpPass& hdr, uint16_t* d_scratch, int smem_bytes, cudaStream_t st) {

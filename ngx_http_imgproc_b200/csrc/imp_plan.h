@@ -82,7 +82,7 @@ struct ImpPass {
                               // alignments), u32 tapv[2][NWV] (dp2a, two parities); ImpBlurDims<R> below
     int max_xtaps, max_ytaps; // AREA_FRAC: largest tap count per output column / row
     int tile_rs, tile_rows;   // tile kernels: shared-memory row stride (bytes) and max source rows per 32x8 tile
-    int tile_smem;            // tile kernels: source-tile bytes (tile_rs*tile_rows); 0 = no tile variant for this pass
+    int tile_smem;            // tile kernels: source-tile bytes (tile_rs*tile_rows); 0 = no tile kernel for this pass
     int xtile_off, ytile_off; // tile kernels: int2 per tile column {first px, last px}; int4 per tile row {first src row, rows, first y tap, y taps}
     int light;                // bit 0: every op of the pass is a fused table (IMP_OP_LUT3 / IMP_OP_MAXLUT3) or there is none: the strip,
                               // gather and cubic kernels then run an instantiation whose op interpreter knows only those two (fewer

@@ -76,6 +76,66 @@ void imp_wm_registry_clear() {
     { std::lock_guard<std::mutex> lk(g_wm_mu); drop.swap(g_wm_registry); }
 }
 
+// ---- launch choice (the runtime picks `tiled` or `fallback` per job: imp_gpu.cu, pick_launch) ---------------------------
+ImpLaunch imp_pass_launch(const ImpPass& h, ImpKernel k) {
+    const int ops16 = (h.nops * (int)sizeof(ImpOp) + h.lut_bytes + 15) & ~15;
+    ImpLaunch l{k, 0, 0, std::max(16, h.nops * (int)sizeof(ImpOp) + h.lut_bytes), 0, 0};     // the direct kernels stage only the ops
+    switch (k) {
+        case ImpKernel::BlurGeneric: break;
+        case ImpKernel::Direct: l.ctas_per_job = ((h.bw + 31) / 32) * ((h.bh + 31) / 32); break;
+        case ImpKernel::CubicRun: l.ctas_per_job = ((h.bw + 31) / 32) * ((h.bh + 8 * IMP_CUBIC_RUN - 1) / (8 * IMP_CUBIC_RUN)); break;
+        case ImpKernel::Strip: {
+            // one ring stage: the source box (+ the staged y taps and the 8 rows' int4 descriptors of fractional AREA)
+            const int extra = h.kind == IMP_G_AREA_FRAC ? (((h.tile_ytaps * 8 + 15) & ~15) + 128) : 0;
+            const int stage = (h.tile_smem + extra + 127) & ~127;
+            // The table-ops-only instantiation runs four CTAs per SM (56 registers), the others three. Ring depth: as many
+            // stages as fit 72 KB (three CTAs of 72 KB + ops still share an SM's 227 KB; 54 KB for four), between 2 and 8.
+            // Small tiles (cfg1: 7 KB) need the depth to keep enough bytes in flight; cfg2's 23.7 KB stage gets 3 (1.5 % over 2).
+            const bool four = (h.light & 1) && h.kind != IMP_G_AREA_FRAC;
+            l.param = std::max(2, std::min(8, ((four ? 54 : 72) * 1024) / stage));
+            l.flavour = (h.light & 1) ? 1 : (h.light & 4) ? 2 : 0;
+            l.smem_bytes = 128 + ((ops16 + 127) & ~127) + l.param * stage + 64;      // +64: padded taps past the last row
+            l.ctas_per_job = (h.bw + 31) / 32;                                          // strips (tile columns)
+            // A launch takes the largest footprint of its group, so strip jobs are grouped by this class as well: a few big
+            // tiles must not drag thousands of small ones down to two CTAs per SM.
+            l.ctas_per_sm = std::max(1, std::min(four ? 4 : 3, (227 * 1024) / (l.smem_bytes + 1024)));
+        } break;
+        case ImpKernel::BlurTile:
+            l.param = h.blur_r;
+            l.flavour = (h.light >> 1) & 1;
+            l.smem_bytes = imp_blur_dyn_smem(h.sc, h.blur_r, ops16, h.tile_rs);
+            l.ctas_per_job = ((h.bw + IMP_BLUR_TW - 1) / IMP_BLUR_TW) * ((h.bh + IMP_BLUR_TH - 1) / IMP_BLUR_TH);    // same count in destination space
+            break;
+        case ImpKernel::CubicTile:
+            l.param = h.gt;
+            l.flavour = h.light & 1;
+            l.smem_bytes = imp_cubic_dyn_smem(h.sc, ops16, h.tile_rs, h.tile_rows, h.gt, h.dc);
+            l.ctas_per_job = ((h.bw + h.gt - 1) / h.gt) * ((h.bh + h.gt - 1) / h.gt);                          // same count in destination space
+            break;
+        case ImpKernel::GatherTile:
+            l.param = h.gt;
+            l.flavour = h.light & 1;
+            l.smem_bytes = imp_gather_dyn_smem(h.gt, ops16, h.tile_rs, h.tile_rows, h.dc);
+            l.ctas_per_job = (((h.bw + h.gt - 1) / h.gt) * ((h.bh + h.gt - 1) / h.gt) + IMP_GATHER_TPC - 1) / IMP_GATHER_TPC;   // IMP_GATHER_TPC tiles each
+            break;
+    }
+    return l;
+}
+
+void imp_pass_launches(const ImpPass& h, ImpLaunch* tiled, ImpLaunch* fallback) {
+    const ImpKernel fb = h.kind == IMP_G_CUBIC ? ImpKernel::CubicRun : h.kind == IMP_G_BLUR ? ImpKernel::BlurGeneric : ImpKernel::Direct;
+    ImpKernel k = fb;
+    if (h.tile_smem > 0) {
+        if (h.kind == IMP_G_CUBIC) k = ImpKernel::CubicTile;
+        else if (h.gt > 0) k = ImpKernel::GatherTile;
+        else if (h.kind == IMP_G_BLUR) k = h.blur_r > 0 ? ImpKernel::BlurTile : fb;
+        else if (h.kind != IMP_G_COPY && h.kind != IMP_G_NN) k = ImpKernel::Strip;
+    }
+    *fallback = imp_pass_launch(h, fb);
+    *tiled = imp_pass_launch(h, k);
+    if (tiled->smem_bytes > IMP_SMEM_OPTIN) *tiled = *fallback;
+}
+
 namespace {
 
 // ---- C-library-faithful helpers ---------------------------------------------------------------------
@@ -206,7 +266,7 @@ std::vector<int> gaussian_taps(double sigma) {
     return k;
 }
 
-// Strip-kernel tables for the plain gathers (imp_tiles.cuh, modes NN / LINEAR / COPY): per strip of 32 output columns the
+// Strip-kernel tables for shrinking INTER_LINEAR (imp_tiles.cuh, mode 3): per strip of 32 output columns the
 // first and last source pixel it touches, per tile of 8 output rows the first source row and the row count; the TMA box is
 // the largest such rectangle. x_lo/x_hi(bx), y_lo/y_hi(by): clamped source coordinates an output column / row reads.
 template <class FXL, class FXH, class FYL, class FYH>
@@ -358,6 +418,7 @@ struct Lower {
         hp.in_w = in_w; hp.in_h = in_h; hp.in_c = in_c;
         hp.out_w = out_w; hp.out_h = out_h; hp.out_c = hdr.dc;
         hp.uses_watermark = uses_wm; hp.sigma = sigma;
+        imp_pass_launches(hdr, &hp.tiled, &hp.fallback);
         plan->passes.push_back(std::move(hp));
     }
     // A Gaussian blur: close the running pass (stored in base orientation) and open a stencil pass.
@@ -827,13 +888,10 @@ int imp_build_plan(const imp_gpu_request* req, const imp_gpu_config* cfg, int w,
                     }
                 }
             } else {
-                // two candidates (A/B with IMP_GPU_LINEAR=strip|tile): the persistent strip kernel's mode 3 and the gather tile kernel
                 // shrinking reads a large source rectangle per output tile: the persistent strip kernel streams it through its
                 // TMA ring (cfg1l: 0.36 ms against 0.56 ms for one box per tile); enlarging reads a small one and is bound by
                 // the stores, which the tile kernel issues 16 bytes at a time
-                static const int force = [] { const char* e = getenv("IMP_GPU_LINEAR"); return !e ? 0 : !strcmp(e, "strip") ? 1 : !strcmp(e, "tile") ? 2 : 0; }();
-                const bool strip = force ? force == 1 : (scale_x > 1.25 || scale_y > 1.25);
-                if (strip)
+                if (scale_x > 1.25 || scale_y > 1.25)
                     gather_strip_tables(L.bb, P, c, [&](int x) { return clampi(xo[x], 0, cw - 1); }, [&](int x) { return clampi(xo[x] + 1, 0, cw - 1); },
                                         [&](int y) { return clampi(yo[y], 0, ch - 1); }, [&](int y) { return clampi(yo[y] + 1, 0, ch - 1); });
                 else
@@ -852,7 +910,7 @@ int imp_build_plan(const imp_gpu_request* req, const imp_gpu_config* cfg, int w,
         if (code) return code;
     }
 
-    // a pass 0 that stayed a plain index map (crop / no resize) streams through the strip kernel as well
+    // a pass 0 that stayed a plain index map (crop / no resize) takes the gather tile kernel as well
     if (!dry && L.hdr.kind == IMP_G_COPY) L.copy_tables();
 
     // step 6: watermark (bridge.c:629-640, 239-281)

@@ -4,7 +4,7 @@
 //
 // The direct-from-global kernels in imp_kernels.cu remain the general path (any pitch/alignment, any
 // footprint); these are selected per job when the source rows are 16-byte addressable
-// (imp_tile_eligible) and the footprint fits the shared-memory budget.
+// (pick_launch, imp_gpu.cu) and the footprint fits the shared-memory budget.
 #pragma once
 #include "imp_gather.cuh"
 
@@ -356,11 +356,11 @@ __device__ __forceinline__ void area_int_strip_consume(const ImpJob& job, const 
     }
 }
 
-// Plain-gather consumers of the strip kernel (modes 2 = INTER_NN, 3 = INTER_LINEAR, 4 = index map / crop): the same TMA ring,
-// one output row per warp, but the pixel comes from one (NN, COPY) or 2x2 (LINEAR) staged source pixels. The per-column
-// part of the gather (source offset, x coefficients) is loaded once per strip.
-template <int SC, int MODE, int FL>
-__device__ __forceinline__ void gather_strip_consume(const ImpJob& job, const ImpPass* __restrict__ P, const uint8_t* __restrict__ blob,
+// INTER_LINEAR consumer of the strip kernel (mode 3; shrinking only, the gather tile kernel enlarges): the same TMA ring,
+// one output row per warp, each pixel from 2x2 staged source pixels. The per-column part of the gather (source offsets,
+// x coefficients) is loaded once per strip.
+template <int SC, int FL>
+__device__ __forceinline__ void linear_strip_consume(const ImpJob& job, const ImpPass* __restrict__ P, const uint8_t* __restrict__ blob,
                                                      const uint8_t* tile0, int stage_bytes, uint64_t* full, uint64_t* empty,
                                                      const uint8_t* s_ops, int nops, int bx0, int col_off, int tiles_y, int NSTAGE) {
     const int bw = P->bw, bh = P->bh, sw = P->sw, sh = P->sh, rs = P->tile_rs, oc = P->oc, dc = P->dc;
@@ -369,15 +369,10 @@ __device__ __forceinline__ void gather_strip_consume(const ImpJob& job, const Im
     const int bx = min(bx0 + lane, bw - 1);
     const int* __restrict__ yofs = reinterpret_cast<const int*>(blob + P->yofs_off);
     const int4* __restrict__ ytile = reinterpret_cast<const int4*>(blob + P->ytile_off);
-    int xo0 = 0, xo1 = 0, a0 = 0, a1 = 0;
-    if (MODE == 2) xo0 = col_off + __ldg(reinterpret_cast<const int*>(blob + P->xofs_off) + bx) * SC;
-    else if (MODE == 4) xo0 = col_off + bx * SC;
-    else {
-        const int xs = __ldg(reinterpret_cast<const int*>(blob + P->xofs_off) + bx);
-        xo0 = col_off + min(max(xs, 0), sw - 1) * SC; xo1 = col_off + min(max(xs + 1, 0), sw - 1) * SC;
-        const short* xa = reinterpret_cast<const short*>(blob + P->xcoef_off);
-        a0 = __ldg(xa + bx * 2); a1 = __ldg(xa + bx * 2 + 1);
-    }
+    const int xs = __ldg(reinterpret_cast<const int*>(blob + P->xofs_off) + bx);
+    const int xo0 = col_off + min(max(xs, 0), sw - 1) * SC, xo1 = col_off + min(max(xs + 1, 0), sw - 1) * SC;
+    const short* xa = reinterpret_cast<const short*>(blob + P->xcoef_off);
+    const int a0 = __ldg(xa + bx * 2), a1 = __ldg(xa + bx * 2 + 1);
     const StripStore st = strip_store_line(P->out, job.dst, job.dst_pitch, dc, bx);
     const StripOpsRows orows = strip_ops_rows(s_ops, nops, bx);
     int stage = 0, phase = 0;
@@ -386,46 +381,29 @@ __device__ __forceinline__ void gather_strip_consume(const ImpJob& job, const Im
         const int by = min(t * TH + warp, bh - 1);
         const bool in_y = t * TH + warp < bh;
         const int row0 = __ldg(ytile + t).x;                            // first source row staged for this tile
-        int r0, r1 = 0, b0 = 0, b1 = 0;
-        if (MODE == 2) r0 = __ldg(yofs + by) - row0;
-        else if (MODE == 4) r0 = by - row0;
-        else {
-            const int ys = __ldg(yofs + by);
-            r0 = min(max(ys, 0), sh - 1) - row0; r1 = min(max(ys + 1, 0), sh - 1) - row0;
-            const short* yb = reinterpret_cast<const short*>(blob + P->ycoef_off);
-            b0 = __ldg(yb + by * 2); b1 = __ldg(yb + by * 2 + 1);
-        }
+        const int ys = __ldg(yofs + by);
+        const int r0 = min(max(ys, 0), sh - 1) - row0, r1 = min(max(ys + 1, 0), sh - 1) - row0;
+        const short* yb = reinterpret_cast<const short*>(blob + P->ycoef_off);
+        const int b0 = __ldg(yb + by * 2), b1 = __ldg(yb + by * 2 + 1);
         mbar_wait_a(full_a + stage * 8, phase);
         const uint8_t* sbase = tile0 + stage * stage_bytes;
         int v[SC];
-        IMP_DBG(r0 >= 0 && r0 < P->tile_rows && xo0 >= 0 && xo0 + SC <= rs && (MODE != 3 || (r1 >= 0 && r1 < P->tile_rows && xo1 >= 0 && xo1 + SC <= rs)), 10);
-        if (MODE == 3) {
-            const uint8_t* q0 = sbase + r0 * rs; const uint8_t* q1 = sbase + r1 * rs;
-            int p00[SC], p01[SC], p10[SC], p11[SC];
-            if (SC == 4) {
-                const uint32_t w00 = *reinterpret_cast<const uint32_t*>(q0 + xo0), w01 = *reinterpret_cast<const uint32_t*>(q0 + xo1);
-                const uint32_t w10 = *reinterpret_cast<const uint32_t*>(q1 + xo0), w11 = *reinterpret_cast<const uint32_t*>(q1 + xo1);
+        IMP_DBG(r0 >= 0 && r0 < P->tile_rows && xo0 >= 0 && xo0 + SC <= rs && (r1 >= 0 && r1 < P->tile_rows && xo1 >= 0 && xo1 + SC <= rs), 10);
+        const uint8_t* q0 = sbase + r0 * rs; const uint8_t* q1 = sbase + r1 * rs;
+        int p00[SC], p01[SC], p10[SC], p11[SC];
+        if (SC == 4) {
+            const uint32_t w00 = *reinterpret_cast<const uint32_t*>(q0 + xo0), w01 = *reinterpret_cast<const uint32_t*>(q0 + xo1);
+            const uint32_t w10 = *reinterpret_cast<const uint32_t*>(q1 + xo0), w11 = *reinterpret_cast<const uint32_t*>(q1 + xo1);
 #pragma unroll
-                for (int c = 0; c < SC; c++) { p00[c] = (w00 >> (8 * c)) & 255; p01[c] = (w01 >> (8 * c)) & 255; p10[c] = (w10 >> (8 * c)) & 255; p11[c] = (w11 >> (8 * c)) & 255; }
-            } else {
-#pragma unroll
-                for (int c = 0; c < SC; c++) { p00[c] = q0[xo0 + c]; p01[c] = q0[xo1 + c]; p10[c] = q1[xo0 + c]; p11[c] = q1[xo1 + c]; }
-            }
-#pragma unroll
-            for (int c = 0; c < SC; c++) {                              // SURVEY App. A.4 / imp_gather_linear
-                const int h0 = p00[c] * a0 + p01[c] * a1, h1 = p10[c] * a0 + p11[c] * a1;
-                v[c] = ((((b0 * (h0 >> 4)) >> 16) + ((b1 * (h1 >> 4)) >> 16) + 2) >> 2) & 255;
-            }
+            for (int c = 0; c < SC; c++) { p00[c] = (w00 >> (8 * c)) & 255; p01[c] = (w01 >> (8 * c)) & 255; p10[c] = (w10 >> (8 * c)) & 255; p11[c] = (w11 >> (8 * c)) & 255; }
         } else {
-            const uint8_t* q = sbase + r0 * rs + xo0;
-            if (SC == 4) {
-                const uint32_t w = *reinterpret_cast<const uint32_t*>(q);
 #pragma unroll
-                for (int c = 0; c < SC; c++) v[c] = (w >> (8 * c)) & 255;
-            } else {
+            for (int c = 0; c < SC; c++) { p00[c] = q0[xo0 + c]; p01[c] = q0[xo1 + c]; p10[c] = q1[xo0 + c]; p11[c] = q1[xo1 + c]; }
+        }
 #pragma unroll
-                for (int c = 0; c < SC; c++) v[c] = q[c];
-            }
+        for (int c = 0; c < SC; c++) {                                  // SURVEY App. A.4 / imp_gather_linear
+            const int h0 = p00[c] * a0 + p01[c] * a1, h1 = p10[c] * a0 + p11[c] * a1;
+            v[c] = ((((b0 * (h0 >> 4)) >> 16) + ((b1 * (h1 >> 4)) >> 16) + 2) >> 2) & 255;
         }
         // every lane's loads must have been performed before lane 0 hands the stage back to the TMA producer
         fence_generic_to_async_smem();
@@ -513,8 +491,8 @@ imp_strip_kernel(const ImpJob* __restrict__ jobs, int first, int count, const __
     // ---- consumers ----
     const int col_off = job.tm_x0 - c0 * 8;                           // tile byte offset of source pixel 0
     const int bx0 = blockIdx.x * TW;
-    if constexpr (MODE >= 2) {
-        gather_strip_consume<SC, MODE, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE);
+    if constexpr (MODE == 3) {
+        linear_strip_consume<SC, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE);
     } else if constexpr (MODE == 0) {
         switch (P->max_xtaps) {                                       // uniform over the pass
         case 1: area_strip_consume<SC, 1, 0, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;

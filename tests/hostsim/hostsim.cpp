@@ -100,3 +100,9 @@ extern "C" void hostsim_plan_tile_info(const imp_gpu_plan* p, int k, int* out) {
     const ImpPass& h = p->passes[k].hdr;
     out[0] = h.tile_rs; out[1] = h.tile_rows; out[2] = h.tile_smem; out[3] = h.max_xtaps; out[4] = h.max_ytaps; out[5] = h.kind;
 }
+// the launch a job of pass k takes (ImpHostPass::tiled when its source rows are 16-byte addressable, else ::fallback):
+// kernel (ImpKernel), param, flavour, ctas_per_job, smem_bytes, ctas_per_sm
+extern "C" void hostsim_plan_launch(const imp_gpu_plan* p, int k, int tiled, int* out) {
+    const ImpLaunch& l = tiled ? p->passes[k].tiled : p->passes[k].fallback;
+    out[0] = (int)l.kernel; out[1] = l.param; out[2] = l.flavour; out[3] = l.ctas_per_job; out[4] = l.smem_bytes; out[5] = l.ctas_per_sm;
+}

@@ -235,6 +235,41 @@ def test_batch_mixed_plans_one_launch_per_variant(gpu, orc):
         _assert_same(out, _oracle(orc, img, rq, kw)[2], rq, False)
 
 
+def test_run_device_matches_oracle(gpu, orc):
+    """imp_gpu_run_device: one frame in device buffers through the batch's launch steps, every job passed by value and the
+    scratch allocated on the stream. A strip pass (cfg2's request, reduced), a gather tile pass, a multi-pass chain through
+    scratch, a blur beyond the tile kernel's radius (two launches through the u16 plane) and a source whose pitch is not a
+    multiple of 16 (a pass-0 blur then takes the two-launch path as well)."""
+    L = gpu.lib
+    kw = dict(allow_experiments=True, max_filters=8)
+    kw_wm = dict(kw, watermark=rnd_image(3, 16, 64, 4), wm_gravity_x="r", wm_gravity_y="b", wm_offset_x=10, wm_offset_y=10, wm_opacity=60)
+    cases = [(smooth_image(1, 540, 960, 4), kw_wm, dict(crop="900px,506px,c,c", resize="200,112"), 0),
+             (smooth_image(2, 300, 400, 3), kw, dict(filters=["rotate=90"]), 0),
+             (smooth_image(3, 120, 160, 3), kw, dict(resize="100,75", filters=["blur=2", "kelvin=1", "blur=0.7"]), 0),
+             (smooth_image(4, 120, 160, 4), kw, dict(filters=["blur=6"]), 0),
+             (smooth_image(5, 135, 240, 3), kw, dict(filters=["blur=2.3", "gamma=1.2"]), 5)]
+    for img, cfgkw, rq, pad in cases:
+        h, w, c = img.shape
+        p = gpu.plan(w, h, c, api.Config(**cfgkw), **rq)
+        d_in, d_out, pi, po = C.c_void_p(), C.c_void_p(), C.c_int(), C.c_int()
+        if pad:
+            sp = w * c + pad
+            gpu.check(L.imp_gpu_malloc_pitch(C.byref(d_in), C.byref(pi), sp * h, 1))
+        else:
+            gpu.check(L.imp_gpu_malloc_pitch(C.byref(d_in), C.byref(pi), w * c, h))
+            sp = pi.value
+        gpu.check(L.imp_gpu_malloc_pitch(C.byref(d_out), C.byref(po), p.out_w * p.out_c, p.out_h))
+        gpu.check(L.imp_gpu_upload_2d(d_in, sp, img.ctypes.data, img.strides[0], w * c, h, None))
+        before = gpu.launch_count()
+        p.run_device(d_in.value, sp, d_out.value, po.value)
+        out = np.empty((p.out_h, p.out_w, p.out_c), np.uint8)
+        gpu.check(L.imp_gpu_download_2d(out.ctypes.data, out.strides[0], d_out, po.value, p.out_w * p.out_c, p.out_h, None))
+        gpu.check(L.imp_gpu_sync(None))
+        assert gpu.launch_count() - before >= p.passes, rq
+        L.imp_gpu_free(d_in); L.imp_gpu_free(d_out); p.close()
+        _assert_same(out, _oracle(orc, img, rq, cfgkw)[2], rq, False)
+
+
 def test_host_batch_and_farm_match_single_runs(gpu, orc):
     kw = dict(max_w=0, max_h=0)
     imgs = [smooth_image(i, 300 + 7 * i, 400 + 5 * i, 3 if i % 3 else 4) for i in range(9)]

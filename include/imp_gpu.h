@@ -22,6 +22,8 @@
  *                                          concurrent requests: one fused launch per kernel variant
  *   imp_gpu_farm_run_host                  independent frames sharded round-robin over the GPUs of
  *                                          one box (no collective: nothing crosses GPUs)
+ *   imp_gpu_batch_brightness_host /        Info (bridge.c:283-300) and ASCII (filters.c:486-522) after the frame loops:
+ *   imp_gpu_batch_ascii_host               the brightness or the text comes back, not the frame
  * The reference-signature operator layer (Crop/Resize/Filter/Watermark/BlendWithPaper on IplImage)
  * is declared in imp_ops.h and is implemented on top of this ABI.
  */
@@ -197,15 +199,30 @@ int  imp_gpu_farm_run_host_policy(int n, imp_gpu_plan* const* plans, const unsig
                                   const int* src_steps, unsigned char* const* dsts, const int* dst_steps,
                                   int n_gpus, int n_streams, int policy);
 
-/* ---- first "next" row (SURVEY 8f-1): CalcPerceivedBrightness (filters.c:707-729) as a device reduction -------- */
-/* What Info() (bridge.c:283-300) prints as round(brightness*100). The reference accumulates float32 in column-major
- * order; the device sums in double, so values agree to ~1e-5 relative and the JSON integer is compared in the tests. */
+/* ---- format=json / format=text: an answer instead of the frame (SURVEY 8f-1, 8f-4) ------------------------------- */
+/* format=json / format=text (bridge.c:659-677) for n jobs without their frames leaving the device: job i runs plans[i]
+ * on srcs[i] exactly as imp_gpu_batch_run_host would, then brightness[i] = CalcPerceivedBrightness of the result
+ * (filters.c:707-729; double sum, deterministic: the same frame gives the same bits whatever the batch, chunking or
+ * n_streams), or texts[i] receives ASCII of the result (filters.c:486-522; args[i] as the reference takes it, NULL = the
+ * 10-level ramp), imp_gpu_ascii_length(out_w, out_h) bytes. Synchronous, on the current device.
+ * Each chunk of jobs costs one launch more than imp_gpu_batch_run_host, and only the floats or the texts cross the bus.
+ * Every job is checked first; IMP_ERROR_INVALID_ARGS, with nothing written, for a NULL array or plan, a plan whose request
+ * packs the result for FreeImage (pack != IMP_PACK_NONE: bottom-up rows would reverse the text) or text_caps[i] smaller
+ * than the text. n == 0: IMP_OK. */
+int  imp_gpu_batch_brightness_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                                   float* brightness, int n_streams);
+int  imp_gpu_batch_ascii_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                              const char* const* args, unsigned char* const* texts, const long* text_caps, int n_streams);
+
+/* One frame already decoded: what Info() (bridge.c:283-300) prints as round(brightness*100). The reference accumulates
+ * float32 in column-major order; the device sums in double (the same reduction as the batch call, so a frame gives the same
+ * bits here as there when its rows are 16-byte aligned: the host form stages them so), and the values agree to ~1e-5
+ * relative. Any base and pitch are accepted on the device. */
 int  imp_gpu_brightness_device(const void* d_img, int pitch, int width, int height, int channels, float* brightness, void* stream);
 int  imp_gpu_brightness_host(const unsigned char* img, int step, int width, int height, int channels, float* brightness);
 
-/* ---- SURVEY 8f-4: ASCII (filters.c:486-522, format=text) on the device -------------------------------------------- */
-/* `args` as the reference takes it ("wide" selects the 70-level ramp, anything else the 10-level one). Writes
- * (width+1)*height-1 bytes: one character per pixel, rows separated by '\n'. The frame itself is not modified (the
+/* ASCII of one frame. `args` as the reference takes it ("wide" selects the 70-level ramp, anything else the 10-level one).
+ * Writes (width+1)*height-1 bytes: one character per pixel, rows separated by '\n'. The frame itself is not modified (the
  * reference converts it to HSV in place, filters.c:504, which nothing reads afterwards). */
 long imp_gpu_ascii_length(int width, int height);
 int  imp_gpu_ascii_host(const unsigned char* img, int step, int width, int height, int channels, const char* args,

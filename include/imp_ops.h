@@ -19,6 +19,7 @@
  *   void BlendWithPaper(IplImage*)           filters.c:666 imp_BlendWithPaper
  *   gray->BGR block                          bridge.c:613-618  implicit (a 1-channel frame leaves imp_Flush as BGR, also when nothing was recorded)
  *   (none)                                   before bridge.c:659   imp_Flush / imp_FlushAll
+ *   CalcPerceivedBrightness / ASCII          bridge.c:296, 668     imp_Brightness / imp_Ascii (the frame stays on the device)
  *   LoadGIF's canvas loop                    advancedio.c:195-248  imp_FlushAllGif (pages expanded on the device; imp_AlbumGifPage in the drop-in)
  *   cvReleaseImage on an error path          bridge.c:714-722  imp_Discard first
  *
@@ -79,6 +80,12 @@ int  imp_FlushAll(IplImage** frames, int count);
  * recorded just receives its canvas). n_pages == count: frame i is page i. count == 1 < n_pages: LoadGIF's `page`
  * request (:264-272) — the frame is the LAST page, the earlier ones are only replayed for their disposal. */
 int  imp_FlushAllGif(IplImage** frames, int count, const imp_gpu_gif_frame* pages, int n_pages, int destructive);
+/* Brightness / ASCII of what imp_Flush would leave in `image`, computed on the device; the frame is not brought back.
+ * What was recorded for `image` STAYS recorded: a later imp_Flush still produces the pixels, imp_Discard still works.
+ * A 1-channel frame is answered as BGR, recorded operators or not (imp_Flush promotes it, bridge.c:613-618). `args` and
+ * out_cap as imp_gpu_ascii_host takes them. Returns IMP_OK, IMP_ERROR_INVALID_ARGS or IMP_ERROR_GPU. */
+int  imp_Brightness(IplImage* image, float* brightness);
+int  imp_Ascii(IplImage* image, const char* args, unsigned char* out, long out_cap);
 /* Forget anything recorded for `image` (call before releasing a frame that was never flushed). */
 void imp_Discard(IplImage* image);
 /* Number of operations currently recorded for `image` (0 = pixels are up to date). */

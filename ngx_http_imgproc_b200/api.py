@@ -142,6 +142,10 @@ class Library:
         L.imp_gpu_sync.argtypes = [C.c_void_p]
         L.imp_gpu_brightness_host.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float)]
         L.imp_gpu_brightness_device.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.c_void_p]
+        L.imp_gpu_ascii_length.restype = C.c_long
+        L.imp_gpu_ascii_length.argtypes = [C.c_int, C.c_int]
+        L.imp_gpu_batch_brightness_host.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
+        L.imp_gpu_batch_ascii_host.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
 
     # ---- lifetime ---------------------------------------------------------------------------------
     def last_error(self) -> str:
@@ -218,6 +222,28 @@ class Library:
         out = C.c_float(0)
         self.check(self.lib.imp_gpu_brightness_host(img.ctypes.data, img.strides[0], img.shape[1], img.shape[0], img.shape[2], C.byref(out)))
         return float(out.value)
+
+    # ---- answers instead of frames: format=json / format=text over a batch ----------------------------
+    def batch_brightness(self, plans: List["Plan"], srcs: List[np.ndarray], n_streams: int = 4) -> np.ndarray:
+        """imp_gpu_batch_brightness_host: job i runs plans[i] on srcs[i]; CalcPerceivedBrightness of each result (float32)."""
+        n = len(plans)
+        P, S, SS = _job_arrays(plans, srcs)
+        out = np.zeros(n, np.float32)
+        self.check(self.lib.imp_gpu_batch_brightness_host(n, P, S, SS, out.ctypes.data, n_streams))
+        return out
+
+    def batch_ascii(self, plans: List["Plan"], srcs: List[np.ndarray], args=None, n_streams: int = 4) -> List[bytes]:
+        """imp_gpu_batch_ascii_host: ASCII of each result. `args`: one value for every job or a list (None: 10-level ramp)."""
+        n = len(plans)
+        P, S, SS = _job_arrays(plans, srcs)
+        args = list(args) if isinstance(args, (list, tuple)) else [args] * n
+        A = (C.c_char_p * max(n, 1))(*[None if a is None else a.encode() for a in args])
+        lens = [self.lib.imp_gpu_ascii_length(p.out_w, p.out_h) for p in plans]
+        bufs = [C.create_string_buffer(max(k, 1)) for k in lens]
+        T = (C.c_void_p * max(n, 1))(*[C.addressof(b) for b in bufs])
+        caps = (C.c_long * max(n, 1))(*lens)
+        self.check(self.lib.imp_gpu_batch_ascii_host(n, P, S, SS, A, T, caps, n_streams))
+        return [b.raw[:k] for b, k in zip(bufs, lens)]
 
     # ---- plans --------------------------------------------------------------------------------------
     def plan(self, w, h, c, cfg: Optional[Config] = None, **req) -> "Plan":
@@ -307,6 +333,12 @@ class Batch:
 
 
 FARM_ROUND_ROBIN, FARM_SIZE_AWARE = 0, 1
+
+
+def _job_arrays(plans, srcs):
+    n = max(len(plans), 1)
+    return ((C.c_void_p * n)(*[p.h for p in plans]), (C.c_void_p * n)(*[s.ctypes.data for s in srcs]),
+            (C.c_int * n)(*[s.strides[0] for s in srcs]))
 
 
 class HostJobs:
@@ -419,6 +451,9 @@ class OpsLayer:
         L.imp_FlushAll.argtypes = [PP, C.c_int]
         L.imp_FlushAllGif.argtypes = [PP, C.c_int, C.c_void_p, C.c_int, C.c_int]
         L.imp_Discard.argtypes = [C.POINTER(IplImage)]
+        L.imp_Brightness.argtypes = [C.POINTER(IplImage), C.POINTER(C.c_float)]
+        L.imp_Ascii.argtypes = [C.POINTER(IplImage), C.c_char_p, C.c_void_p, C.c_long]
+        L.imp_ops_pending.argtypes = [C.POINTER(IplImage)]
         self.keep = []
         self._cb = (self.CREATE_T(self._create), self.RELEASE_T(self._release))
         L.imp_ops_set_image_allocator.argtypes = [self.CREATE_T, self.RELEASE_T]
@@ -447,18 +482,16 @@ class OpsLayer:
     def _release(self, pp):
         pp[0] = None
 
-    def request(self, frames, cfg: Config, crop=None, gravity=None, resize=None, filters=(), simple=False, flatten=False, gif_pages=None, destructive=False):
-        """Steps 3-7 of RunJob over `frames` (numpy images): returns (code, list of results or None).
-        gif_pages (dicts as Library.gif_pages takes them): `frames` are only canvas-sized 4-channel placeholders whose pixels
-        are never read; the flush is imp_FlushAllGif (pages expanded on the device)."""
+    def record(self, frames, cfg: Config, crop=None, gravity=None, resize=None, filters=(), simple=False, flatten=False):
+        """The per-frame operator calls of RunJob (bridge.c:576-656) over `frames` (numpy images), nothing run yet.
+        Returns (code, IplImage pointers or None); on an error everything recorded is discarded."""
         L = self.L.lib
         self.keep = []
         ccfg, keep = cfg.to_c()
         enc = lambda t: None if t is None else t.encode("latin-1")
-        hdrs = [self.header(f) for f in frames]
-        ptrs = [C.pointer(h) for h in hdrs]
+        ptrs = [C.pointer(self.header(f)) for f in frames]
         code = 0
-        for p in ptrs:                                                   # the per-frame loops of bridge.c:576-656
+        for p in ptrs:
             if crop is not None and not code: code = L.imp_Crop(C.byref(p), enc(crop), enc(gravity))
             if resize is not None and not code: code = L.imp_Resize(C.byref(p), enc(resize), C.byref(ccfg), 1 if simple else 0)
             for f in filters:
@@ -467,6 +500,46 @@ class OpsLayer:
             if flatten and not code: code = L.imp_BlendWithPaper(p)
         if code:
             for p in ptrs: L.imp_Discard(p)
+            return code, None
+        return 0, ptrs
+
+    def brightness(self, frames, cfg: Config, **req):
+        """Records like request() and returns (code, [imp_Brightness of each frame] or None); the recording is then discarded."""
+        code, ptrs = self.record(frames, cfg, **req)
+        if code:
+            return code, None
+        out, v = [], C.c_float()
+        for p in ptrs:
+            if not code:
+                code = self.L.lib.imp_Brightness(p, C.byref(v))
+                out.append(float(v.value))
+            self.L.lib.imp_Discard(p)
+        return (code, None) if code else (0, out)
+
+    def ascii(self, frames, cfg: Config, args=None, **req):
+        """Records like request() and returns (code, [imp_Ascii of each frame] or None); the recording is then discarded."""
+        code, ptrs = self.record(frames, cfg, **req)
+        if code:
+            return code, None
+        out = []
+        for p in ptrs:
+            if not code:
+                im = p.contents                                          # the header describes the result the flush would leave
+                w, h = (im.width, im.height)
+                n = self.L.lib.imp_gpu_ascii_length(w, h)
+                buf = C.create_string_buffer(max(n, 1))
+                code = self.L.lib.imp_Ascii(p, None if args is None else args.encode(), buf, n)
+                out.append(buf.raw[:n])
+            self.L.lib.imp_Discard(p)
+        return (code, None) if code else (0, out)
+
+    def request(self, frames, cfg: Config, crop=None, gravity=None, resize=None, filters=(), simple=False, flatten=False, gif_pages=None, destructive=False):
+        """Steps 3-7 of RunJob over `frames` (numpy images): returns (code, list of results or None).
+        gif_pages (dicts as Library.gif_pages takes them): `frames` are only canvas-sized 4-channel placeholders whose pixels
+        are never read; the flush is imp_FlushAllGif (pages expanded on the device)."""
+        L = self.L.lib
+        code, ptrs = self.record(frames, cfg, crop, gravity, resize, filters, simple, flatten)
+        if code:
             return code, None
         arr = (C.POINTER(IplImage) * len(ptrs))(*ptrs)
         if gif_pages is not None:

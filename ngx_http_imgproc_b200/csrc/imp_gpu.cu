@@ -103,6 +103,8 @@ struct Lane {            // one in-flight chunk of host jobs of the end-to-end p
     Buf d_in, d_out, d_stage;                    // device: re-pitched crop windows, results, linear landing zone of short rows
     Buf h_in, h_out;                             // pinned staging for host buffers that are not page-locked
     imp_gpu_batch batch;                         // the chunk's job table, scratch and tensor maps
+    Buf d_info, h_info;                          // brightness / ASCII: job table, partial sums, answers, texts; the table's pinned staging
+    Buf d_tickets;                               // brightness: one ticket per job of a chunk, zeroed once (the kernel leaves them 0)
     struct Out { int job; long long staged_off; };   // staged_off >= 0: copy from h_out after the sync
     std::vector<Out> pend;
 };
@@ -522,7 +524,18 @@ struct HostJobs {
     int n; imp_gpu_plan* const* plans; const unsigned char* const* srcs; const int* src_steps;
     unsigned char* const* dsts; const int* dst_steps;
     bool src_device = false;       // srcs[] are whole frames already on this device (pitch % 16 == 0): nothing to upload
+    // What comes back: the frames (dsts), or one more launch per chunk reduces the results on the device and only its
+    // answers come back: brightness[i], or texts[i] (ASCII with the 70-level ramp where wide[i]).
+    enum Result { Frame, Brightness, Ascii } result = Frame;
+    float* brightness = nullptr;
+    unsigned char* const* texts = nullptr; const unsigned char* wide = nullptr;
 };
+
+// The answer of job i when it is not a frame: where it goes on the host and its size.
+uint8_t* answer_dst(const HostJobs& J, int i) { return J.result == HostJobs::Ascii ? J.texts[i] : reinterpret_cast<uint8_t*>(J.brightness + i); }
+size_t answer_bytes(const HostJobs& J, int i) {
+    return J.result == HostJobs::Ascii ? (size_t)imp_gpu_ascii_length(J.plans[i]->out_w, J.plans[i]->out_h) : sizeof(float);
+}
 
 bool is_pinned(const void* p) {
     cudaPointerAttributes a;
@@ -642,7 +655,15 @@ template <class F> void run_parts(int n, int parts, F fn) {
 int lane_finish(Lane& L, const HostJobs& J) {
     if (L.pend.empty()) return IMP_OK;
     cudaError_t e = cudaStreamSynchronize(L.st);
-    if (e == cudaSuccess) {
+    if (e == cudaSuccess && J.result != HostJobs::Frame) {
+        std::vector<const Lane::Out*> staged; size_t bytes = 0;
+        for (const Lane::Out& o : L.pend) if (o.staged_off >= 0) { staged.push_back(&o); bytes += answer_bytes(J, o.job); }
+        const Lane::Out* const* sg = staged.data();
+        const uint8_t* h_out = L.h_out.p;
+        run_parts((int)staged.size(), stage_parts(bytes, (int)staged.size()), [=, &J](int k0, int k1) {
+            for (int k = k0; k < k1; k++) copy_stream(answer_dst(J, sg[k]->job), h_out + sg[k]->staged_off, answer_bytes(J, sg[k]->job));
+        });
+    } else if (e == cudaSuccess) {
         // results for pageable destinations (the frames cvCreateImage hands out) leave the pinned staging here; a 200-frame GIF
         // is 400 MB of it
         const uint8_t* h_out = L.h_out.p;
@@ -675,6 +696,68 @@ int lane_finish(Lane& L, const HostJobs& J) {
     return IMP_OK;
 }
 
+// The 256-entry ramps of ASCII (filters.c:486-522), derived with the reference's float maths (filters.c:496,509).
+const ImpAsciiRamps& ascii_ramps() {
+    static const ImpAsciiRamps r = [] {
+        static const char kWide[] = "$@B%8&WM#*oahkbdpqwmZO0QLCJUYXzcvunxrjft/\\|()1{}[]?-_+~<>i!lI;:,\"^`'. ";   // filters.c:486-487
+        static const char kNarrow[] = "@%8#*+=-:. ";
+        ImpAsciiRamps t;
+        for (int wide = 0; wide < 2; wide++) {
+            const char* table = wide ? kWide : kNarrow;
+            const float factor = 256.0 / (int)strlen(table);
+            for (int v = 0; v < 256; v++) t.lut[wide][v] = (uint8_t)table[(int)floor((double)((float)v / factor))];
+        }
+        return t;
+    }();
+    return r;
+}
+
+// Brightness / ASCII of the chunk's m results (out_off / out_pitch in L.d_out): ONE launch over all of them, then only the
+// answers cross the link — straight into pinned destinations, into h_out at staged[k] >= 0 otherwise (lane_finish copies on).
+int lane_answers(Lane& L, const HostJobs& J, int first, int m, const std::vector<size_t>& out_off, const std::vector<int>& out_pitch,
+                 const std::vector<long long>& staged) {
+    const bool ascii = J.result == HostJobs::Ascii;
+    std::vector<ImpInfoJob> tab(m);
+    int parts = 0, max_ctas = 1;
+    size_t text_total = 0;
+    for (int k = 0; k < m; k++) {
+        const imp_gpu_plan* p = J.plans[first + k];
+        ImpInfoJob& q = tab[k];
+        q = ImpInfoJob{};
+        q.img = L.d_out.p + out_off[k]; q.pitch = out_pitch[k];          // 256-byte aligned slot, 16-byte pitch
+        q.w = p->out_w; q.h = p->out_h; q.c = p->out_c; q.vec = 1;
+        if (ascii) {
+            q.ctas = imp_ascii_ctas(q.w, q.h); q.wide = J.wide[first + k] ? 1 : 0;
+            q.text_off = (long long)text_total; text_total += align256(answer_bytes(J, first + k));
+        } else {
+            q.ctas = imp_brightness_ctas(q.w, q.h); q.part_off = parts; parts += q.ctas;
+        }
+        max_ctas = std::max(max_ctas, q.ctas);
+    }
+    const size_t tab_bytes = align256(sizeof(ImpInfoJob) * m), part_bytes = align256(sizeof(double) * parts), ans_bytes = align256(sizeof(float) * m);
+    int r;
+    if ((r = L.d_info.grow(tab_bytes + part_bytes + ans_bytes + text_total, false)) || (r = L.h_info.grow(tab_bytes, true))) return r;
+    if (!ascii && !L.d_tickets.p) {
+        if ((r = L.d_tickets.grow(sizeof(unsigned) * kChunkJobs, false))) return r;
+        CK(cudaMemsetAsync(L.d_tickets.p, 0, L.d_tickets.cap, L.st));
+    }
+    memcpy(L.h_info.p, tab.data(), sizeof(ImpInfoJob) * m);
+    CK(cudaMemcpyAsync(L.d_info.p, L.h_info.p, sizeof(ImpInfoJob) * m, cudaMemcpyHostToDevice, L.st));
+    const ImpInfoJob* d_tab = reinterpret_cast<const ImpInfoJob*>(L.d_info.p);
+    uint8_t* d_ans = L.d_info.p + tab_bytes + part_bytes;
+    uint8_t* d_text = d_ans + ans_bytes;
+    if (ascii) CK(imp_launch_ascii(d_tab, tab[0], m, max_ctas, ascii_ramps(), d_text, L.st));
+    else CK(imp_launch_brightness(d_tab, tab[0], m, max_ctas, reinterpret_cast<double*>(L.d_info.p + tab_bytes),
+                                  reinterpret_cast<unsigned*>(L.d_tickets.p), reinterpret_cast<float*>(d_ans), L.st));
+    if (!ascii) CK(cudaMemcpyAsync(staged[0] >= 0 ? L.h_out.p + staged[0] : answer_dst(J, first), d_ans, sizeof(float) * m, cudaMemcpyDeviceToHost, L.st));
+    for (int k = 0; k < m; k++) {
+        const int i = first + k;
+        if (ascii) CK(cudaMemcpyAsync(staged[k] >= 0 ? L.h_out.p + staged[k] : answer_dst(J, i), d_text + tab[k].text_off, answer_bytes(J, i), cudaMemcpyDeviceToHost, L.st));
+        L.pend.push_back(Lane::Out{i, staged[k]});
+    }
+    return IMP_OK;
+}
+
 int lane_issue(Lane& L, const HostJobs& J, int first, int last) {
     const int m = last - first;
     struct Lay { size_t in_off, out_off, stage_off, hin_off; long long hout_off; int in_pitch, out_pitch; bool src_pinned, dst_pinned, linear; size_t lin_bytes; };
@@ -683,14 +766,16 @@ int lane_issue(Lane& L, const HostJobs& J, int first, int last) {
     for (int k = 0; k < m; k++) {
         const int i = first + k;
         imp_gpu_plan* p = J.plans[i];
-        if (!p || !J.srcs[i] || !J.dsts[i]) return IMP_ERROR_INVALID_ARGS;
+        const bool frame = J.result == HostJobs::Frame;
+        if (!p || !J.srcs[i] || (frame && !J.dsts[i])) return IMP_ERROR_INVALID_ARGS;
         Lay& l = lay[k];
         const size_t in_row = (size_t)p->win_w * p->src_c, out_row = (size_t)p->out_w * p->out_c;
         l.in_pitch = align16((int)in_row); l.out_pitch = align16((int)out_row);
         l.in_off = in_total;
         if (!J.src_device) in_total += align256((size_t)l.in_pitch * p->win_h);                       // landing zone of the crop window
         l.out_off = out_total; out_total += align256((size_t)l.out_pitch * p->out_h);
-        l.src_pinned = is_pinned(J.srcs[i]); l.dst_pinned = is_pinned(J.dsts[i]);
+        l.src_pinned = is_pinned(J.srcs[i]);
+        l.dst_pinned = frame ? is_pinned(J.dsts[i]) : J.result == HostJobs::Ascii ? is_pinned(J.texts[i]) : is_pinned(J.brightness + first);
         l.linear = false; l.lin_bytes = 0; l.stage_off = 0; l.hin_off = 0; l.hout_off = -1;
         if (J.src_device) {
             if ((reinterpret_cast<uintptr_t>(J.srcs[i]) & 15) || (J.src_steps[i] & 15) || (size_t)J.src_steps[i] < (size_t)p->src_w * p->src_c) return IMP_ERROR_INVALID_ARGS;
@@ -709,7 +794,11 @@ int lane_issue(Lane& L, const HostJobs& J, int first, int last) {
         } else {
             l.hin_off = hin_total; hin_total += align256((size_t)l.in_pitch * p->win_h);       // packed with the device pitch
         }
-        if (!l.dst_pinned) { l.hout_off = (long long)hout_total; hout_total += align256(out_row * p->out_h); }
+        if (!l.dst_pinned) {
+            l.hout_off = (long long)hout_total;
+            // brightness answers are staged back to back: the chunk's floats come back in one copy
+            hout_total += frame ? align256(out_row * p->out_h) : J.result == HostJobs::Ascii ? align256(answer_bytes(J, i)) : sizeof(float);
+        }
     }
     int r;
     if ((r = L.d_in.grow(in_total, false)) || (r = L.d_out.grow(out_total, false)) || (r = L.d_stage.grow(stage_total, false)) ||
@@ -770,6 +859,13 @@ int lane_issue(Lane& L, const HostJobs& J, int first, int last) {
     for (const Repitch& q : repitch) CK(imp_launch_repitch(q.src, q.sp, q.dst, q.dp, q.row_bytes, q.rows, L.st));
     if ((r = batch_compile(&B, L.st))) return r;
     if ((r = launch_steps(B.steps, B.h_jobs, B.d_jobs, L.st))) return r;
+    if (J.result != HostJobs::Frame) {
+        std::vector<size_t> out_off(m); std::vector<int> out_pitch(m);
+        for (int k = 0; k < m; k++) { out_off[k] = lay[k].out_off; out_pitch[k] = lay[k].out_pitch; }
+        std::vector<long long> staged(m);
+        for (int k = 0; k < m; k++) staged[k] = lay[k].dst_pinned ? -1 : lay[k].hout_off;
+        return lane_answers(L, J, first, m, out_off, out_pitch, staged);
+    }
     for (int k = 0; k < m; k++) {
         const int i = first + k;
         const imp_gpu_plan* p = J.plans[i];
@@ -919,6 +1015,7 @@ void imp_gpu_shutdown(void) {
             for (Lane* L : c.lanes) {
                 L->d_in.release(false); L->d_out.release(false); L->d_stage.release(false);
                 L->h_in.release(true); L->h_out.release(true);
+                L->d_info.release(false); L->h_info.release(true); L->d_tickets.release(false);
                 batch_release(&L->batch);
                 if (L->up_done) cudaEventDestroy(L->up_done);
                 if (L->st) cudaStreamDestroy(L->st);
@@ -1222,19 +1319,68 @@ int imp_gpu_farm_run_host(int n, imp_gpu_plan* const* plans, const unsigned char
     return imp_gpu_farm_run_host_policy(n, plans, srcs, src_steps, dsts, dst_steps, n_gpus, n_streams, IMP_FARM_ROUND_ROBIN);
 }
 
-// ---- "next" row §8f-1: perceived brightness as a device reduction ------------------------------------------
+// ---- format=json / format=text without the frames: brightness and ASCII of the results, reduced on the device ---------
+namespace {
+// Every job is checked before any work starts: nothing is written when one is unusable. A packed (bottom-up) result would
+// reverse the text, and the JSON and text exits never reach the FreeImage packer.
+int check_answer_jobs(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps) {
+    if (!plans || !srcs || !src_steps) return IMP_ERROR_INVALID_ARGS;
+    for (int i = 0; i < n; i++)
+        if (!plans[i] || !srcs[i] || plans[i]->pack != IMP_PACK_NONE) return IMP_ERROR_INVALID_ARGS;
+    return IMP_OK;
+}
+}  // namespace
+
+int imp_gpu_batch_brightness_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                                  float* brightness, int n_streams) {
+    int rc = bind(); if (rc) return rc;
+    if (n <= 0) return IMP_OK;
+    if ((rc = check_answer_jobs(n, plans, srcs, src_steps))) return rc;
+    if (!brightness) return IMP_ERROR_INVALID_ARGS;
+    HostJobs J{n, plans, srcs, src_steps, nullptr, nullptr};
+    J.result = HostJobs::Brightness; J.brightness = brightness;
+    try { return run_host_chunked(J, n_streams); } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+}
+
+int imp_gpu_batch_ascii_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                             const char* const* args, unsigned char* const* texts, const long* text_caps, int n_streams) {
+    int rc = bind(); if (rc) return rc;
+    if (n <= 0) return IMP_OK;
+    if ((rc = check_answer_jobs(n, plans, srcs, src_steps))) return rc;
+    if (!args || !texts || !text_caps) return IMP_ERROR_INVALID_ARGS;
+    for (int i = 0; i < n; i++)
+        if (!texts[i] || text_caps[i] < imp_gpu_ascii_length(plans[i]->out_w, plans[i]->out_h)) return IMP_ERROR_INVALID_ARGS;
+    try {
+        std::vector<unsigned char> wide(n);
+        for (int i = 0; i < n; i++) wide[i] = args[i] && strcmp(args[i], "wide") == 0;        // filters.c:490-494
+        HostJobs J{n, plans, srcs, src_steps, nullptr, nullptr};
+        J.result = HostJobs::Ascii; J.texts = texts; J.wide = wide.data();
+        return run_host_chunked(J, n_streams);
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+}
+
+// One frame: the batch kernels over a single job passed by value. Rows take the 16-byte path when base and pitch allow it.
 int imp_gpu_brightness_device(const void* d_img, int pitch, int w, int h, int c, float* brightness, void* stream) {
     int rc = bind(); if (rc) return rc;
     if (!d_img || !brightness || w <= 0 || h <= 0 || (c != 1 && c != 3 && c != 4)) return IMP_ERROR_INVALID_ARGS;
     cudaStream_t st = pick_stream(stream);
-    double* d_acc = nullptr;
-    CK(cudaMallocAsync((void**)&d_acc, sizeof(double), st));
-    CK(imp_launch_brightness((const uint8_t*)d_img, pitch, w, h, c, d_acc, st));
-    double sum = 0;
-    CK(cudaMemcpyAsync(&sum, d_acc, sizeof(double), cudaMemcpyDeviceToHost, st));
-    CK(cudaFreeAsync(d_acc, st));
-    CK(cudaStreamSynchronize(st));
-    *brightness = (float)(sum / ((double)w * h) / 255.0);          // filters.c:728
+    ImpInfoJob q{};
+    q.img = (const uint8_t*)d_img; q.pitch = pitch; q.w = w; q.h = h; q.c = c;
+    q.vec = (reinterpret_cast<uintptr_t>(d_img) % 16 == 0 && pitch % 16 == 0) ? 1 : 0;
+    q.ctas = imp_brightness_ctas(w, h);
+    const size_t part = align256(sizeof(double) * q.ctas);
+    uint8_t* d = nullptr;                                              // partials | ticket | answer
+    CK(cudaMallocAsync((void**)&d, part + 256, st));
+    unsigned* ticket = reinterpret_cast<unsigned*>(d + part);
+    float* d_ans = reinterpret_cast<float*>(d + part + 16);
+    float v = 0;
+    cudaError_t e = cudaMemsetAsync(ticket, 0, sizeof(unsigned), st);
+    if (e == cudaSuccess) e = imp_launch_brightness(nullptr, q, 1, q.ctas, reinterpret_cast<double*>(d), ticket, d_ans, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&v, d_ans, sizeof(float), cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(d, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(e, "brightness", __LINE__);
+    *brightness = v;
     return IMP_OK;
 }
 
@@ -1242,7 +1388,7 @@ int imp_gpu_brightness_host(const unsigned char* img, int step, int w, int h, in
     int rc = bind(); if (rc) return rc;
     if (!img || !brightness || w <= 0 || h <= 0 || (c != 1 && c != 3 && c != 4)) return IMP_ERROR_INVALID_ARGS;
     cudaStream_t st = g_dev[t_dev].stream;
-    const int pitch = align16(w * c);
+    const int pitch = align16(w * c);                                  // staged aligned: the 16-byte path, as on the batch path
     uint8_t* d = nullptr;
     CK(cudaMallocAsync((void**)&d, (size_t)pitch * h, st));
     CK(cudaMemcpy2DAsync(d, pitch, img, step, (size_t)w * c, h, cudaMemcpyHostToDevice, st));
@@ -1251,11 +1397,6 @@ int imp_gpu_brightness_host(const unsigned char* img, int step, int w, int h, in
     return rc;
 }
 
-// ---- "next" row §8f-4: ASCII (format=text) ---------------------------------------------------------------------
-// Density ramps of filters.c:486-487 (the reference's data; the classic 70- and 10-level ASCII-art ramps).
-static const char kAsciiWide[] = "$@B%8&WM#*oahkbdpqwmZO0QLCJUYXzcvunxrjft/\\|()1{}[]?-_+~<>i!lI;:,\"^`'. ";
-static const char kAsciiNarrow[] = "@%8#*+=-:. ";
-
 long imp_gpu_ascii_length(int width, int height) { return (long)(width + 1) * height - 1; }
 
 int imp_gpu_ascii_host(const unsigned char* img, int step, int w, int h, int c, const char* args, unsigned char* out, long out_cap) {
@@ -1263,23 +1404,20 @@ int imp_gpu_ascii_host(const unsigned char* img, int step, int w, int h, int c, 
     if (!img || !out || w <= 0 || h <= 0 || (c != 1 && c != 3 && c != 4)) return IMP_ERROR_INVALID_ARGS;
     const long len = imp_gpu_ascii_length(w, h);
     if (out_cap < len) return IMP_ERROR_INVALID_ARGS;
-    const char* table = (args && strcmp(args, "wide") == 0) ? kAsciiWide : kAsciiNarrow;     // filters.c:490-494
-    const int tablelen = (int)strlen(table);
-    const float factor = 256.0 / tablelen;                                                   // filters.c:496
-    unsigned char lut[256];
-    for (int v = 0; v < 256; v++) lut[v] = (unsigned char)table[(int)floor((double)((float)v / factor))];   // filters.c:509
     cudaStream_t st = g_dev[t_dev].stream;
-    const int pitch = align16(w * c);
-    uint8_t *d_img = nullptr, *d_lut = nullptr, *d_out = nullptr;
-    CK(cudaMallocAsync((void**)&d_img, (size_t)pitch * h, st));
-    CK(cudaMallocAsync((void**)&d_lut, 256, st));
+    ImpInfoJob q{};
+    q.pitch = align16(w * c); q.w = w; q.h = h; q.c = c; q.vec = 1;
+    q.ctas = imp_ascii_ctas(w, h);
+    q.wide = (args && strcmp(args, "wide") == 0) ? 1 : 0;                                  // filters.c:490-494
+    uint8_t *d_img = nullptr, *d_out = nullptr;
+    CK(cudaMallocAsync((void**)&d_img, (size_t)q.pitch * h, st));
     CK(cudaMallocAsync((void**)&d_out, (size_t)len + 1, st));
-    CK(cudaMemcpy2DAsync(d_img, pitch, img, step, (size_t)w * c, h, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(d_lut, lut, 256, cudaMemcpyHostToDevice, st));
-    CK(imp_launch_ascii(d_img, pitch, w, h, c, d_lut, d_out, st));
+    q.img = d_img;
+    CK(cudaMemcpy2DAsync(d_img, q.pitch, img, step, (size_t)w * c, h, cudaMemcpyHostToDevice, st));
+    CK(imp_launch_ascii(nullptr, q, 1, q.ctas, ascii_ramps(), d_out, st));
     CK(cudaMemcpyAsync(out, d_out, (size_t)len, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    cudaFreeAsync(d_img, st); cudaFreeAsync(d_lut, st); cudaFreeAsync(d_out, st);
+    cudaFreeAsync(d_img, st); cudaFreeAsync(d_out, st);
     return IMP_OK;
 }
 

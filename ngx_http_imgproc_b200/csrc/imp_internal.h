@@ -75,6 +75,7 @@ struct imp_gpu_plan {
     int out_w, out_h, out_c;
     unsigned long long algo_bytes;     // SURVEY §8d
     std::shared_ptr<ImpWmImage> wm;    // overlay the plan blends (shared, uploaded once per device), or null
+    int pack = IMP_PACK_NONE;          // the request's IMP_PACK_*: the layout of the stored result
     std::atomic<int> refs{1};          // the plan cache and every imp_gpu_plan_create caller hold one reference each
     // per-device state: ONE stream-ordered allocation holds every pass blob (+ vignette tables), filled by an
     // asynchronous copy from pinned staging; `ready_ev` orders the first kernels behind it
@@ -145,6 +146,21 @@ cudaError_t imp_launch_gather_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs
 // rows of `row_bytes` bytes from (src, sp) to (dst, dp); dst and dp are multiples of 4 (the library's own pitched buffers)
 cudaError_t imp_launch_repitch(const uint8_t* d_src, int sp, uint8_t* d_dst, int dp, int row_bytes, int rows, cudaStream_t st);
 cudaError_t imp_launch_gif_expand(const ImpGifFrame* d_frames, int n, int cw, int ch, int destructive, uint8_t* d_canvases, int cpitch, cudaStream_t st);
-cudaError_t imp_launch_ascii(const uint8_t* d_img, int pitch, int w, int h, int c, const uint8_t* d_lut, uint8_t* d_out, cudaStream_t st);
-cudaError_t imp_launch_brightness(const uint8_t* d_img, int pitch, int w, int h, int c, double* d_acc, cudaStream_t st);
+// One frame of a brightness or ASCII launch: a result on the device and where its answer goes.
+struct ImpInfoJob {
+    const uint8_t* img;          // rows of w*c bytes (c in {1,3,4}), `pitch` apart
+    long long text_off;          // ASCII: the job's first byte in the text arena
+    int pitch, w, h, c;
+    int vec;                     // 1: img and pitch are multiples of 16 (rows are read 16 bytes at a time)
+    int ctas;                    // CTAs over this job: imp_brightness_ctas / imp_ascii_ctas of (w, h)
+    int part_off;                // brightness: the first of the job's `ctas` partial sums
+    int wide;                    // ASCII: 1 = the 70-level ramp, 0 = the 10-level one
+};
+struct ImpAsciiRamps { uint8_t lut[2][256]; };   // HSV value -> character, [0] 10-level ramp, [1] 70-level ramp
+int imp_brightness_ctas(int w, int h);
+int imp_ascii_ctas(int w, int h);
+// n jobs from the device table d_jobs, or (d_jobs == nullptr, n == 1) the job `one` passed by value; grid.x = max_ctas, the
+// largest ctas of the jobs. Brightness: out[j] = brightness of job j; tickets[0..n) must be 0 and are left 0.
+cudaError_t imp_launch_brightness(const ImpInfoJob* d_jobs, const ImpInfoJob& one, int n, int max_ctas, double* partials, unsigned* tickets, float* out, cudaStream_t st);
+cudaError_t imp_launch_ascii(const ImpInfoJob* d_jobs, const ImpInfoJob& one, int n, int max_ctas, const ImpAsciiRamps& ramps, uint8_t* text, cudaStream_t st);
 cudaError_t imp_build_vignette_table(float* d_tab, int nx, int ny, float maxr, float intensity, cudaStream_t st);          // per-device constant tables of imp_pixel.cuh

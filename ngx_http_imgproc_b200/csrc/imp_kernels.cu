@@ -42,59 +42,159 @@ cudaError_t imp_build_vignette_table(float* d_tab, int nx, int ny, float maxr, f
     return cudaGetLastError();
 }
 
-// CalcPerceivedBrightness (filters.c:707-729): sum over pixels of sqrt(r*r*0.241 + g*g*0.691 + b*b*0.068) (or of the gray
-// value), as a device reduction so that `format=json` (Info, bridge.c:283-300) needs 8 bytes back instead of the frame.
-// The reference's running float32 sum in column-major order is not reproducible in parallel; this sums in double and the
-// caller divides by w*h*255. Parity is stated on the JSON integer round(brightness*100) (tests/test_gpu_parity.py).
-__global__ void __launch_bounds__(256) imp_brightness_kernel(const uint8_t* __restrict__ img, int pitch, int w, int h, int c, double* __restrict__ acc) {
-    double s = 0.0;
-    for (int y = blockIdx.y; y < h; y += gridDim.y) {
-        const uint8_t* row = img + (size_t)y * pitch;
-        for (int x = blockIdx.x * blockDim.x + threadIdx.x; x < w; x += gridDim.x * blockDim.x) {
-            if (c == 1) s += (double)row[x];
-            else {
-                const uint8_t* p = row + (size_t)x * c;
-                const int b = p[0], g = p[1], r = p[2];
-                s += sqrt(r * r * 0.241 + g * g * 0.691 + b * b * 0.068);
-            }
+// ---- answers instead of frames: Info's brightness (format=json) and ASCII (format=text) over a batch of results ------
+// One launch covers every job of a chunk: grid = (CTAs per job, jobs), each job described by an ImpInfoJob. A job's pixels
+// are cut into items, one item = a group of up to 16 consecutive pixels of a row (rows of 16-byte aligned frames are read
+// 16 bytes at a time); thread t of a CTA takes items t, t + 256, ... of the CTA's contiguous share.
+constexpr int INFO_THREADS = 256, INFO_GROUP = 16;
+
+int imp_brightness_ctas(int w, int h) {
+    const long long items = (long long)h * ((w + INFO_GROUP - 1) / INFO_GROUP);
+    return (int)std::min<long long>(256, std::max<long long>(1, (items + 2047) / 2048));
+}
+int imp_ascii_ctas(int w, int h) {
+    const long long items = (long long)h * ((w + INFO_GROUP - 1) / INFO_GROUP);
+    return (int)std::min<long long>(1024, std::max<long long>(1, (items + 1023) / 1024));
+}
+
+namespace {
+
+// byte i (a constant after unrolling) of N 16-byte words
+template <int N>
+__device__ __forceinline__ int byte_of(const uint4 (&q)[N], int i) {
+    const uint4 w = q[i >> 4];
+    const int k = (i >> 2) & 3;
+    const unsigned v = k == 0 ? w.x : k == 1 ? w.y : k == 2 ? w.z : w.w;
+    return (int)((v >> (8 * (i & 3))) & 255u);
+}
+
+// f(b, g, r, k) for pixel k = 0..n-1 of the group at p (gray: f(v, v, v, k)). VEC and a full group: C 16-byte loads (p is
+// 16-byte aligned); otherwise byte loads.
+template <int C, bool VEC, class F>
+__device__ __forceinline__ void for_group(const uint8_t* p, int n, F f) {
+    if (VEC && n == INFO_GROUP) {
+        uint4 q[C];
+#pragma unroll
+        for (int k = 0; k < C; k++) q[k] = __ldg(reinterpret_cast<const uint4*>(p) + k);
+#pragma unroll
+        for (int k = 0; k < INFO_GROUP; k++) {
+            if (C == 1) { const int v = byte_of(q, k); f(v, v, v, k); }
+            else f(byte_of(q, k * C), byte_of(q, k * C + 1), byte_of(q, k * C + 2), k);
         }
-    }
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
-    __shared__ double ws[8];
-    if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = s;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double t = 0.0;
-        for (int i = 0; i < 8; i++) t += ws[i];
-        atomicAdd(acc, t);
+    } else {
+        for (int k = 0; k < n; k++) {
+            const uint8_t* s = p + k * C;
+            if (C == 1) { const int v = __ldg(s); f(v, v, v, k); }
+            else f(__ldg(s), __ldg(s + 1), __ldg(s + 2), k);
+        }
     }
 }
 
-cudaError_t imp_launch_brightness(const uint8_t* d_img, int pitch, int w, int h, int c, double* d_acc, cudaStream_t st) {
-    cudaError_t e = cudaMemsetAsync(d_acc, 0, sizeof(double), st);
-    if (e != cudaSuccess) return e;
-    dim3 grid((w + 255) / 256 > 8 ? 8 : (w + 255) / 256, h < 1184 ? h : 1184);
-    imp_brightness_kernel<<<grid, 256, 0, st>>>(d_img, pitch, w, h, c, d_acc);
+// The item range [i0, i1) of CTA k: a function of (w, h) and J.ctas alone.
+__device__ __forceinline__ void cta_share(const ImpInfoJob& J, int k, int& i0, int& i1) {
+    const int total = J.h * ((J.w + INFO_GROUP - 1) / INFO_GROUP), per = (total + J.ctas - 1) / J.ctas;
+    i0 = min(total, k * per); i1 = min(total, i0 + per);
+}
+
+// The slow path of the double square root is a subroutine call, and values held in registers across it spill: the
+// channel count stays a run-time value (one call site), and a full group of an aligned frame is parked in the thread's own
+// shared-memory slot, so that both paths then read the pixels one by one.
+__device__ double brightness_share(const ImpInfoJob& J, int i0, int i1, uint4* slot) {
+    const int c = J.c, gpr = (J.w + INFO_GROUP - 1) / INFO_GROUP;
+    double s = 0.0;
+    for (int i = i0 + (int)threadIdx.x; i < i1; i += INFO_THREADS) {
+        const int y = i / gpr, g = i - y * gpr, n = min(INFO_GROUP, J.w - g * INFO_GROUP);
+        const uint8_t* p = J.img + (size_t)y * J.pitch + (size_t)g * (INFO_GROUP * c);
+        if (J.vec && n == INFO_GROUP) {
+            for (int k = 0; k < c; k++) slot[k] = __ldg(reinterpret_cast<const uint4*>(p) + k);
+            p = reinterpret_cast<const uint8_t*>(slot);
+        }
+        for (int k = 0; k < n; k++) {
+            const uint8_t* q = p + k * c;
+            if (c == 1) s += (double)q[0];
+            else { const int b = q[0], gg = q[1], r = q[2]; s += sqrt(r * r * 0.241 + gg * gg * 0.691 + b * b * 0.068); }
+        }
+    }
+    return s;
+}
+
+template <int C, bool VEC>
+__device__ void ascii_share(const ImpInfoJob& J, const uint8_t* lut, uint8_t* __restrict__ text, int i0, int i1) {
+    const int gpr = (J.w + INFO_GROUP - 1) / INFO_GROUP;
+    for (int i = i0 + (int)threadIdx.x; i < i1; i += INFO_THREADS) {
+        const int y = i / gpr, g = i - y * gpr, n = min(INFO_GROUP, J.w - g * INFO_GROUP);
+        uint8_t* o = text + J.text_off + (size_t)y * (J.w + 1) + (size_t)g * INFO_GROUP;
+        for_group<C, VEC>(J.img + (size_t)y * J.pitch + (size_t)g * (INFO_GROUP * C), n,
+                          [&](int b, int gg, int r, int k) { o[k] = lut[C == 1 ? b : max(b, max(gg, r))]; });
+        if (g == gpr - 1 && y + 1 < J.h) o[n] = '\n';                  // rows separated, no trailing newline
+    }
+}
+
+}  // namespace
+
+// CalcPerceivedBrightness (filters.c:707-729): the sum over pixels of sqrt(r*r*0.241 + g*g*0.691 + b*b*0.068) (or of the gray
+// value) in double, divided by w*h*255. The reference's float32 running sum in column-major order is not reproducible in
+// parallel; this sum is reproducible instead: each CTA sums its share in a fixed thread order and a fixed tree, writes
+// partials[part_off + k], and the job's last CTA (a per-job ticket, reset for the next launch) adds the partials in index
+// order. CTAs per job depend on (w, h) only, so a frame gives the same bits in any batch, chunk or lane.
+__global__ void __launch_bounds__(INFO_THREADS) imp_brightness_kernel(const ImpInfoJob* __restrict__ jobs, const ImpInfoJob one, double* __restrict__ partials,
+                                                                     unsigned* __restrict__ tickets, float* __restrict__ out) {
+    const int j = blockIdx.y, k = blockIdx.x;
+    const ImpInfoJob J = jobs ? jobs[j] : one;
+    if (k >= J.ctas) return;
+    int i0, i1;
+    cta_share(J, k, i0, i1);
+    __shared__ uint4 stage[INFO_THREADS][4];
+    double s = brightness_share(J, i0, i1, stage[threadIdx.x]);
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+    __shared__ double ws[INFO_THREADS / 32];
+    if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    double t = 0.0;
+    for (int w = 0; w < INFO_THREADS / 32; w++) t += ws[w];
+    partials[J.part_off + k] = t;
+    __threadfence();                                                   // the partial is visible before the ticket is taken
+    if (atomicAdd(&tickets[j], 1u) != (unsigned)J.ctas - 1) return;
+    const volatile double* P = partials + J.part_off;
+    double sum = 0.0;
+    for (int q = 0; q < J.ctas; q++) sum += P[q];
+    out[j] = (float)(sum / ((double)J.w * J.h) / 255.0);               // filters.c:728
+    tickets[j] = 0;
+}
+
+// ASCII (filters.c:486-522, format=text): one character per pixel from the HSV value V = max(B,G,R) through the job's
+// 256-entry ramp (built on the host with the reference's float maths); rows separated by '\n', no trailing newline.
+__global__ void __launch_bounds__(INFO_THREADS) imp_ascii_kernel(const ImpInfoJob* __restrict__ jobs, const ImpInfoJob one, const ImpAsciiRamps ramps,
+                                                                 uint8_t* __restrict__ text) {
+    const int j = blockIdx.y, k = blockIdx.x;
+    const ImpInfoJob J = jobs ? jobs[j] : one;
+    if (k >= J.ctas) return;
+    __shared__ uint8_t lut[256];
+    lut[threadIdx.x] = ramps.lut[J.wide ? 1 : 0][threadIdx.x];
+    __syncthreads();
+    int i0, i1;
+    cta_share(J, k, i0, i1);
+    switch (J.c * 2 + J.vec) {
+        case 2: ascii_share<1, false>(J, lut, text, i0, i1); break;
+        case 3: ascii_share<1, true>(J, lut, text, i0, i1); break;
+        case 6: ascii_share<3, false>(J, lut, text, i0, i1); break;
+        case 7: ascii_share<3, true>(J, lut, text, i0, i1); break;
+        case 8: ascii_share<4, false>(J, lut, text, i0, i1); break;
+        case 9: ascii_share<4, true>(J, lut, text, i0, i1); break;
+    }
+}
+
+cudaError_t imp_launch_brightness(const ImpInfoJob* d_jobs, const ImpInfoJob& one, int n, int max_ctas, double* partials, unsigned* tickets, float* out, cudaStream_t st) {
+    if (n <= 0 || n > 65535 || max_ctas <= 0) return cudaErrorInvalidValue;
+    imp_brightness_kernel<<<dim3(max_ctas, n), INFO_THREADS, 0, st>>>(d_jobs, one, partials, tickets, out);
     g_imp_launches++;
     return cudaGetLastError();
 }
 
-// ASCII (filters.c:486-522, `format=text`): one character per pixel from the HSV value V = max(B,G,R) through a 256-entry
-// table the host derives with the reference's float maths; rows are separated by '\n' (no trailing newline).
-__global__ void __launch_bounds__(256) imp_ascii_kernel(const uint8_t* __restrict__ img, int pitch, int w, int h, int c,
-                                                        const uint8_t* __restrict__ lut, uint8_t* __restrict__ out) {
-    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-    if (x > w || y >= h) return;
-    uint8_t* o = out + (size_t)y * (w + 1) + x;
-    if (x == w) { if (y + 1 < h) *o = '\n'; return; }
-    const uint8_t* p = img + (size_t)y * pitch + (size_t)x * c;
-    const int v = c == 1 ? p[0] : max(p[0], max(p[1], p[2]));
-    *o = __ldg(lut + v);
-}
-
-cudaError_t imp_launch_ascii(const uint8_t* d_img, int pitch, int w, int h, int c, const uint8_t* d_lut, uint8_t* d_out, cudaStream_t st) {
-    dim3 grid((w + 1 + 255) / 256, h);
-    imp_ascii_kernel<<<grid, 256, 0, st>>>(d_img, pitch, w, h, c, d_lut, d_out);
+cudaError_t imp_launch_ascii(const ImpInfoJob* d_jobs, const ImpInfoJob& one, int n, int max_ctas, const ImpAsciiRamps& ramps, uint8_t* text, cudaStream_t st) {
+    if (n <= 0 || n > 65535 || max_ctas <= 0) return cudaErrorInvalidValue;
+    imp_ascii_kernel<<<dim3(max_ctas, n), INFO_THREADS, 0, st>>>(d_jobs, one, ramps, text);
     g_imp_launches++;
     return cudaGetLastError();
 }

@@ -42,6 +42,12 @@ void default_release(IplImage** p) {
     if (p && *p) { free((*p)->imageDataOrigin); free((*p)->roi); free(*p); *p = nullptr; }
 }
 
+Pending from_header(const IplImage* im) {
+    Pending p;
+    p.data = im->imageData; p.w = p.cur_w = im->width; p.h = p.cur_h = im->height; p.c = p.cur_c = im->nChannels; p.step = im->widthStep;
+    return p;
+}
+
 Pending& entry(IplImage* im) {
     auto it = g_pending.find(im);
     if (it != g_pending.end()) {
@@ -49,9 +55,7 @@ Pending& entry(IplImage* im) {
         if (p.data == im->imageData && p.cur_w == im->width && p.cur_h == im->height && p.cur_c == im->nChannels) return p;
         g_pending.erase(it);                              // a different image now lives at this address
     }
-    Pending p;
-    p.data = im->imageData; p.w = p.cur_w = im->width; p.h = p.cur_h = im->height; p.c = p.cur_c = im->nChannels; p.step = im->widthStep;
-    return g_pending.emplace(im, p).first->second;
+    return g_pending.emplace(im, from_header(im)).first->second;
 }
 
 struct Built { imp_gpu_request req; imp_gpu_config cfg; std::vector<const char*> fp; };
@@ -85,10 +89,25 @@ int validate(IplImage* im, Pending& p) {
     return IMP_OK;
 }
 
-int run_one(IplImage** pointer, Pending& p, imp_gpu_plan** plan_out, IplImage** out_img) {
+// What a flush runs for `im` (caller holds g_ops_mu): the recorded chain, or — nothing recorded, `*idle` — the frame as it
+// is, held in `scratch`. An idle frame only has to run when it has 1 channel: the empty plan promotes gray to BGR
+// (bridge.c:613-618).
+const Pending& flush_entry(IplImage* im, Pending& scratch, bool* idle) {
+    auto it = g_pending.find(im);
+    *idle = it == g_pending.end() || it->second.n_ops == 0;
+    if (!*idle) return it->second;
+    scratch = from_header(im);
+    return scratch;
+}
+
+int make_plan(const Pending& p, imp_gpu_plan** plan_out) {
     Built b; to_request(p, b);
     int step = 0;
-    int rc = imp_gpu_plan_create(&b.req, &b.cfg, p.w, p.h, p.c, plan_out, &step);
+    return imp_gpu_plan_create(&b.req, &b.cfg, p.w, p.h, p.c, plan_out, &step);
+}
+
+int run_one(IplImage** pointer, const Pending& p, imp_gpu_plan** plan_out, IplImage** out_img) {
+    int rc = make_plan(p, plan_out);
     if (rc) return rc;
     imp_ops_create_image_fn create = g_create ? g_create : default_create;
     IplImage* out = create((*plan_out)->out_w, (*plan_out)->out_h, (*pointer)->depth ? (*pointer)->depth : 8, (*plan_out)->out_c);
@@ -209,12 +228,9 @@ static int flush_all(IplImage** frames, int count, const imp_gpu_gif_frame* page
         std::lock_guard<std::mutex> lk(g_ops_mu);
         for (int i = 0; i < count && rc == IMP_OK; i++) {
             if (!frames[i]) { if (pages) rc = IMP_ERROR_INVALID_ARGS; continue; }
-            auto it = g_pending.find(frames[i]);
-            const bool idle = it == g_pending.end() || it->second.n_ops == 0;
-            // bridge.c:613-618 turns EVERY 1-channel frame into BGR at the filter step, even when no operator was asked for:
-            // such a frame still takes the (empty) plan, whose store promotes gray to B,G,R
-            if (idle && frames[i]->nChannels != 1 && !pages) { if (it != g_pending.end()) g_pending.erase(it); continue; }
-            Pending& p = idle ? entry(frames[i]) : it->second;
+            Pending scratch; bool idle;
+            const Pending& p = flush_entry(frames[i], scratch, &idle);
+            if (idle && frames[i]->nChannels != 1 && !pages) { g_pending.erase(frames[i]); continue; }
             if (pages) {
                 if (i == 0) { cw = p.w; ch = p.h; }
                 if (p.c != 4 || p.w != cw || p.h != ch) { rc = IMP_ERROR_INVALID_ARGS; break; }
@@ -267,6 +283,41 @@ int imp_FlushAllGif(IplImage** frames, int count, const imp_gpu_gif_frame* pages
 int imp_Flush(IplImage** pointer) {
     if (!pointer || !*pointer) return IMP_ERROR_INVALID_ARGS;
     return imp_FlushAll(pointer, 1);
+}
+
+// The job imp_Flush would run for `image` (an idle multi-channel frame: the empty plan, a copy), its answer computed on the
+// device. Nothing recorded is consumed.
+static int answer_job(IplImage* image, imp_gpu_plan** plan, const unsigned char** src, int* step) {
+    std::lock_guard<std::mutex> lk(g_ops_mu);
+    Pending scratch; bool idle;
+    const Pending& p = flush_entry(image, scratch, &idle);
+    *src = (const unsigned char*)p.data; *step = p.step;
+    return make_plan(p, plan);
+}
+
+int imp_Brightness(IplImage* image, float* brightness) {
+    IMP_OPS_TRY
+    if (!image || !brightness) return IMP_ERROR_INVALID_ARGS;
+    imp_gpu_plan* plan = nullptr; const unsigned char* src = nullptr; int step = 0;
+    int rc = answer_job(image, &plan, &src, &step);
+    if (rc) return rc;
+    rc = imp_gpu_batch_brightness_host(1, &plan, &src, &step, brightness, 1);
+    imp_gpu_plan_destroy(plan);
+    return rc;
+    IMP_OPS_CATCH
+}
+
+int imp_Ascii(IplImage* image, const char* args, unsigned char* out, long out_cap) {
+    IMP_OPS_TRY
+    if (!image || !out) return IMP_ERROR_INVALID_ARGS;
+    imp_gpu_plan* plan = nullptr; const unsigned char* src = nullptr; int step = 0;
+    int rc = answer_job(image, &plan, &src, &step);
+    if (rc) return rc;
+    unsigned char* texts[1] = {out};
+    rc = imp_gpu_batch_ascii_host(1, &plan, &src, &step, &args, texts, &out_cap, 1);
+    imp_gpu_plan_destroy(plan);
+    return rc;
+    IMP_OPS_CATCH
 }
 
 }  // extern "C"

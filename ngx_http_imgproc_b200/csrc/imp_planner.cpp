@@ -958,6 +958,7 @@ int imp_build_plan(const imp_gpu_request* req, const imp_gpu_config* cfg, int w,
     }
     L.end_pass(L.fr.map(), L.fr.w, L.fr.h);
     plan->out_w = L.fr.w; plan->out_h = L.fr.h; plan->out_c = L.final_dc ? L.final_dc : L.fr.c;
+    plan->pack = req->pack;
     plan->algo_bytes = (unsigned long long)cw * ch * c + (unsigned long long)plan->out_w * plan->out_h * plan->out_c + wm_bytes;
     return IMP_OK;
 }

@@ -173,13 +173,15 @@ int  imp_gpu_batch_launches_per_run(const imp_gpu_batch* batch);
  * jobs; each chunk's crop windows are copied H2D, the whole chunk runs as ONE grouped launch per kernel variant
  * (device job table, as imp_gpu_batch_launch), its results are copied D2H; `n_streams` (1..8) chunks are in flight on
  * their own streams and pinned staging lanes, so copies and kernels overlap. The frame loops of RunJob
- * (bridge.c:576-656) over album.Frames[] map onto one call. */
+ * (bridge.c:576-656) over album.Frames[] map onto one call. Every job is checked before any work starts: a NULL plan,
+ * source or destination, or a step shorter than its row returns IMP_ERROR_INVALID_ARGS with nothing written. */
 int  imp_gpu_batch_run_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs,
                             const int* src_steps, unsigned char* const* dsts, const int* dst_steps,
                             int n_streams);
-/* Asynchronous form (SURVEY 8b-4 submit/wait): returns at once with a ticket; a helper thread drives the batch on the
- * caller's current device. The argument arrays are copied, the pixel buffers must stay valid until imp_gpu_batch_wait,
- * which blocks, returns the batch's code and frees the ticket. imp_gpu_batch_poll: 1 when finished, 0 while running. */
+/* Asynchronous form (SURVEY 8b-4 submit/wait): checks every job (a bad one: IMP_ERROR_INVALID_ARGS, no ticket), then
+ * returns at once with a ticket; a helper thread drives the batch on the caller's current device. The argument arrays
+ * are copied, the pixel buffers must stay valid until imp_gpu_batch_wait, which blocks, returns the batch's code and
+ * frees the ticket. imp_gpu_batch_poll: 1 when finished, 0 while running. */
 int  imp_gpu_batch_submit_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs,
                                const int* src_steps, unsigned char* const* dsts, const int* dst_steps,
                                int n_streams, imp_gpu_ticket** ticket);

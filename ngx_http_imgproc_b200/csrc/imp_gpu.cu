@@ -38,9 +38,6 @@ int fail_msg(const char* msg) { snprintf(t_err, sizeof t_err, "%s", msg); return
 
 #define CK(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return fail(e__, #call, __LINE__); } while (0)
 
-int align16(int v) { return (v + 15) & ~15; }
-size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
-
 // A growable buffer (device or pinned host) that is only ever re-allocated when a request outgrows it.
 struct Buf {
     uint8_t* p = nullptr; size_t cap = 0;
@@ -105,7 +102,8 @@ struct Lane {            // one in-flight chunk of host jobs of the end-to-end p
     imp_gpu_batch batch;                         // the chunk's job table, scratch and tensor maps
     Buf d_info, h_info;                          // brightness / ASCII: job table, partial sums, answers, texts; the table's pinned staging
     Buf d_tickets;                               // brightness: one ticket per job of a chunk, zeroed once (the kernel leaves them 0)
-    struct Out { int job; long long staged_off; };   // staged_off >= 0: copy from h_out after the sync
+    bool busy = false;                           // a chunk was issued and is not finished
+    struct Out { uint8_t* dst; size_t dst_step, row_bytes; int rows; size_t hout_off; };   // staged results: copied from h_out after the sync
     std::vector<Out> pend;
 };
 struct DevCtx {
@@ -513,29 +511,12 @@ void batch_release(imp_gpu_batch* b) {          // device/pinned memory of a bat
 
 
 // ---- the chunked end-to-end path over host buffers ---------------------------------------------------------------------
-// Requests are cut into CHUNKS of consecutive jobs (up to kChunkJobs jobs / kChunkBytes of crop windows); a chunk owns one
-// lane (stream + staging) while it is in flight: H2D of every window, ONE launch per (pass, kernel choice) over the whole
-// chunk through a device job table (the path the device-resident batches take), D2H of every result. Lanes rotate, so the
-// copies of chunk k+1 overlap the kernels of chunk k and the D2H of chunk k-1 (PCIe is full duplex).
-constexpr int kChunkJobs = 256;
-constexpr size_t kChunkBytes = 128u << 20;
-
-struct HostJobs {
-    int n; imp_gpu_plan* const* plans; const unsigned char* const* srcs; const int* src_steps;
-    unsigned char* const* dsts; const int* dst_steps;
-    bool src_device = false;       // srcs[] are whole frames already on this device (pitch % 16 == 0): nothing to upload
-    // What comes back: the frames (dsts), or one more launch per chunk reduces the results on the device and only its
-    // answers come back: brightness[i], or texts[i] (ASCII with the 70-level ramp where wide[i]).
-    enum Result { Frame, Brightness, Ascii } result = Frame;
-    float* brightness = nullptr;
-    unsigned char* const* texts = nullptr; const unsigned char* wide = nullptr;
-};
-
-// The answer of job i when it is not a frame: where it goes on the host and its size.
-uint8_t* answer_dst(const HostJobs& J, int i) { return J.result == HostJobs::Ascii ? J.texts[i] : reinterpret_cast<uint8_t*>(J.brightness + i); }
-size_t answer_bytes(const HostJobs& J, int i) {
-    return J.result == HostJobs::Ascii ? (size_t)imp_gpu_ascii_length(J.plans[i]->out_w, J.plans[i]->out_h) : sizeof(float);
-}
+// Requests are cut into CHUNKS of consecutive jobs (imp_chunk_bounds); a chunk owns one lane (stream + staging) while it is
+// in flight: H2D of every window, ONE launch per (pass, kernel choice) over the whole chunk through a device job table (the
+// path the device-resident batches take), D2H of every result. Lanes rotate, so the copies of chunk k+1 overlap the kernels
+// of chunk k and the D2H of chunk k-1 (PCIe is full duplex). How each job's bytes travel is imp_chunk_layout's choice.
+// What comes back: the frames, or one more launch per chunk reduces the results on the device and only the answers come
+// back (ImpResult::Brightness, ::Ascii).
 
 bool is_pinned(const void* p) {
     cudaPointerAttributes a;
@@ -561,11 +542,10 @@ int stage_parts(size_t bytes, int items) {
 // The big host-side copies (pageable frame -> pinned staging, pinned staging -> pageable result) use streaming stores: the
 // destination is written once and not read by this core again, so it need not be read into the cache first as a plain
 // memcpy's write-allocate does — on the B200 box one request's 29 MB window went from 2.4 to 1.2 ms, a 64-request batch
-// from 29 to 42 GB/s. IMP_GPU_STAGE_NT=0 falls back to memcpy (tuning knob).
+// from 29 to 42 GB/s.
 void copy_stream(uint8_t* dst, const uint8_t* src, size_t n) {
 #if defined(__SSE2__)
-    static const bool nt = [] { const char* e = getenv("IMP_GPU_STAGE_NT"); return !e || atoi(e) != 0; }();
-    if (nt && n >= 4096) {
+    if (n >= 4096) {
         const size_t head = (16 - (reinterpret_cast<uintptr_t>(dst) & 15)) & 15;
         if (head) { memcpy(dst, src, head); dst += head; src += head; n -= head; }
         const size_t v = n >> 6;
@@ -581,6 +561,11 @@ void copy_stream(uint8_t* dst, const uint8_t* src, size_t n) {
     }
 #endif
     memcpy(dst, src, n);
+}
+// `rows` rows of `row_bytes`: one copy when both sides are dense, else row by row
+void copy_rows(uint8_t* dst, size_t dst_step, const uint8_t* src, size_t src_step, size_t row_bytes, int rows) {
+    if (dst_step == row_bytes && src_step == row_bytes) copy_stream(dst, src, row_bytes * rows);
+    else for (int y = 0; y < rows; y++) copy_stream(dst + (size_t)y * dst_step, src + (size_t)y * src_step, row_bytes);
 }
 // The copy workers: a small persistent pool (spawning threads per copy costs ~50 us each, more than a 2 MB slice takes).
 // Created on first use — after nginx has forked its workers — and again in a child should a process fork later.
@@ -652,46 +637,28 @@ template <class F> void run_parts(int n, int parts, F fn) {
     latch.c.wait(lk, [&] { return latch.left == 0; });
 }
 
-int lane_finish(Lane& L, const HostJobs& J) {
-    if (L.pend.empty()) return IMP_OK;
+int lane_finish(Lane& L) {
+    if (!L.busy) return IMP_OK;
     cudaError_t e = cudaStreamSynchronize(L.st);
-    if (e == cudaSuccess && J.result != HostJobs::Frame) {
-        std::vector<const Lane::Out*> staged; size_t bytes = 0;
-        for (const Lane::Out& o : L.pend) if (o.staged_off >= 0) { staged.push_back(&o); bytes += answer_bytes(J, o.job); }
-        const Lane::Out* const* sg = staged.data();
-        const uint8_t* h_out = L.h_out.p;
-        run_parts((int)staged.size(), stage_parts(bytes, (int)staged.size()), [=, &J](int k0, int k1) {
-            for (int k = k0; k < k1; k++) copy_stream(answer_dst(J, sg[k]->job), h_out + sg[k]->staged_off, answer_bytes(J, sg[k]->job));
-        });
-    } else if (e == cudaSuccess) {
+    if (e == cudaSuccess) {
         // results for pageable destinations (the frames cvCreateImage hands out) leave the pinned staging here; a 200-frame GIF
-        // is 400 MB of it
+        // is 400 MB of it. Big frames one after the other, each frame's rows over the threads; the other results of the
+        // chunk (answers whatever their size) shared out whole.
         const uint8_t* h_out = L.h_out.p;
-        // big frames one after the other, each frame's rows over the threads; the small ones of the chunk shared out whole
         std::vector<const Lane::Out*> small; size_t small_bytes = 0;
         for (const Lane::Out& o : L.pend) {
-            if (o.staged_off < 0) continue;
-            const imp_gpu_plan* p = J.plans[o.job];
-            const size_t row = (size_t)p->out_w * p->out_c, bytes = row * p->out_h;
-            if (bytes < (4u << 20)) { small.push_back(&o); small_bytes += bytes; continue; }
-            uint8_t* dst = J.dsts[o.job]; const int step = J.dst_steps[o.job]; const uint8_t* src = h_out + o.staged_off;
-            run_parts(p->out_h, stage_parts(bytes, p->out_h), [=](int y0, int y1) {
-                if ((size_t)step == row) copy_stream(dst + (size_t)y0 * row, src + (size_t)y0 * row, row * (size_t)(y1 - y0));
-                else for (int y = y0; y < y1; y++) copy_stream(dst + (size_t)y * step, src + (size_t)y * row, row);
+            const size_t bytes = o.row_bytes * o.rows;
+            if (o.rows == 1 || bytes < (4u << 20)) { small.push_back(&o); small_bytes += bytes; continue; }
+            run_parts(o.rows, stage_parts(bytes, o.rows), [&o, h_out](int y0, int y1) {
+                copy_rows(o.dst + (size_t)y0 * o.dst_step, o.dst_step, h_out + o.hout_off + y0 * o.row_bytes, o.row_bytes, o.row_bytes, y1 - y0);
             });
         }
         const Lane::Out* const* sm = small.data();
-        run_parts((int)small.size(), stage_parts(small_bytes, (int)small.size()), [=, &J](int k0, int k1) {
-            for (int k = k0; k < k1; k++) {
-                const Lane::Out& o = *sm[k];
-                const imp_gpu_plan* p = J.plans[o.job];
-                const size_t row = (size_t)p->out_w * p->out_c;
-                if ((size_t)J.dst_steps[o.job] == row) copy_stream(J.dsts[o.job], h_out + o.staged_off, row * p->out_h);
-                else for (int y = 0; y < p->out_h; y++) copy_stream(J.dsts[o.job] + (size_t)y * J.dst_steps[o.job], h_out + o.staged_off + (size_t)y * row, row);
-            }
+        run_parts((int)small.size(), stage_parts(small_bytes, (int)small.size()), [sm, h_out](int k0, int k1) {
+            for (int k = k0; k < k1; k++) copy_rows(sm[k]->dst, sm[k]->dst_step, h_out + sm[k]->hout_off, sm[k]->row_bytes, sm[k]->row_bytes, sm[k]->rows);
         });
     }
-    L.pend.clear();
+    L.pend.clear(); L.busy = false;
     if (e != cudaSuccess) return fail(e, "cudaStreamSynchronize", __LINE__);
     return IMP_OK;
 }
@@ -712,23 +679,23 @@ const ImpAsciiRamps& ascii_ramps() {
     return r;
 }
 
-// Brightness / ASCII of the chunk's m results (out_off / out_pitch in L.d_out): ONE launch over all of them, then only the
-// answers cross the link — straight into pinned destinations, into h_out at staged[k] >= 0 otherwise (lane_finish copies on).
-int lane_answers(Lane& L, const HostJobs& J, int first, int m, const std::vector<size_t>& out_off, const std::vector<int>& out_pitch,
-                 const std::vector<long long>& staged) {
-    const bool ascii = J.result == HostJobs::Ascii;
+// Brightness / ASCII of the chunk's m results (in L.d_out): ONE launch over all of them, then only the answers cross the
+// link — straight into pinned destinations, through h_out otherwise (lane_finish copies on).
+int lane_answers(Lane& L, const ImpHostJob* jobs, int m, ImpResult kind, const ImpChunkLayout& lay) {
+    const bool ascii = kind == ImpResult::Ascii;
     std::vector<ImpInfoJob> tab(m);
     int parts = 0, max_ctas = 1;
     size_t text_total = 0;
     for (int k = 0; k < m; k++) {
-        const imp_gpu_plan* p = J.plans[first + k];
+        const imp_gpu_plan* p = jobs[k].plan;
+        const ImpJobLayout& l = lay.jobs[k];
         ImpInfoJob& q = tab[k];
         q = ImpInfoJob{};
-        q.img = L.d_out.p + out_off[k]; q.pitch = out_pitch[k];          // 256-byte aligned slot, 16-byte pitch
+        q.img = L.d_out.p + l.out_off; q.pitch = l.out_pitch;                // 256-byte aligned slot, 16-byte pitch
         q.w = p->out_w; q.h = p->out_h; q.c = p->out_c; q.vec = 1;
         if (ascii) {
-            q.ctas = imp_ascii_ctas(q.w, q.h); q.wide = J.wide[first + k] ? 1 : 0;
-            q.text_off = (long long)text_total; text_total += align256(answer_bytes(J, first + k));
+            q.ctas = imp_ascii_ctas(q.w, q.h); q.wide = jobs[k].wide ? 1 : 0;
+            q.text_off = (long long)text_total; text_total += align256(l.res_bytes);
         } else {
             q.ctas = imp_brightness_ctas(q.w, q.h); q.part_off = parts; parts += q.ctas;
         }
@@ -738,7 +705,7 @@ int lane_answers(Lane& L, const HostJobs& J, int first, int m, const std::vector
     int r;
     if ((r = L.d_info.grow(tab_bytes + part_bytes + ans_bytes + text_total, false)) || (r = L.h_info.grow(tab_bytes, true))) return r;
     if (!ascii && !L.d_tickets.p) {
-        if ((r = L.d_tickets.grow(sizeof(unsigned) * kChunkJobs, false))) return r;
+        if ((r = L.d_tickets.grow(sizeof(unsigned) * IMP_CHUNK_JOBS, false))) return r;
         CK(cudaMemsetAsync(L.d_tickets.p, 0, L.d_tickets.cap, L.st));
     }
     memcpy(L.h_info.p, tab.data(), sizeof(ImpInfoJob) * m);
@@ -746,145 +713,105 @@ int lane_answers(Lane& L, const HostJobs& J, int first, int m, const std::vector
     const ImpInfoJob* d_tab = reinterpret_cast<const ImpInfoJob*>(L.d_info.p);
     uint8_t* d_ans = L.d_info.p + tab_bytes + part_bytes;
     uint8_t* d_text = d_ans + ans_bytes;
+    auto dst = [&](int k) { return lay.jobs[k].dst == ImpRoute::Staged ? L.h_out.p + lay.jobs[k].hout_off : jobs[k].dst; };
     if (ascii) CK(imp_launch_ascii(d_tab, tab[0], m, max_ctas, ascii_ramps(), d_text, L.st));
     else CK(imp_launch_brightness(d_tab, tab[0], m, max_ctas, reinterpret_cast<double*>(L.d_info.p + tab_bytes),
                                   reinterpret_cast<unsigned*>(L.d_tickets.p), reinterpret_cast<float*>(d_ans), L.st));
-    if (!ascii) CK(cudaMemcpyAsync(staged[0] >= 0 ? L.h_out.p + staged[0] : answer_dst(J, first), d_ans, sizeof(float) * m, cudaMemcpyDeviceToHost, L.st));
+    if (!ascii) CK(cudaMemcpyAsync(dst(0), d_ans, sizeof(float) * m, cudaMemcpyDeviceToHost, L.st));
     for (int k = 0; k < m; k++) {
-        const int i = first + k;
-        if (ascii) CK(cudaMemcpyAsync(staged[k] >= 0 ? L.h_out.p + staged[k] : answer_dst(J, i), d_text + tab[k].text_off, answer_bytes(J, i), cudaMemcpyDeviceToHost, L.st));
-        L.pend.push_back(Lane::Out{i, staged[k]});
+        const ImpJobLayout& l = lay.jobs[k];
+        if (ascii) CK(cudaMemcpyAsync(dst(k), d_text + tab[k].text_off, l.res_bytes, cudaMemcpyDeviceToHost, L.st));
+        if (l.dst == ImpRoute::Staged) L.pend.push_back(Lane::Out{jobs[k].dst, l.res_bytes, l.res_bytes, 1, l.hout_off});
     }
     return IMP_OK;
 }
 
-int lane_issue(Lane& L, const HostJobs& J, int first, int last) {
-    const int m = last - first;
-    struct Lay { size_t in_off, out_off, stage_off, hin_off; long long hout_off; int in_pitch, out_pitch; bool src_pinned, dst_pinned, linear; size_t lin_bytes; };
-    std::vector<Lay> lay(m);
-    size_t in_total = 0, out_total = 0, stage_total = 0, hin_total = 0, hout_total = 0;
+// Issues one chunk of m jobs on lane L. The order on the lane's stream: every upload in job order, the up_done record, the
+// window extractions (a kernel never sits between two copies of the stream and idles the copy engine), the grouped
+// launches, then the answer launch or the downloads.
+int lane_issue(Lane& L, const ImpHostJob* jobs, int m, ImpResult kind, bool resident) {
+    std::unique_ptr<bool[]> pinned(new bool[2 * (size_t)m]);
+    bool* src_pinned = pinned.get(); bool* dst_pinned = src_pinned + m;
     for (int k = 0; k < m; k++) {
-        const int i = first + k;
-        imp_gpu_plan* p = J.plans[i];
-        const bool frame = J.result == HostJobs::Frame;
-        if (!p || !J.srcs[i] || (frame && !J.dsts[i])) return IMP_ERROR_INVALID_ARGS;
-        Lay& l = lay[k];
-        const size_t in_row = (size_t)p->win_w * p->src_c, out_row = (size_t)p->out_w * p->out_c;
-        l.in_pitch = align16((int)in_row); l.out_pitch = align16((int)out_row);
-        l.in_off = in_total;
-        if (!J.src_device) in_total += align256((size_t)l.in_pitch * p->win_h);                       // landing zone of the crop window
-        l.out_off = out_total; out_total += align256((size_t)l.out_pitch * p->out_h);
-        l.src_pinned = is_pinned(J.srcs[i]);
-        l.dst_pinned = frame ? is_pinned(J.dsts[i]) : J.result == HostJobs::Ascii ? is_pinned(J.texts[i]) : is_pinned(J.brightness + first);
-        l.linear = false; l.lin_bytes = 0; l.stage_off = 0; l.hin_off = 0; l.hout_off = -1;
-        if (J.src_device) {
-            if ((reinterpret_cast<uintptr_t>(J.srcs[i]) & 15) || (J.src_steps[i] & 15) || (size_t)J.src_steps[i] < (size_t)p->src_w * p->src_c) return IMP_ERROR_INVALID_ARGS;
-            l.src_pinned = true;
-        } else if (l.src_pinned) {
-            // A 2-D host-to-device copy pays ~0.15 us per row whatever its width (measured: 3.5 KB rows move at 23 GB/s,
-            // 14 KB rows at the link's 54 GB/s). Short rows therefore travel as ONE linear copy of the rows the window
-            // touches (full width) and a small kernel extracts / re-pitches the window on the device.
-            // (a window that IS the frame's contiguous rows is one linear copy whatever its row length)
-            if (J.src_steps[i] <= 8192 || ((size_t)J.src_steps[i] == (size_t)l.in_pitch && p->win_x == 0 && in_row == (size_t)l.in_pitch)) {
-                l.linear = true;
-                l.lin_bytes = (size_t)(p->win_h - 1) * J.src_steps[i] + (size_t)p->win_x * p->src_c + in_row;
-                const bool direct = J.src_steps[i] == l.in_pitch && p->win_x == 0;
-                if (!direct) { l.stage_off = stage_total; stage_total += align256(l.lin_bytes); }
-            }
-        } else {
-            l.hin_off = hin_total; hin_total += align256((size_t)l.in_pitch * p->win_h);       // packed with the device pitch
-        }
-        if (!l.dst_pinned) {
-            l.hout_off = (long long)hout_total;
-            // brightness answers are staged back to back: the chunk's floats come back in one copy
-            hout_total += frame ? align256(out_row * p->out_h) : J.result == HostJobs::Ascii ? align256(answer_bytes(J, i)) : sizeof(float);
-        }
+        src_pinned[k] = resident || is_pinned(jobs[k].src);
+        dst_pinned[k] = is_pinned(jobs[k].dst);
     }
+    const ImpChunkLayout lay = imp_chunk_layout(jobs, m, kind, resident, src_pinned, dst_pinned);
     int r;
-    if ((r = L.d_in.grow(in_total, false)) || (r = L.d_out.grow(out_total, false)) || (r = L.d_stage.grow(stage_total, false)) ||
-        (r = L.h_in.grow(hin_total, true)) || (r = L.h_out.grow(hout_total, true))) return r;
+    if ((r = L.d_in.grow(lay.in_total, false)) || (r = L.d_out.grow(lay.out_total, false)) || (r = L.d_stage.grow(lay.stage_total, false)) ||
+        (r = L.h_in.grow(lay.hin_total, true)) || (r = L.h_out.grow(lay.hout_total, true))) return r;
+    L.busy = true;
     imp_gpu_batch& B = L.batch;
     B.items.clear(); B.dirty = true;
-    // window extractions of the linear uploads: launched after ALL copies of the chunk, so that a kernel never sits between
-    // two copies of this stream and idles the copy engine
     struct Repitch { const uint8_t* src; int sp; uint8_t* dst; int dp, row_bytes, rows; };
     std::vector<Repitch> repitch;
     for (int k = 0; k < m; k++) {
-        const int i = first + k;
-        imp_gpu_plan* p = J.plans[i];
-        const Lay& l = lay[k];
+        const ImpHostJob& j = jobs[k];
+        const ImpJobLayout& l = lay.jobs[k];
+        imp_gpu_plan* p = j.plan;
         const int sc = p->src_c;
         const size_t in_row = (size_t)p->win_w * sc;
         uint8_t* d_in = L.d_in.p + l.in_off;
-        const uint8_t* win = J.srcs[i] + (size_t)p->win_y * J.src_steps[i] + (size_t)p->win_x * sc;
-        if (J.src_device) {
-            B.items.push_back(imp_gpu_batch::Item{p, J.srcs[i], J.src_steps[i], L.d_out.p + l.out_off, l.out_pitch});
+        uint8_t* d_out = L.d_out.p + l.out_off;
+        const uint8_t* rows = j.src + (size_t)p->win_y * j.src_step;          // the rows the crop window touches
+        switch (l.src) {
+        case ImpRoute::Resident:
+            B.items.push_back(imp_gpu_batch::Item{p, j.src, j.src_step, d_out, l.out_pitch});
             continue;
-        }
-        if (!l.src_pinned) {
+        case ImpRoute::Staged: {
             // a pageable frame (what cvDecodeImage hands RunJob) goes through the lane's pinned staging, laid out with the
-            // device pitch, by several cores at once (stage_threads above)
+            // device pitch, by several cores at once (stage_threads above), in row slices each uploaded once staged
             uint8_t* h = L.h_in.p + l.hin_off;
-            const int step = J.src_steps[i], pitch = l.in_pitch;
-            auto stage_rows = [=](int y0, int y1) {
-                if ((size_t)step == (size_t)pitch && in_row == (size_t)pitch) copy_stream(h + (size_t)y0 * pitch, win + (size_t)y0 * step, (size_t)pitch * (y1 - y0));
-                else for (int y = y0; y < y1; y++) copy_stream(h + (size_t)y * pitch, win + (size_t)y * step, in_row);
-            };
-            // in slices of rows, each uploaded as soon as it is staged: the copy engine works on slice k while the cores stage
-            // slice k+1 (a lone request — one nginx worker — has no other job's upload to overlap its staging with)
-            const size_t bytes = in_row * p->win_h;
-            const int slices = std::min(p->win_h, (m > 1 || bytes < (16u << 20)) ? 1 : 4);      // cfg2's 29 MB window: 1.16 -> 1.04 ms; smaller ones do not repay the extra dispatches
-            for (int sidx = 0; sidx < slices; sidx++) {
-                const int r0 = (int)((long long)p->win_h * sidx / slices), r1 = (int)((long long)p->win_h * (sidx + 1) / slices);
-                run_parts(r1 - r0, stage_parts(in_row * (size_t)(r1 - r0), r1 - r0), [=](int y0, int y1) { stage_rows(r0 + y0, r0 + y1); });
-                CK(cudaMemcpyAsync(d_in + (size_t)r0 * l.in_pitch, h + (size_t)r0 * l.in_pitch, (size_t)l.in_pitch * (r1 - r0), cudaMemcpyHostToDevice, L.st));    // already in the device layout
+            const uint8_t* win = rows + (size_t)p->win_x * sc;
+            for (int s = 0; s < l.slices; s++) {
+                const int r0 = (int)((long long)p->win_h * s / l.slices), r1 = (int)((long long)p->win_h * (s + 1) / l.slices);
+                run_parts(r1 - r0, stage_parts(in_row * (size_t)(r1 - r0), r1 - r0), [=, &j](int y0, int y1) {
+                    copy_rows(h + (size_t)(r0 + y0) * l.in_pitch, l.in_pitch, win + (size_t)(r0 + y0) * j.src_step, j.src_step, in_row, y1 - y0);
+                });
+                CK(cudaMemcpyAsync(d_in + (size_t)r0 * l.in_pitch, h + (size_t)r0 * l.in_pitch, (size_t)l.in_pitch * (r1 - r0), cudaMemcpyHostToDevice, L.st));
             }
-        } else if (l.linear) {
-            const uint8_t* h_lin = J.srcs[i] + (size_t)p->win_y * J.src_steps[i];
-            if (J.src_steps[i] == l.in_pitch && p->win_x == 0) {
-                CK(cudaMemcpyAsync(d_in, h_lin, l.lin_bytes, cudaMemcpyHostToDevice, L.st));
-            } else {
-                uint8_t* stage = L.d_stage.p + l.stage_off;
-                CK(cudaMemcpyAsync(stage, h_lin, l.lin_bytes, cudaMemcpyHostToDevice, L.st));
-                repitch.push_back(Repitch{stage + (size_t)p->win_x * sc, J.src_steps[i], d_in, l.in_pitch, (int)in_row, p->win_h});
-            }
-        } else {
-            CK(cudaMemcpy2DAsync(d_in, l.in_pitch, win, J.src_steps[i], in_row, p->win_h, cudaMemcpyHostToDevice, L.st));
+            break;
+        }
+        case ImpRoute::Linear:
+            CK(cudaMemcpyAsync(d_in, rows, l.lin_bytes, cudaMemcpyHostToDevice, L.st));
+            break;
+        case ImpRoute::LinearRepitch: {
+            uint8_t* stage = L.d_stage.p + l.stage_off;
+            CK(cudaMemcpyAsync(stage, rows, l.lin_bytes, cudaMemcpyHostToDevice, L.st));
+            repitch.push_back(Repitch{stage + (size_t)p->win_x * sc, j.src_step, d_in, l.in_pitch, (int)in_row, p->win_h});
+            break;
+        }
+        default:                                                               // Rows2D
+            CK(cudaMemcpy2DAsync(d_in, l.in_pitch, rows + (size_t)p->win_x * sc, j.src_step, in_row, p->win_h, cudaMemcpyHostToDevice, L.st));
         }
         // The device copy holds only the crop window; bias the base pointer so the pass's (sx0,sy0) lands on it.
         const uint8_t* biased = d_in - ((size_t)p->win_y * l.in_pitch + (size_t)p->win_x * sc);
-        B.items.push_back(imp_gpu_batch::Item{p, biased, l.in_pitch, L.d_out.p + l.out_off, l.out_pitch});
+        B.items.push_back(imp_gpu_batch::Item{p, biased, l.in_pitch, d_out, l.out_pitch});
     }
     if (L.up_done) CK(cudaEventRecord(L.up_done, L.st));
     for (const Repitch& q : repitch) CK(imp_launch_repitch(q.src, q.sp, q.dst, q.dp, q.row_bytes, q.rows, L.st));
     if ((r = batch_compile(&B, L.st))) return r;
     if ((r = launch_steps(B.steps, B.h_jobs, B.d_jobs, L.st))) return r;
-    if (J.result != HostJobs::Frame) {
-        std::vector<size_t> out_off(m); std::vector<int> out_pitch(m);
-        for (int k = 0; k < m; k++) { out_off[k] = lay[k].out_off; out_pitch[k] = lay[k].out_pitch; }
-        std::vector<long long> staged(m);
-        for (int k = 0; k < m; k++) staged[k] = lay[k].dst_pinned ? -1 : lay[k].hout_off;
-        return lane_answers(L, J, first, m, out_off, out_pitch, staged);
-    }
+    if (kind != ImpResult::Frame) return lane_answers(L, jobs, m, kind, lay);
     for (int k = 0; k < m; k++) {
-        const int i = first + k;
-        const imp_gpu_plan* p = J.plans[i];
-        const Lay& l = lay[k];
+        const ImpHostJob& j = jobs[k];
+        const ImpJobLayout& l = lay.jobs[k];
+        const imp_gpu_plan* p = j.plan;
         const size_t out_row = (size_t)p->out_w * p->out_c;
         const uint8_t* d_out = L.d_out.p + l.out_off;
-        if (l.dst_pinned) {
-            if ((size_t)J.dst_steps[i] == (size_t)l.out_pitch) CK(cudaMemcpyAsync(J.dsts[i], d_out, (size_t)l.out_pitch * (p->out_h - 1) + out_row, cudaMemcpyDeviceToHost, L.st));
-            else CK(cudaMemcpy2DAsync(J.dsts[i], J.dst_steps[i], d_out, l.out_pitch, out_row, p->out_h, cudaMemcpyDeviceToHost, L.st));
-        } else {
+        if (l.dst == ImpRoute::Linear) CK(cudaMemcpyAsync(j.dst, d_out, (size_t)l.out_pitch * (p->out_h - 1) + out_row, cudaMemcpyDeviceToHost, L.st));
+        else if (l.dst == ImpRoute::Rows2D) CK(cudaMemcpy2DAsync(j.dst, j.dst_step, d_out, l.out_pitch, out_row, p->out_h, cudaMemcpyDeviceToHost, L.st));
+        else {
             CK(cudaMemcpy2DAsync(L.h_out.p + l.hout_off, out_row, d_out, l.out_pitch, out_row, p->out_h, cudaMemcpyDeviceToHost, L.st));
+            L.pend.push_back(Lane::Out{j.dst, (size_t)j.dst_step, out_row, p->out_h, l.hout_off});
         }
-        L.pend.push_back(Lane::Out{i, l.hout_off});
     }
     return IMP_OK;
 }
 
-// `after`: an event every lane waits for before its first chunk (the producer of device-resident sources). Caller holds run_mu.
-int run_host_chunked_locked(const HostJobs& J, int n_streams, cudaEvent_t after) {
+// Runs jobs [0, n) over n_streams lanes of the current device. `resident`: the sources are already on the device;
+// `after`: an event every lane waits for before its first chunk (their producer). Caller holds run_mu.
+int run_host_chunked_locked(const ImpHostJob* jobs, int n, ImpResult kind, int n_streams, bool resident, cudaEvent_t after) {
     DevCtx& ctx = g_dev[t_dev];
     n_streams = std::max(1, std::min(n_streams, 8));
     while ((int)ctx.lanes.size() < n_streams) {
@@ -896,43 +823,57 @@ int run_host_chunked_locked(const HostJobs& J, int n_streams, cudaEvent_t after)
         if (e != cudaSuccess) { cudaStreamDestroy(L->st); delete L; return fail(e, "cudaEventCreateWithFlags", __LINE__); }
         ctx.lanes.push_back(L);
     }
-    int result = IMP_OK, chunk = 0, i = 0;
     if (after) for (int k = 0; k < n_streams; k++) CK(cudaStreamWaitEvent(ctx.lanes[k]->st, after, 0));
-    // Uploads of different lanes issued together are time-sliced by the copy engines: every chunk's upload then ends at the
-    // END of all uploads and nothing overlaps the way back (a same-size request moved 26 GB/s per direction where the duplex
-    // link gives 48). Each chunk's uploads therefore wait for the previous chunk's — they run back to back in chunk order,
-    // kernels and downloads of earlier chunks alongside — and a call is cut into at least 2 chunks per lane when its bytes
-    // allow (>= 4 MB per chunk), so that the pipeline has stages to overlap. IMP_GPU_CHAIN_H2D=0 turns both off (tuning knob).
-    static const bool chain = [] { const char* e = getenv("IMP_GPU_CHAIN_H2D"); return !e || atoi(e) != 0; }();
-    size_t total_bytes = 0;
-    for (int k = 0; k < J.n; k++) if (J.plans[k]) total_bytes += (size_t)align16(J.plans[k]->win_w * J.plans[k]->src_c) * J.plans[k]->win_h + (size_t)J.plans[k]->out_w * J.plans[k]->out_c * J.plans[k]->out_h;
-    const size_t chunk_bytes = chain ? std::min(kChunkBytes, std::max<size_t>(4u << 20, total_bytes / (2 * (size_t)n_streams))) : kChunkBytes;
-    Lane* prev = nullptr;
-    while (i < J.n && result == IMP_OK) {
-        Lane& L = *ctx.lanes[chunk % n_streams];
-        if ((result = lane_finish(L, J))) break;
-        if (chain && prev && prev != &L && !J.src_device) CK(cudaStreamWaitEvent(L.st, prev->up_done, 0));
-        prev = &L;
-        int e = i; size_t bytes = 0;
-        // small batches are spread over the lanes instead of filling one chunk, so that copies and kernels still overlap
-        const int max_jobs = std::max(1, std::min(kChunkJobs, (J.n + n_streams - 1) / n_streams));
-        while (e < J.n && e - i < max_jobs) {
-            const imp_gpu_plan* p = J.plans[e];
-            if (!p) break;
-            const size_t need = (size_t)align16(p->win_w * p->src_c) * p->win_h + (chain ? (size_t)p->out_w * p->out_c * p->out_h : 0);
-            if (e > i && bytes + need > chunk_bytes) break;
-            bytes += need; e++;
+    int result = IMP_OK;
+    try {
+        const std::vector<int> bounds = imp_chunk_bounds(jobs, n, n_streams);
+        Lane* prev = nullptr;
+        for (size_t c = 0; c + 1 < bounds.size() && result == IMP_OK; c++) {
+            Lane& L = *ctx.lanes[c % n_streams];
+            if ((result = lane_finish(L))) break;
+            // each chunk's uploads wait for the previous chunk's: they run back to back in chunk order (imp_chunk_bounds)
+            if (prev && prev != &L && !resident) CK(cudaStreamWaitEvent(L.st, prev->up_done, 0));
+            prev = &L;
+            result = lane_issue(L, jobs + bounds[c], bounds[c + 1] - bounds[c], kind, resident);
         }
-        if (e == i) { result = IMP_ERROR_INVALID_ARGS; break; }
-        try { result = lane_issue(L, J, i, e); } catch (const std::bad_alloc&) { result = IMP_ERROR_MALLOC_FAILED; }
-        i = e; chunk++;
-    }
-    for (Lane* L : ctx.lanes) { int r = lane_finish(*L, J); if (result == IMP_OK) result = r; }
+    } catch (const std::bad_alloc&) { result = IMP_ERROR_MALLOC_FAILED; }
+    for (Lane* L : ctx.lanes) { int r = lane_finish(*L); if (result == IMP_OK) result = r; }
     return result;
 }
-int run_host_chunked(const HostJobs& J, int n_streams) {
+int run_host_chunked(const std::vector<ImpHostJob>& jobs, ImpResult kind, int n_streams) {
     std::lock_guard<std::mutex> run_lk(g_dev[t_dev].run_mu);
-    return run_host_chunked_locked(J, n_streams, nullptr);
+    return run_host_chunked_locked(jobs.data(), (int)jobs.size(), kind, n_streams, false, nullptr);
+}
+
+// Every job of a host call is checked before any work starts, so a bad one leaves every output as it was. A packed
+// (bottom-up) result would reverse an answer's text, and the JSON and text exits never reach the FreeImage packer.
+// text_caps: ASCII only, the capacity of each text.
+int check_host_jobs(ImpResult kind, const std::vector<ImpHostJob>& jobs, const long* text_caps = nullptr) {
+    for (size_t i = 0; i < jobs.size(); i++) {
+        const ImpHostJob& j = jobs[i];
+        const imp_gpu_plan* p = j.plan;
+        if (!p || !j.src || !j.dst || (long long)j.src_step < (long long)p->src_w * p->src_c) return IMP_ERROR_INVALID_ARGS;
+        if (kind == ImpResult::Frame ? (long long)j.dst_step < (long long)p->out_w * p->out_c : p->pack != IMP_PACK_NONE) return IMP_ERROR_INVALID_ARGS;
+        if (kind == ImpResult::Ascii && text_caps[i] < imp_gpu_ascii_length(p->out_w, p->out_h)) return IMP_ERROR_INVALID_ARGS;
+    }
+    return IMP_OK;
+}
+
+// The job list of a host call (answers fill in dst themselves).
+std::vector<ImpHostJob> host_jobs(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                                  unsigned char* const* dsts = nullptr, const int* dst_steps = nullptr) {
+    std::vector<ImpHostJob> v(n);
+    for (int i = 0; i < n; i++) v[i] = ImpHostJob{plans[i], srcs[i], src_steps[i], dsts ? dsts[i] : nullptr, dst_steps ? dst_steps[i] : 0, false};
+    return v;
+}
+
+// The checks imp_gpu_run_device and imp_gpu_batch_add make on a device job.
+int check_device_job(const imp_gpu_plan* plan, const void* d_src, int sp, const void* d_dst, int dp) {
+    if (!plan || !d_src || !d_dst) return IMP_ERROR_INVALID_ARGS;
+    if (sp < plan->src_w * plan->src_c || dp < plan->out_w * plan->out_c) return IMP_ERROR_INVALID_ARGS;
+    if (plan->out_c == 4 && (dp % 4 || ((uintptr_t)d_dst) % 4)) return IMP_ERROR_INVALID_ARGS;
+    if (plan->src_c == 4 && (sp % 4 || ((uintptr_t)d_src) % 4)) return IMP_ERROR_INVALID_ARGS;
+    return IMP_OK;
 }
 
 }  // namespace
@@ -941,7 +882,7 @@ struct imp_gpu_ticket {
     std::thread th;
     int rc = IMP_OK; std::string err;
     std::atomic<bool> done{false};
-    std::vector<imp_gpu_plan*> plans; std::vector<const unsigned char*> srcs; std::vector<unsigned char*> dsts; std::vector<int> ss, ds;
+    std::vector<ImpHostJob> jobs;
 };
 
 extern "C" {
@@ -1145,10 +1086,8 @@ unsigned long long imp_gpu_batch_algorithmic_bytes(const imp_gpu_batch* b) { ret
 int imp_gpu_batch_launches_per_run(const imp_gpu_batch* b) { return b->launches; }
 
 int imp_gpu_batch_add(imp_gpu_batch* b, imp_gpu_plan* plan, const void* d_src, int sp, void* d_dst, int dp) {
-    if (!b || !plan || !d_src || !d_dst) return IMP_ERROR_INVALID_ARGS;
-    if (sp < plan->src_w * plan->src_c || dp < plan->out_w * plan->out_c) return IMP_ERROR_INVALID_ARGS;
-    if (plan->out_c == 4 && (dp % 4 || ((uintptr_t)d_dst) % 4)) return IMP_ERROR_INVALID_ARGS;
-    if (plan->src_c == 4 && (sp % 4 || ((uintptr_t)d_src) % 4)) return IMP_ERROR_INVALID_ARGS;
+    if (!b) return IMP_ERROR_INVALID_ARGS;
+    if (int rc = check_device_job(plan, d_src, sp, d_dst, dp)) return rc;
     try { b->items.push_back(imp_gpu_batch::Item{plan, (const uint8_t*)d_src, sp, (uint8_t*)d_dst, dp}); }
     catch (...) { return IMP_ERROR_MALLOC_FAILED; }
     b->dirty = true;
@@ -1170,10 +1109,7 @@ int imp_gpu_batch_launch(imp_gpu_batch* b, void* stream) {
 // ---- one frame -----------------------------------------------------------------------------------------
 int imp_gpu_run_device(imp_gpu_plan* plan, const void* d_src, int sp, void* d_dst, int dp, void* stream) {
     int rc = bind(); if (rc) return rc;
-    if (!plan || !d_src || !d_dst) return IMP_ERROR_INVALID_ARGS;
-    if (sp < plan->src_w * plan->src_c || dp < plan->out_w * plan->out_c) return IMP_ERROR_INVALID_ARGS;
-    if (plan->out_c == 4 && (dp % 4 || ((uintptr_t)d_dst) % 4)) return IMP_ERROR_INVALID_ARGS;
-    if (plan->src_c == 4 && (sp % 4 || ((uintptr_t)d_src) % 4)) return IMP_ERROR_INVALID_ARGS;
+    if ((rc = check_device_job(plan, d_src, sp, d_dst, dp))) return rc;
     if ((rc = plan_to_device(plan))) return rc;
     cudaStream_t st = pick_stream(stream);
     if ((rc = plan_wait_ready(plan, st))) return rc;
@@ -1208,12 +1144,16 @@ int imp_gpu_batch_run_host(int n, imp_gpu_plan* const* plans, const unsigned cha
     int rc = bind(); if (rc) return rc;
     if (n <= 0) return IMP_OK;
     if (!plans || !srcs || !src_steps || !dsts || !dst_steps) return IMP_ERROR_INVALID_ARGS;
-    const HostJobs J{n, plans, srcs, src_steps, dsts, dst_steps};
-    try { return run_host_chunked(J, n_streams); } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+    try {
+        const std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps, dsts, dst_steps);
+        if ((rc = check_host_jobs(ImpResult::Frame, jobs))) return rc;
+        return run_host_chunked(jobs, ImpResult::Frame, n_streams);
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
 
-// Asynchronous form: the call returns at once, a helper thread of the library drives the batch on the caller's current
-// device, imp_gpu_batch_wait() joins it. The argument arrays are copied; the pixel buffers must stay valid until the wait.
+// Asynchronous form: the jobs are checked, then the call returns, a helper thread of the library drives the batch on the
+// caller's current device, imp_gpu_batch_wait() joins it. The argument arrays are copied; the pixel buffers must stay valid
+// until the wait.
 int imp_gpu_batch_submit_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                               unsigned char* const* dsts, const int* dst_steps, int n_streams, imp_gpu_ticket** ticket) {
     if (!ticket) return IMP_ERROR_INVALID_ARGS;
@@ -1223,19 +1163,21 @@ int imp_gpu_batch_submit_host(int n, imp_gpu_plan* const* plans, const unsigned 
     imp_gpu_ticket* t = nullptr;
     try {
         t = new imp_gpu_ticket();
-        t->plans.assign(plans, plans + n); t->srcs.assign(srcs, srcs + n); t->dsts.assign(dsts, dsts + n);
-        t->ss.assign(src_steps, src_steps + n); t->ds.assign(dst_steps, dst_steps + n);
-        for (imp_gpu_plan* p : t->plans) if (p) p->refs.fetch_add(1);          // the batch keeps its plans alive
+        t->jobs = host_jobs(n, plans, srcs, src_steps, dsts, dst_steps);
+        if ((rc = check_host_jobs(ImpResult::Frame, t->jobs))) { delete t; return rc; }
+        for (const ImpHostJob& j : t->jobs) j.plan->refs.fetch_add(1);       // the batch keeps its plans alive
         const int dev = t_dev;
-        t->th = std::thread([t, dev, n, n_streams]() {
+        t->th = std::thread([t, dev, n_streams]() {
             int r = imp_gpu_set_device(dev);
-            if (r == IMP_OK) r = imp_gpu_batch_run_host(n, t->plans.data(), t->srcs.data(), t->ss.data(), t->dsts.data(), t->ds.data(), n_streams);
+            if (r == IMP_OK && !t->jobs.empty()) {
+                try { r = run_host_chunked(t->jobs, ImpResult::Frame, n_streams); } catch (const std::bad_alloc&) { r = IMP_ERROR_MALLOC_FAILED; }
+            }
             t->rc = r;
             if (r) t->err = t_err;
             t->done.store(true, std::memory_order_release);
         });
     } catch (...) {
-        if (t) { for (imp_gpu_plan* p : t->plans) if (p) plan_release(p); delete t; }
+        if (t) { for (const ImpHostJob& j : t->jobs) plan_release(j.plan); delete t; }
         return IMP_ERROR_MALLOC_FAILED;
     }
     *ticket = t;
@@ -1249,7 +1191,7 @@ int imp_gpu_batch_wait(imp_gpu_ticket* ticket) {
     if (ticket->th.joinable()) ticket->th.join();
     const int rc = ticket->rc;
     if (rc) snprintf(t_err, sizeof t_err, "%s", ticket->err.c_str());
-    for (imp_gpu_plan* p : ticket->plans) if (p) plan_release(p);
+    for (const ImpHostJob& j : ticket->jobs) plan_release(j.plan);
     delete ticket;
     return rc;
 }
@@ -1280,17 +1222,19 @@ int imp_gpu_farm_assign(int n, imp_gpu_plan* const* plans, int n_gpus, int polic
 // algorithmic bytes so far (mixed-size farms: evens out the bytes per GPU).
 int imp_gpu_farm_run_host_policy(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                                  unsigned char* const* dsts, const int* dst_steps, int n_gpus, int n_streams, int policy) {
-    if (n_gpus <= 0 || (policy != IMP_FARM_ROUND_ROBIN && policy != IMP_FARM_SIZE_AWARE)) return IMP_ERROR_INVALID_ARGS;
+    if (n < 0 || n_gpus <= 0 || (policy != IMP_FARM_ROUND_ROBIN && policy != IMP_FARM_SIZE_AWARE)) return IMP_ERROR_INVALID_ARGS;
     if (n > 0 && (!plans || !srcs || !src_steps || !dsts || !dst_steps)) return IMP_ERROR_INVALID_ARGS;
     const int avail = imp_gpu_device_count();
     if (avail <= 0) return fail_msg("no CUDA device available; libimp_gpu has no CPU fallback");
     if (n_gpus > avail || n_gpus > MAX_DEV) return fail_msg("imp_gpu_farm_run_host: more GPUs requested than present");
-    std::vector<std::vector<int>> share(n_gpus);
+    std::vector<std::vector<ImpHostJob>> share(n_gpus);
     try {
-        std::vector<int> owner(std::max(n, 1));
-        int rc = imp_gpu_farm_assign(n, plans, n_gpus, policy, owner.data());
+        const std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps, dsts, dst_steps);
+        int rc = check_host_jobs(ImpResult::Frame, jobs);
         if (rc) return rc;
-        for (int i = 0; i < n; i++) share[owner[i]].push_back(i);          // each GPU walks its jobs in request order
+        std::vector<int> owner(std::max(n, 1));
+        if ((rc = imp_gpu_farm_assign(n, plans, n_gpus, policy, owner.data()))) return rc;
+        for (int i = 0; i < n; i++) share[owner[i]].push_back(jobs[i]);    // each GPU walks its jobs in request order
     } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
     std::vector<int> rcs(n_gpus, IMP_OK);
     std::vector<std::string> errs(n_gpus);
@@ -1299,10 +1243,8 @@ int imp_gpu_farm_run_host_policy(int n, imp_gpu_plan* const* plans, const unsign
     for (int g = 0; g < n_gpus; g++) {
         th.emplace_back([&, g]() {
             int rc = imp_gpu_set_device(g);
-            if (rc == IMP_OK) {
-                std::vector<imp_gpu_plan*> pl; std::vector<const unsigned char*> sr; std::vector<unsigned char*> ds; std::vector<int> ss, dd;
-                for (int i : share[g]) { pl.push_back(plans[i]); sr.push_back(srcs[i]); ds.push_back(dsts[i]); ss.push_back(src_steps[i]); dd.push_back(dst_steps[i]); }
-                if (!pl.empty()) rc = imp_gpu_batch_run_host((int)pl.size(), pl.data(), sr.data(), ss.data(), ds.data(), dd.data(), n_streams);
+            if (rc == IMP_OK && !share[g].empty()) {
+                try { rc = run_host_chunked(share[g], ImpResult::Frame, n_streams); } catch (const std::bad_alloc&) { rc = IMP_ERROR_MALLOC_FAILED; }
             }
             rcs[g] = rc;
             if (rc) errs[g] = t_err;
@@ -1320,42 +1262,32 @@ int imp_gpu_farm_run_host(int n, imp_gpu_plan* const* plans, const unsigned char
 }
 
 // ---- format=json / format=text without the frames: brightness and ASCII of the results, reduced on the device ---------
-namespace {
-// Every job is checked before any work starts: nothing is written when one is unusable. A packed (bottom-up) result would
-// reverse the text, and the JSON and text exits never reach the FreeImage packer.
-int check_answer_jobs(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps) {
-    if (!plans || !srcs || !src_steps) return IMP_ERROR_INVALID_ARGS;
-    for (int i = 0; i < n; i++)
-        if (!plans[i] || !srcs[i] || plans[i]->pack != IMP_PACK_NONE) return IMP_ERROR_INVALID_ARGS;
-    return IMP_OK;
-}
-}  // namespace
-
 int imp_gpu_batch_brightness_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                                   float* brightness, int n_streams) {
     int rc = bind(); if (rc) return rc;
     if (n <= 0) return IMP_OK;
-    if ((rc = check_answer_jobs(n, plans, srcs, src_steps))) return rc;
-    if (!brightness) return IMP_ERROR_INVALID_ARGS;
-    HostJobs J{n, plans, srcs, src_steps, nullptr, nullptr};
-    J.result = HostJobs::Brightness; J.brightness = brightness;
-    try { return run_host_chunked(J, n_streams); } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+    if (!plans || !srcs || !src_steps || !brightness) return IMP_ERROR_INVALID_ARGS;
+    try {
+        std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps);
+        for (int i = 0; i < n; i++) jobs[i].dst = reinterpret_cast<uint8_t*>(brightness + i);
+        if ((rc = check_host_jobs(ImpResult::Brightness, jobs))) return rc;
+        return run_host_chunked(jobs, ImpResult::Brightness, n_streams);
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
 
 int imp_gpu_batch_ascii_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                              const char* const* args, unsigned char* const* texts, const long* text_caps, int n_streams) {
     int rc = bind(); if (rc) return rc;
     if (n <= 0) return IMP_OK;
-    if ((rc = check_answer_jobs(n, plans, srcs, src_steps))) return rc;
-    if (!args || !texts || !text_caps) return IMP_ERROR_INVALID_ARGS;
-    for (int i = 0; i < n; i++)
-        if (!texts[i] || text_caps[i] < imp_gpu_ascii_length(plans[i]->out_w, plans[i]->out_h)) return IMP_ERROR_INVALID_ARGS;
+    if (!plans || !srcs || !src_steps || !args || !texts || !text_caps) return IMP_ERROR_INVALID_ARGS;
     try {
-        std::vector<unsigned char> wide(n);
-        for (int i = 0; i < n; i++) wide[i] = args[i] && strcmp(args[i], "wide") == 0;        // filters.c:490-494
-        HostJobs J{n, plans, srcs, src_steps, nullptr, nullptr};
-        J.result = HostJobs::Ascii; J.texts = texts; J.wide = wide.data();
-        return run_host_chunked(J, n_streams);
+        std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps);
+        for (int i = 0; i < n; i++) {
+            jobs[i].dst = texts[i];
+            jobs[i].wide = args[i] && strcmp(args[i], "wide") == 0;                  // filters.c:490-494
+        }
+        if ((rc = check_host_jobs(ImpResult::Ascii, jobs, text_caps))) return rc;
+        return run_host_chunked(jobs, ImpResult::Ascii, n_streams);
     } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
 
@@ -1396,8 +1328,6 @@ int imp_gpu_brightness_host(const unsigned char* img, int step, int w, int h, in
     cudaFreeAsync(d, st);
     return rc;
 }
-
-long imp_gpu_ascii_length(int width, int height) { return (long)(width + 1) * height - 1; }
 
 int imp_gpu_ascii_host(const unsigned char* img, int step, int w, int h, int c, const char* args, unsigned char* out, long out_cap) {
     int rc = bind(); if (rc) return rc;
@@ -1481,36 +1411,35 @@ int imp_gpu_gif_album_run_host(const imp_gpu_gif_frame* frames, int n, int canva
                                imp_gpu_plan* const* plans, unsigned char* const* dsts, const int* dst_steps, int n_streams) {
     int rc = bind(); if (rc) return rc;
     if (!frames || n <= 0 || canvas_w <= 0 || canvas_h <= 0 || !plans || !dsts || !dst_steps) return IMP_ERROR_INVALID_ARGS;
-    int n_run = 0;
     for (int f = 0; f < n; f++) {
-        const imp_gpu_plan* p = plans[f];
-        if (!p) continue;                                             // replayed for the pages after it, no result wanted
-        if (!dsts[f] || p->src_w != canvas_w || p->src_h != canvas_h || p->src_c != 4) return IMP_ERROR_INVALID_ARGS;
-        if ((size_t)dst_steps[f] < (size_t)p->out_w * p->out_c) return IMP_ERROR_INVALID_ARGS;
-        n_run++;
+        const imp_gpu_plan* p = plans[f];                             // null: replayed for the pages after it, no result wanted
+        if (p && (p->src_w != canvas_w || p->src_h != canvas_h || p->src_c != 4)) return IMP_ERROR_INVALID_ARGS;
     }
     size_t meta_bytes = 0, total = 0;
     if ((rc = gif_validate(frames, n, &meta_bytes, &total))) return rc;
-    DevCtx& ctx = g_dev[t_dev];
-    std::lock_guard<std::mutex> run_lk(ctx.run_mu);
     const int pitch = align16(canvas_w * 4);
     const size_t canvas_bytes = (size_t)pitch * canvas_h;
+    // a frame's source is its page's canvas; the page stands in for it until the canvases are allocated, so that a bad job
+    // is refused before any buffer grows
+    std::vector<ImpHostJob> jobs;
+    try {
+        for (int f = 0; f < n; f++)
+            if (plans[f]) jobs.push_back(ImpHostJob{plans[f], frames[f].indices, pitch, dsts[f], dst_steps[f], false});
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+    if ((rc = check_host_jobs(ImpResult::Frame, jobs))) return rc;
+    DevCtx& ctx = g_dev[t_dev];
+    std::lock_guard<std::mutex> run_lk(ctx.run_mu);
     if ((rc = ctx.h_gif.grow(total, true)) || (rc = ctx.d_gif.grow(total, false)) || (rc = ctx.d_canvas.grow(canvas_bytes * n, false))) return rc;
     if (!ctx.gif_ev) CK(cudaEventCreateWithFlags(&ctx.gif_ev, cudaEventDisableTiming));
+    for (int f = 0, k = 0; f < n; f++)
+        if (plans[f]) jobs[k++].src = ctx.d_canvas.p + (size_t)f * canvas_bytes;
     try {                                                             // the C caller cannot unwind: bad_alloc ends as a code
     gif_pack(frames, n, meta_bytes, ctx.h_gif.p, ctx.d_gif.p);
     CK(cudaMemcpyAsync(ctx.d_gif.p, ctx.h_gif.p, total, cudaMemcpyHostToDevice, ctx.stream));
     CK(imp_launch_gif_expand(reinterpret_cast<const ImpGifFrame*>(ctx.d_gif.p), n, canvas_w, canvas_h, destructive ? 1 : 0, ctx.d_canvas.p, pitch, ctx.stream));
     CK(cudaEventRecord(ctx.gif_ev, ctx.stream));
-    std::vector<imp_gpu_plan*> run_plans; std::vector<const unsigned char*> srcs; std::vector<unsigned char*> outs; std::vector<int> steps, out_steps;
-    for (int f = 0; f < n; f++) {
-        if (!plans[f]) continue;
-        run_plans.push_back(plans[f]); srcs.push_back(ctx.d_canvas.p + (size_t)f * canvas_bytes); steps.push_back(pitch);
-        outs.push_back(dsts[f]); out_steps.push_back(dst_steps[f]);
-    }
-    if (n_run == 0) { CK(cudaStreamSynchronize(ctx.stream)); return IMP_OK; }
-    HostJobs J{n_run, run_plans.data(), srcs.data(), steps.data(), outs.data(), out_steps.data(), true};
-    rc = run_host_chunked_locked(J, n_streams, ctx.gif_ev);
+    if (jobs.empty()) { CK(cudaStreamSynchronize(ctx.stream)); return IMP_OK; }
+    rc = run_host_chunked_locked(jobs.data(), (int)jobs.size(), ImpResult::Frame, n_streams, true, ctx.gif_ev);
     } catch (const std::bad_alloc&) { rc = IMP_ERROR_MALLOC_FAILED; }
     if (rc != IMP_OK) cudaStreamSynchronize(ctx.stream);           // the staging buffers are reused by the next call
     return rc;

@@ -94,6 +94,49 @@ struct imp_gpu_plan {
 int imp_build_plan(const imp_gpu_request* req, const imp_gpu_config* cfg, int w, int h, int c,
                    imp_gpu_plan* plan, int* step, bool dry = false);
 
+inline int align16(int v) { return (v + 15) & ~15; }
+inline size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
+
+// ---- host jobs and how they cross the link (imp_transfer.cpp: pure host logic, no CUDA call) ----------------------
+// One job of the chunked host path. A frame result goes to (dst, dst_step); an answer is a one-row result: brightness
+// writes 4 bytes (a float) at dst, ASCII imp_gpu_ascii_length bytes with the 70-level ramp where `wide`.
+struct ImpHostJob { imp_gpu_plan* plan; const uint8_t* src; int src_step; uint8_t* dst; int dst_step; bool wide; };
+enum class ImpResult { Frame, Brightness, Ascii };
+constexpr int IMP_CHUNK_JOBS = 256;                  // the most jobs a chunk holds
+constexpr size_t IMP_CHUNK_BYTES = 128u << 20;       // the most crop-window + result bytes a chunk holds (one job may exceed it)
+// The chunk boundaries [0, e1, ..., n] of n jobs over n_streams lanes (clamped to 1..8).
+std::vector<int> imp_chunk_bounds(const ImpHostJob* jobs, int n, int n_streams);
+
+// How a job's source reaches the device and its result the host.
+enum class ImpRoute : uint8_t {
+    Resident,        // source: already on this device (GIF canvases), nothing to upload
+    Staged,          // pageable host memory, through the lane's pinned staging (h_in / h_out)
+    Linear,          // pinned: one linear copy (source: into d_in at the device pitch; frame result: out of d_out)
+    LinearRepitch,   // pinned source of short rows: one linear copy of the rows the window touches into d_stage, then a
+                     // re-pitch kernel into d_in
+    Rows2D,          // pinned: one 2-D copy
+    Direct,          // pinned answer: straight from the device into the destination
+};
+struct ImpJobLayout {
+    ImpRoute src, dst;
+    int in_pitch, out_pitch;     // device pitches of the crop window (d_in) and of the result (d_out)
+    size_t in_off, out_off;      // d_in, d_out
+    size_t lin_bytes;            // Linear, LinearRepitch sources: bytes of the one copy
+    size_t stage_off;            // LinearRepitch: d_stage
+    size_t hin_off;              // Staged source: h_in, rows at in_pitch
+    size_t hout_off;             // Staged result: h_out, frame rows packed at out_w*out_c
+    size_t res_bytes;            // bytes handed to the host: the frame's rows, 4 (brightness) or the text's length
+    int slices;                  // Staged source: uploaded in this many row slices (each as soon as it is staged)
+};
+struct ImpChunkLayout {
+    std::vector<ImpJobLayout> jobs;
+    size_t in_total = 0, out_total = 0, stage_total = 0, hin_total = 0, hout_total = 0;   // buffer sizes the chunk needs
+};
+// The routes and offsets of a chunk of m jobs. `resident`: every source is already on the device; src_pinned[k] /
+// dst_pinned[k]: whether job k's source / destination is page-locked (brightness: dst_pinned[0] decides for the chunk,
+// whose floats come back in one copy).
+ImpChunkLayout imp_chunk_layout(const ImpHostJob* jobs, int m, ImpResult kind, bool resident, const bool* src_pinned, const bool* dst_pinned);
+
 // imp_kernels.cu
 #define IMP_CUBIC_RUN 8           // imp_cubic_run_kernel: output rows per thread; a CTA covers 32 x (8 * IMP_CUBIC_RUN) pixels
 unsigned long long imp_launches();

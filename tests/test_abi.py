@@ -58,6 +58,14 @@ def test_validation_needs_no_gpu_and_matches_reference_codes():
     plan.close()
 
 
+def test_farm_rejects_a_negative_job_count():
+    """A negative n is an argument error (with or without a device), never an exception escaping the C ABI."""
+    L = M.library()
+    for fn in (L.lib.imp_gpu_farm_run_host_policy, L.lib.imp_gpu_farm_run_host):
+        extra = (1, 4, 0) if fn is L.lib.imp_gpu_farm_run_host_policy else (1, 4)
+        assert fn(-1, None, None, None, None, None, *extra) == M.IMP_ERROR_INVALID_ARGS
+
+
 def test_no_cpu_fallback_without_a_gpu():
     """On a box without a GPU every compute entry point must fail with IMP_ERROR_GPU, never produce pixels."""
     L = M.library()

@@ -449,3 +449,48 @@ def test_pageable_frames_at_odd_addresses_and_strides(gpu, orc):
                 gap = np.lib.stride_tricks.as_strided(o[off + 5 + orow:], shape=(p.out_h - 1, ostep - orow), strides=(ostep, 1))
                 assert not gap.any() and not o[:off + 5].any()              # nothing written between or before the rows
             p.close()
+
+
+@pytest.mark.parametrize("case", ["null_plan", "short_src_step", "short_dst_step"])
+def test_a_bad_job_is_refused_before_any_output_is_written(gpu, case):
+    """Every host entry point checks all its jobs before it stages, copies or writes anything: a NULL plan in a later chunk
+    than the first (job 39 of 40 on 4 lanes, chunks of 10 jobs), a source step shorter than a source row, or a frame
+    destination step shorter than a result row (a pageable destination would otherwise be written past its end) return
+    IMP_ERROR_INVALID_ARGS with every output as it was."""
+    import ctypes as C
+    import ngx_http_imgproc_b200 as M
+    L = gpu.lib
+    n, bad = 40, 39
+    imgs = [rnd_image(200 + i, 48, 64, 3) for i in range(n)]
+    plan = gpu.plan(64, 48, 3, api.Config(max_w=0, max_h=0), resize="32,24")
+    row = plan.out_w * plan.out_c
+    dsts = [np.full((plan.out_h, row), 0x5a, np.uint8) for _ in range(n)]
+    P = (C.c_void_p * n)(*[None if (case == "null_plan" and i == bad) else plan.h for i in range(n)])
+    S = (C.c_void_p * n)(*[im.ctypes.data for im in imgs])
+    SS = (C.c_int * n)(*[im.strides[0] - (1 if (case == "short_src_step" and i == bad) else 0) for i, im in enumerate(imgs)])
+    D = (C.c_void_p * n)(*[d.ctypes.data for d in dsts])
+    DS = (C.c_int * n)(*[row - (1 if (case == "short_dst_step" and i == bad) else 0) for i in range(n)])
+    INVALID = M.IMP_ERROR_INVALID_ARGS
+
+    def untouched():
+        return all((d == 0x5a).all() for d in dsts)
+
+    assert L.imp_gpu_batch_run_host(n, P, S, SS, D, DS, 4) == INVALID and untouched()
+    t = C.c_void_p()
+    assert L.imp_gpu_batch_submit_host(n, P, S, SS, D, DS, 4, C.byref(t)) == INVALID and not t.value and untouched()
+    assert L.imp_gpu_farm_run_host_policy(n, P, S, SS, D, DS, 1, 4, api.FARM_ROUND_ROBIN) == INVALID and untouched()
+    if case != "short_dst_step":                                            # answers have no destination step
+        b = np.full(n, -7.0, np.float32)
+        assert L.imp_gpu_batch_brightness_host(n, P, S, SS, b.ctypes.data, 4) == INVALID and (b == -7.0).all()
+        k = L.imp_gpu_ascii_length(plan.out_w, plan.out_h)
+        bufs = [C.create_string_buffer(b"\x5a" * k, k) for _ in range(n)]
+        T = (C.c_void_p * n)(*[C.addressof(x) for x in bufs])
+        A = (C.c_char_p * n)(*[b"wide"] * n)
+        caps = (C.c_long * n)(*[k] * n)
+        assert L.imp_gpu_batch_ascii_host(n, P, S, SS, A, T, caps, 4) == INVALID and all(x.raw == b"\x5a" * k for x in bufs)
+    # the same call without the bad job writes every result
+    P[bad], SS[bad], DS[bad] = plan.h.value, imgs[bad].strides[0], row
+    assert L.imp_gpu_batch_run_host(n, P, S, SS, D, DS, 4) == M.IMP_OK
+    ref = plan.run_host(imgs[0]).reshape(plan.out_h, row)
+    assert np.array_equal(dsts[0], ref) and not untouched()
+    plan.close()

@@ -151,8 +151,13 @@ unsigned long long imp_gpu_plan_algorithmic_bytes(const imp_gpu_plan* plan);
 /* Host buffers: H2D of the crop window, kernels, D2H; synchronous. dst must hold out_h rows of dst_step. */
 int  imp_gpu_run_host(imp_gpu_plan* plan, const unsigned char* src, int src_step,
                       unsigned char* dst, int dst_step);
-/* Device buffers (pitches multiples of 16, bases 16-byte aligned); asynchronous on `stream`
- * (a cudaStream_t passed as void*, NULL = the library's stream for this device). */
+/* Device buffers; asynchronous on `stream` (a cudaStream_t passed as void*, NULL = the library's stream for this
+ * device). Any pitch at least one row long (src_w*src_c, out_w*out_c bytes) and any base are accepted, except that
+ * 4-channel rows (a 4-channel source, a 4-channel or FI32 result) must have a pitch and a base that are multiples of 4;
+ * anything else returns IMP_ERROR_INVALID_ARGS. Only the out_w*out_c bytes of each result row are written, never the
+ * pitch padding. A source whose pitch is a multiple of 16 and whose image or crop window starts 16-byte aligned takes
+ * the shared-memory tile kernels; any other source the general kernels, with the same results. imp_gpu_batch_add takes
+ * the same buffers. */
 int  imp_gpu_run_device(imp_gpu_plan* plan, const void* d_src, int src_pitch,
                         void* d_dst, int dst_pitch, void* stream);
 

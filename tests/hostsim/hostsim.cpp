@@ -106,3 +106,21 @@ extern "C" void hostsim_plan_launch(const imp_gpu_plan* p, int k, int tiled, int
     const ImpLaunch& l = tiled ? p->passes[k].tiled : p->passes[k].fallback;
     out[0] = (int)l.kernel; out[1] = l.param; out[2] = l.flavour; out[3] = l.ctas_per_job; out[4] = l.smem_bytes; out[5] = l.ctas_per_sm;
 }
+// What decides the device code a job of pass k runs (the `tiled` launch when its source rows are 16-byte addressable, else
+// `fallback`): kind, sc, dc, kernel (ImpKernel), flavour, param, max_xtaps, nx, ny, gt, blur_r, the blur's effective tap
+// radius (zero outer taps trimmed, as the planner does before it pads to blur_r), tile_rs, tile_rows, tile_smem, smem_bytes.
+extern "C" void hostsim_plan_branch(const imp_gpu_plan* p, int k, int tiled, int* out) {
+    const ImpHostPass& hp = p->passes[k];
+    const ImpPass& h = hp.hdr;
+    const ImpLaunch& l = tiled ? hp.tiled : hp.fallback;
+    int r_eff = 0;
+    if (h.kind == IMP_G_BLUR) {
+        const int* t = (const int*)(hp.blob.data() + h.taps_off);
+        int lo = 0, hi = h.ksize - 1;
+        while (lo < hi && t[lo] == 0 && t[hi] == 0) { lo++; hi--; }
+        r_eff = (hi - lo) / 2;
+    }
+    const int v[16] = {h.kind, h.sc, h.dc, (int)l.kernel, l.flavour, l.param, h.max_xtaps, h.nx, h.ny, h.gt, h.blur_r, r_eff,
+                       h.tile_rs, h.tile_rows, h.tile_smem, l.smem_bytes};
+    memcpy(out, v, sizeof v);
+}

@@ -248,9 +248,9 @@ IMP_HD void imp_op_scanline(ImpPx& p, int y, int period, int freq, int sbyte, in
 }
 
 // filters.c:693-703 RadialGradient + helpers.c:46-48 Dist for one pixel.
-// dx*dx+dy*dy is exact in double, sqrt is correctly rounded, narrowing matches the reference; cos and
-// the 4th power are double, then narrowed (libm vs CUDA may differ in the last double ulp, which the
-// float narrowing hides except with probability ~2^-29: tested as <= 1 LSB).
+// dx*dx+dy*dy is exact in double, sqrt is correctly rounded, narrowing matches the reference; cos and the 4th power are
+// double, then narrowed: within 9.5 double ulp of cos^4 for glibc's cos+pow and CUDA's cos+2 squarings, so the float agrees
+// unless a float rounding boundary is that close (no such entry in any frame the tests use: tests/vignette_ref.py).
 #if defined(__CUDACC__)
 static __host__ __device__ __noinline__     // double cos + its slow path: large and rare, keep one copy per kernel
 #else

@@ -204,6 +204,10 @@ float orc_vignette_mask(int x, int y, int w, int h, float power, float radius) {
     float raw = distance / maxr * power;
     return (float)pow(cos((double)raw), 4);
 }
+/* orc_vignette_mask at |dx| = i < nx, |dy| = j < ny from the centre of a w x h frame, into out[j * nx + i]. */
+void orc_vignette_mask_table(float* out, int nx, int ny, int w, int h, float power, float radius) {
+    for (int j = 0; j < ny; j++) for (int i = 0; i < nx; i++) out[(long)j * nx + i] = orc_vignette_mask(w / 2 - i, h / 2 - j, w, h, power, radius);
+}
 /* filters.c:295-323 Vignette. */
 void orc_vignette(orc_img* im, float intensity, float radius) {
     int w = im->width, h = im->height, cx = w / 2, cy = h / 2;

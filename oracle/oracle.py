@@ -65,6 +65,7 @@ class _Orc:
         L = self.lib
         L.orc_vignette_mask.restype = C.c_float
         L.orc_vignette_mask.argtypes = [C.c_int] * 4 + [C.c_float] * 2
+        L.orc_vignette_mask_table.argtypes = [C.c_void_p] + [C.c_int] * 4 + [C.c_float] * 2
         L.orc_perceived_brightness.restype = C.c_float
         for n in ("orc_add_color",):
             getattr(L, n).argtypes = [C.c_void_p, C.c_void_p, C.c_float]
@@ -158,6 +159,12 @@ class _Orc:
 
     def vignette_mask(self, x, y, w, h, power, radius):
         return float(self.lib.orc_vignette_mask(x, y, w, h, C.c_float(power), C.c_float(radius)))
+
+    def vignette_mask_table(self, nx, ny, w, h, power, radius):
+        """vignette_mask at |dx| = i < nx, |dy| = j < ny from the frame's centre: float32 (ny, nx)."""
+        out = np.empty((ny, nx), np.float32)
+        self.lib.orc_vignette_mask_table(out.ctypes.data_as(C.c_void_p), nx, ny, w, h, C.c_float(power), C.c_float(radius))
+        return out
 
     # -- geometry ------------------------------------------------------------------------------
     def crop(self, img, x, y, w, h):

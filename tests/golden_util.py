@@ -1,4 +1,5 @@
 """Loads tests/golden/golden_v1.npz (made by tests/golden/make_golden.py from the compiled reference + cv2)."""
+import ctypes as C
 import hashlib
 import json
 import os
@@ -34,7 +35,114 @@ def split_query(query):
 
 
 # gradmap LUT tails the reference leaves uninitialised (SURVEY App. C-4): no golden case uses 4/6/7/8 colours.
-VIGNETTE_TOL = 1   # <= 1 LSB where libm's and CUDA's double cos may differ (DESIGN.md §Exactness)
+
+
+# ---- vignette: exact except at pixels whose mask rounding is ambiguous (tests/vignette_ref.py) -----------------------
+_HOSTSIM = []
+
+
+def _hostsim():
+    if not _HOSTSIM:
+        from conftest import HostSim
+        _HOSTSIM.append(HostSim())
+    return _HOSTSIM[0]
+
+
+def vignette_ops(shape, cfgkw, req, must_plan=True):
+    """The planner's vignette ops of a request on an h x w x c source, in order, as dicts: cx, cy, the op's frame w, h,
+    its table's nx, ny (0: evaluated per pixel), maxr, intensity (through tests/hostsim, hostsim_vignette_ops). A request
+    the planner refuses fails, or gives [] when must_plan is False."""
+    hs = _hostsim()
+    lib = hs.lib
+    lib.hostsim_vignette_ops.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_float), C.c_int]
+    h, w = shape[0], shape[1]
+    c = shape[2] if len(shape) == 3 else 1
+    ccfg, k1 = hs.api.Config(**cfgkw).to_c()
+    creq, k2 = hs.api.make_request(**req)
+    plan, step = C.c_void_p(), C.c_int(-1)
+    rc = lib.hostsim_plan_create(C.byref(creq), C.byref(ccfg), w, h, c, C.byref(plan), C.byref(step))
+    if rc and not must_plan:
+        return []
+    assert rc == 0, (req, rc)
+    try:
+        cap = 64
+        iv, fv = (C.c_int * (8 * cap))(), (C.c_float * (2 * cap))()
+        n = lib.hostsim_vignette_ops(plan, iv, fv, cap)
+        assert n <= cap
+        return [dict(cx=iv[8 * k], cy=iv[8 * k + 1], w=iv[8 * k + 2], h=iv[8 * k + 3], nx=iv[8 * k + 4], ny=iv[8 * k + 5],
+                     maxr=np.float32(fv[2 * k]), intensity=np.float32(fv[2 * k + 1])) for k in range(n)]
+    finally:
+        lib.hostsim_plan_destroy(plan)
+
+
+# Filters that neither move nor mix pixels, and the orientations, which move them without mixing: after the last vignette
+# only these let an ambiguous mask entry be traced to the output pixels it can touch.
+PER_PIXEL = {"modulate", "colorize", "gamma", "contrast", "gradmap", "vignette", "gotham", "lomo", "kelvin", "rainbow", "scanline"}
+ORIENT = {"flip", "rotate"}
+
+# Requests whose vignette frames hold an ambiguous entry but whose later steps mix or reorder pixels in ways the ambiguous
+# pixels cannot be traced through (blur, packed bottom-up output): {repr(label): ambiguous entries}. They keep the bound
+# of one LSB at under 1 in 1000 bytes. For the fixed seeds and shapes of the suite no such request exists.
+UNMAPPED_AMBIGUOUS = {}
+
+
+def _name(f):
+    return f.split("=", 1)[0]
+
+
+def vignette_allowance(shape, cfgkw, req, out_shape):
+    """None when every vignette frame of the request is free of ambiguous entries (the result must be exact). Else a
+    boolean image of out_shape[:2], the output pixels an ambiguous entry can reach, or the string "unmapped" when later
+    steps mix pixels. Also returns the number of ambiguous table entries."""
+    import vignette_ref as VR
+    from oracle import oracle as O
+    ops = vignette_ops(shape, cfgkw, req)
+    filters = req.get("filters", []) or []
+    at = [k for k, f in enumerate(filters) if _name(f) == "vignette"]
+    assert len(at) == len(ops), (req, len(at), len(ops))
+    allowed, n_amb, unmapped = None, 0, False
+    for k, op in zip(at, ops):
+        nx, ny = VR.table_dims(op["w"], op["h"], op["cx"], op["cy"])
+        n = VR.classify(op["maxr"], op["intensity"], nx, ny).count
+        if not n:
+            continue
+        n_amb += n
+        rest = filters[k + 1:]
+        if req.get("pack") or any(_name(f) not in PER_PIXEL | ORIENT for f in rest):
+            unmapped = True
+            continue
+        _, amb = VR.frame_mask(op)
+        img = np.repeat(amb[:, :, None].astype(np.uint8) * 255, 3, axis=2)
+        for f in rest:
+            if _name(f) in ORIENT:
+                code, img = O.apply_filter(img, f, True)
+                assert code == 0, f
+        assert img.shape[:2] == tuple(out_shape[:2]), (req, img.shape, out_shape)
+        allowed = (img[:, :, 0] > 0) if allowed is None else allowed | (img[:, :, 0] > 0)
+    if unmapped:
+        return "unmapped", n_amb
+    return allowed, n_amb
+
+
+# what the allowance was used for over the session: [(label, ambiguous entries, bytes that differed)]
+VIGNETTE_ALLOWANCE_USED = []
+
+
+def assert_vignette_exact(out, ref, shape, cfgkw, req, label):
+    """A result of a request with vignette ops against the oracle's (or the reference mask's): exact, except by at most 1
+    at output pixels an ambiguous mask entry reaches (tests/vignette_ref.py). shape: the request's source h, w[, c]."""
+    assert out.shape == ref.shape, (label, out.shape, ref.shape)
+    d = np.abs(out.astype(int) - ref.astype(int))
+    allowed, n_amb = vignette_allowance(shape, cfgkw, req, out.shape)
+    if allowed is None:
+        assert d.max() == 0, (label, int(d.max()), int((d > 0).sum()), d.size)
+        return
+    if isinstance(allowed, str):
+        assert UNMAPPED_AMBIGUOUS.get(repr(label)) == n_amb, (label, n_amb)
+        assert d.max() <= 1 and (d > 0).mean() < 1e-3, (label, int(d.max()), float((d > 0).mean()))
+    else:
+        assert d.max() <= 1 and d[~allowed].max(initial=0) == 0, (label, int(d.max()), int((d[~allowed] > 0).sum()))
+    VIGNETTE_ALLOWANCE_USED.append((repr(label), n_amb, int((d > 0).sum())))
 
 
 IO_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_io_v1.npz")

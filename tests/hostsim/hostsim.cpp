@@ -124,3 +124,29 @@ extern "C" void hostsim_plan_branch(const imp_gpu_plan* p, int k, int tiled, int
                        h.tile_rs, h.tile_rows, h.tile_smem, l.smem_bytes};
     memcpy(out, v, sizeof v);
 }
+// Per vignette op of the plan, in pass and op order, 8 ints: cx, cy, the op's frame w, h, the table's nx, ny as the
+// planner sized it (0, 0: no table, each pixel evaluates imp_vignette_mask), the frame map's swap and flip flags packed
+// as swap | flipx << 1 | flipy << 2, and 0; and 2 floats: maxr, intensity. Returns the number of ops (at most cap are written).
+extern "C" int hostsim_vignette_ops(const imp_gpu_plan* p, int* iout, float* fout, int cap) {
+    int n = 0;
+    for (const ImpHostPass& hp : p->passes) {
+        const ImpOp* ops = (const ImpOp*)(hp.blob.data() + hp.hdr.ops_off);
+        for (int k = 0; k < hp.hdr.nops; k++) {
+            const ImpOp& o = ops[k];
+            if (o.kind != IMP_OP_VIGNETTE) continue;
+            if (n < cap) {
+                const int v[8] = {o.i[0], o.i[1], o.map.w, o.map.h, o.i[2], o.i[3], o.map.swap | o.map.flipx << 1 | o.map.flipy << 2, 0};
+                memcpy(iout + 8 * n, v, sizeof v);
+                fout[2 * n] = o.f[0]; fout[2 * n + 1] = o.f[1];
+            }
+            n++;
+        }
+    }
+    return n;
+}
+// out[j * nx + i] = the CPU build of imp_vignette_mask at |dx| = i, |dy| = j (the code the device table kernel and the
+// per-pixel path compile).
+extern "C" void hostsim_vignette_mask_table(float* out, int nx, int ny, float maxr, float intensity) {
+    for (int j = 0; j < ny; j++)
+        for (int i = 0; i < nx; i++) out[(size_t)j * nx + i] = imp_vignette_mask(0, 0, i, j, maxr, intensity);
+}

@@ -1,6 +1,6 @@
 """Parity report (GPU box): max |diff| and PSNR of the CUDA path against the CPU oracle for the five BASELINE configs
 and every filter, through the C ABI. Test infrastructure: `python tests/parity_report.py > profiles/r01_parity_report.txt`.
-PSNR is reported as 'inf' for bit-exact results. Tolerances enforced by the test-suite: 0 everywhere, <= 1 LSB Vignette."""
+PSNR is reported as 'inf' for bit-exact results. The test-suite enforces 0 everywhere; a vignette may differ by 1 only at pixels whose mask rounding is ambiguous (tests/vignette_ref.py)."""
 import math
 import os
 import sys

@@ -207,6 +207,7 @@ from ngx_http_imgproc_b200 import api
 from oracle import oracle as O
 from conftest import rnd_image, smooth_image
 from test_planner_host import REQS, _oracle
+import golden_util as G
 L = M.library(); L.init(0)
 L.lib.imp_gpu_debug_flags.restype = C.c_uint
 wm = rnd_image(7, 12, 20, 4)
@@ -219,8 +220,11 @@ def check(img, rq, kwx=kw):
     assert code == c2, (rq, code, c2)
     if code: return
     out = p.run_host(img); p.close()
-    d = np.abs(out.astype(int) - ref.astype(int)).max()
-    assert d <= (1 if any("vignette" in f for f in rq.get("filters", [])) else 0), (rq, int(d))
+    if any("vignette" in f for f in rq.get("filters", [])):
+        G.assert_vignette_exact(out, ref, img.shape, kwx, rq, rq)
+    else:
+        d = np.abs(out.astype(int) - ref.astype(int)).max()
+        assert d == 0, (rq, int(d))
     n += 1
 for (h, w, c) in [(60, 80, 3), (45, 64, 4), (33, 47, 1), (97, 33, 3), (131, 259, 4)]:
     img = smooth_image(h + w, h, w, c)

@@ -107,7 +107,7 @@ def _assert_same(out, ref, case):
     assert out.shape == ref.shape, (case.name, out.shape, ref.shape)
     d = np.abs(out.astype(int) - ref.astype(int))
     if case.vignette:
-        assert d.max() <= G.VIGNETTE_TOL and (d > 0).mean() < 1e-3, (case.name, int(d.max()), float((d > 0).mean()))
+        G.assert_vignette_exact(out, ref, case.shape, case.cfgkw, case.req, case.name)
     else:
         assert d.max() == 0, (case.name, int(d.max()), int((d > 0).sum()), d.size)
 

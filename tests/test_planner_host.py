@@ -28,8 +28,10 @@ def test_hostsim_matches_golden(hostsim, case):
         assert step == case["step"] or code == 55
         return
     assert out.shape == case["out"].shape
-    tol = G.VIGNETTE_TOL if "vignette" in case["query"] else 0
-    assert np.abs(out.astype(int) - case["out"].astype(int)).max() <= tol
+    if "vignette" in case["query"]:
+        G.assert_vignette_exact(out, case["out"], case["img"].shape, case["cfgkw"], req, case["name"])
+    else:
+        assert np.array_equal(out, case["out"])
 
 
 REQS = [dict(resize="30,20"), dict(crop="1,1"), dict(crop="16,9,l,t"), dict(crop="40px,20px,6px,0px"), dict(crop="40px,20"),
@@ -101,8 +103,7 @@ def test_long_filter_lists_split_into_passes_and_validate_mode_agrees(hostsim, o
         code, step, out, info = hostsim.run(img, api.Config(**kw), want_info=True, **rq)
         c2, s2, ref = _oracle(orc, img, rq, kw)
         assert code == c2 == 0
-        tol = 1 if any("vignette" in x for x in f) else 0
-        assert np.abs(out.astype(int) - ref.astype(int)).max() <= tol
+        G.assert_vignette_exact(out, ref, img.shape, kw, rq, f[:3])
     assert hostsim.run(img, api.Config(**kw), want_info=True, filters=chains[0])[3]["passes"] == 2
     one = hostsim.run(img, api.Config(**kw), want_info=True, filters=["gotham=1", "modulate=0,0,100", "colorize=704214,0.6", "contrast=1.2"])[3]
     assert one["passes"] == 1
@@ -209,8 +210,9 @@ def test_hostsim_random_requests_vs_oracle(hostsim, orc):
         if code:
             assert step == s2, (it, rq)
             continue
-        tol = 1 if any("vignette" in f for f in rq["filters"]) else 0
-        assert out.shape == o2.shape, (it, rq)
-        assert np.abs(out.astype(int) - o2.astype(int)).max() <= tol, (it, (h, w, c), rq)
+        if any("vignette" in f for f in rq["filters"]):
+            G.assert_vignette_exact(out, o2, img.shape, kw, rq, (it, (h, w, c), rq))
+        else:
+            assert np.array_equal(out, o2), (it, (h, w, c), rq)
         done += 1
     assert done > 100

@@ -9,8 +9,9 @@
  * device every compute entry point returns IMP_ERROR_GPU.
  *
  * What each group replaces in the reference:
- *   imp_gpu_init / imp_gpu_shutdown        OnEnvStart / OnEnvDestroy      bridge.c:10-16 (no-ops there;
- *                                          called per worker from module.c:100-107, i.e. after fork)
+ *   imp_gpu_init_worker / imp_gpu_shutdown OnEnvStart / OnEnvDestroy      bridge.c:10-16 (no-ops there;
+ *                                          called per worker from module.c:100-107, i.e. after fork): worker k
+ *                                          takes device list[k % length] of IMP_GPU_DEVICES (below)
  *   imp_gpu_request + imp_gpu_config       the strings RunJob extracts from the query (bridge.c:346-372)
  *                                          and the Config fields the ops read (required.h:110-120)
  *   imp_gpu_plan_create                    argument validation of Crop (bridge.c:18-128), Resize
@@ -26,6 +27,11 @@
  *   imp_gpu_batch_ascii_host               the brightness or the text comes back, not the frame
  * The reference-signature operator layer (Crop/Resize/Filter/Watermark/BlendWithPaper on IplImage)
  * is declared in imp_ops.h and is implemented on top of this ABI.
+ *
+ * IMP_GPU_DEVICES (environment): the devices this process may use, in order, as comma-separated decimal
+ * ordinals ("4,0,5,1"); unset or empty means 0..n-1 for the n devices present. imp_gpu_init_worker maps
+ * nginx worker k onto entry k % length, and the farm runs GPU g of its assignment on entry g. Read at each
+ * of those calls; imp_gpu_init(device) ignores it.
  */
 #ifndef IMP_GPU_H
 #define IMP_GPU_H
@@ -111,7 +117,18 @@ void imp_gpu_shutdown(void);
 int  imp_gpu_device_count(void);
 /* Selects which initialised device subsequent calls from THIS thread use. */
 int  imp_gpu_set_device(int device);
-const char* imp_gpu_last_error(void);          /* thread-local text of the last IMP_ERROR_GPU */
+/* The device worker `worker` takes (pure host logic, needs no device): *device = list[worker % length], where the list
+ * is `devices` in IMP_GPU_DEVICES's syntax, or 0..n_devices-1 when `devices` is NULL or empty. IMP_ERROR_INVALID_ARGS
+ * for a negative worker or a bad list (an empty or non-decimal entry, a trailing comma, an ordinal >= n_devices or
+ * >= 16, a repeated ordinal, more than 16 entries; imp_gpu_last_error() names the entry); IMP_ERROR_GPU for
+ * n_devices <= 0. *device = -1 on failure. */
+int  imp_gpu_worker_device(int worker, int n_devices, const char* devices, int* device);
+/* OnEnvStart of nginx worker `worker` (ngx_worker): counts the devices, maps the worker through imp_gpu_worker_device
+ * with IMP_GPU_DEVICES from the environment, then imp_gpu_init on the result, which also makes it the calling thread's
+ * device. *device (may be NULL) = the device, or -1 on failure; then nothing is initialised and compute calls fail
+ * with IMP_ERROR_GPU as they do before any imp_gpu_init. */
+int  imp_gpu_init_worker(int worker, int* device);
+const char* imp_gpu_last_error(void);          /* thread-local text of the last IMP_ERROR_GPU or rejected device list */
 /* Diagnostics: bounds assertions violated by the tile kernels on the current device since start-up, as a bit set. Always 0
  * for the release build; the debug build (python -m ngx_http_imgproc_b200.build --debug -> libimp_gpu_dbg.so, compiled
  * with -DIMP_DEBUG_BOUNDS) checks every staged-tile, lookup, out-stage and destination address the tile kernels form —
@@ -194,7 +211,9 @@ int  imp_gpu_batch_poll(const imp_gpu_ticket* ticket);
 int  imp_gpu_batch_wait(imp_gpu_ticket* ticket);
 /* Same work sharded over devices 0..n_gpus-1 with one host thread per GPU; no inter-GPU traffic (nothing crosses
  * GPUs: docs/02 - Configuration.md:18 worker_processes is the reference's scale-out model). All devices are
- * initialised on demand. imp_gpu_farm_run_host is round-robin (job i -> GPU i mod n_gpus). */
+ * initialised on demand. imp_gpu_farm_run_host is round-robin (job i -> GPU i mod n_gpus). With IMP_GPU_DEVICES set,
+ * GPU g runs on its entry g, n_gpus larger than the list returns IMP_ERROR_GPU like n_gpus larger than the box, and a
+ * bad list returns IMP_ERROR_INVALID_ARGS before any work. */
 #define IMP_FARM_ROUND_ROBIN 0
 #define IMP_FARM_SIZE_AWARE  1   /* largest job first onto the GPU with the fewest algorithmic bytes so far (mixed sizes) */
 /* The assignment itself (pure host logic, needs no device): owner[i] = the GPU job i runs on under `policy`. */

@@ -128,6 +128,8 @@ class Library:
         L.imp_gpu_batch_submit_host.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]
         L.imp_gpu_batch_wait.argtypes = [C.c_void_p]
         L.imp_gpu_batch_poll.argtypes = [C.c_void_p]
+        L.imp_gpu_worker_device.argtypes = [C.c_int, C.c_int, C.c_char_p, C.POINTER(C.c_int)]
+        L.imp_gpu_init_worker.argtypes = [C.c_int, C.POINTER(C.c_int)]
         L.imp_gpu_upload_watermark.argtypes = [C.POINTER(CWatermark)]
         L.imp_gpu_plan_cache_stats.argtypes = [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong), C.POINTER(C.c_int)]
         L.imp_gpu_plan_cache_stats.restype = None
@@ -160,6 +162,23 @@ class Library:
 
     def set_device(self, device: int):
         self.check(self.lib.imp_gpu_set_device(device))
+
+    def worker_device(self, worker: int, n_devices: int, spec: Optional[str] = None) -> int:
+        """imp_gpu_worker_device: the device worker `worker` takes from `spec` (IMP_GPU_DEVICES's syntax; None or "" =
+        0..n_devices-1). Host logic only; raises ImpError (with the offending entry) on a bad list."""
+        d = C.c_int(-1)
+        rc = self.lib.imp_gpu_worker_device(worker, n_devices, None if spec is None else spec.encode(), C.byref(d))
+        if rc != IMP_OK:
+            raise ImpError(rc, None, self.last_error())
+        return d.value
+
+    def init_worker(self, worker: int) -> int:
+        """imp_gpu_init_worker: OnEnvStart of worker `worker` (IMP_GPU_DEVICES from the environment); returns the device."""
+        d = C.c_int(-1)
+        rc = self.lib.imp_gpu_init_worker(worker, C.byref(d))
+        if rc != IMP_OK:
+            raise ImpError(rc, None, self.last_error())
+        return d.value
 
     def shutdown(self):
         self.lib.imp_gpu_shutdown()

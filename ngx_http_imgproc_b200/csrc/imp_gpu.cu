@@ -876,6 +876,59 @@ int check_device_job(const imp_gpu_plan* plan, const void* d_src, int sp, const 
     return IMP_OK;
 }
 
+// How many devices the box has; IMP_ERROR_GPU with the reason when it has none.
+int count_devices(int* n) {
+    *n = 0;
+    cudaError_t e = cudaGetDeviceCount(n);
+    if (e != cudaSuccess || *n == 0) {
+        *n = 0;
+        snprintf(t_err, sizeof t_err, "no CUDA device available (%s); libimp_gpu has no CPU fallback", e == cudaSuccess ? "count == 0" : cudaGetErrorString(e));
+        return IMP_ERROR_GPU;
+    }
+    return IMP_OK;
+}
+
+int bad_device_list(const char* spec, int entry, const char* tok, int tok_len, const char* why) {
+    snprintf(t_err, sizeof t_err, "device list \"%s\": entry %d (\"%.*s\") %s", spec, entry, std::min(tok_len, 64), tok, why);
+    return IMP_ERROR_INVALID_ARGS;
+}
+
+// Which devices this process may use, in order: the one parser of IMP_GPU_DEVICES (the worker mapping and the farm both
+// read the list through here). `spec` NULL or empty: 0 .. n_devices-1, at most MAX_DEV of them. Otherwise comma-separated
+// decimal ordinals, each below n_devices and MAX_DEV, none twice, at most MAX_DEV entries; anything else is
+// IMP_ERROR_INVALID_ARGS with the offending entry in t_err.
+int device_list(const char* spec, int n_devices, int* list, int* len) {
+    *len = 0;
+    if (n_devices <= 0) return fail_msg("no CUDA device to choose from (0 devices); libimp_gpu has no CPU fallback");
+    if (!spec || !*spec) {
+        for (int d = 0; d < std::min(n_devices, MAX_DEV); d++) list[(*len)++] = d;
+        return IMP_OK;
+    }
+    for (const char* p = spec;; p++) {
+        const char* tok = p;
+        const int entry = *len + 1;
+        long v = 0;
+        for (; *p >= '0' && *p <= '9'; p++) v = std::min(v * 10 + (*p - '0'), 1000000L);
+        if (*p && *p != ',') {
+            while (*p && *p != ',') p++;
+            return bad_device_list(spec, entry, tok, (int)(p - tok), "is not a decimal device ordinal");
+        }
+        const int tok_len = (int)(p - tok);
+        if (tok_len == 0) return bad_device_list(spec, entry, tok, 0, "is empty");
+        if (*len == MAX_DEV) return bad_device_list(spec, entry, tok, tok_len, "is past the 16 entries a list may hold");
+        if (v >= n_devices) {
+            char why[48];
+            snprintf(why, sizeof why, "names no device: %d present", n_devices);
+            return bad_device_list(spec, entry, tok, tok_len, why);
+        }
+        if (v >= MAX_DEV) return bad_device_list(spec, entry, tok, tok_len, "is beyond device 15, the last libimp_gpu drives");
+        for (int k = 0; k < *len; k++)
+            if (list[k] == v) return bad_device_list(spec, entry, tok, tok_len, "names a device already listed");
+        list[(*len)++] = (int)v;
+        if (!*p) return IMP_OK;
+    }
+}
+
 }  // namespace
 
 struct imp_gpu_ticket {
@@ -896,11 +949,7 @@ int imp_gpu_device_count(void) {
 int imp_gpu_init(int device) {
     if (device < 0 || device >= MAX_DEV) return fail_msg("imp_gpu_init: device index out of range");
     int n = 0;
-    cudaError_t e = cudaGetDeviceCount(&n);
-    if (e != cudaSuccess || n == 0) {
-        snprintf(t_err, sizeof t_err, "no CUDA device available (%s); libimp_gpu has no CPU fallback", e == cudaSuccess ? "count == 0" : cudaGetErrorString(e));
-        return IMP_ERROR_GPU;
-    }
+    if (int rc = count_devices(&n)) return rc;
     if (device >= n) return fail_msg("imp_gpu_init: no such device");
     CK(cudaSetDevice(device));
     {
@@ -933,6 +982,26 @@ int imp_gpu_init(int device) {
     }
     t_dev = device;
     return IMP_OK;
+}
+
+// Pure host logic, like imp_gpu_farm_assign: testable without a device.
+int imp_gpu_worker_device(int worker, int n_devices, const char* devices, int* device) {
+    if (!device) return IMP_ERROR_INVALID_ARGS;
+    *device = -1;
+    if (worker < 0) { snprintf(t_err, sizeof t_err, "worker index %d is negative", worker); return IMP_ERROR_INVALID_ARGS; }
+    int list[MAX_DEV], len = 0;
+    if (int rc = device_list(devices, n_devices, list, &len)) return rc;
+    *device = list[worker % len];
+    return IMP_OK;
+}
+
+int imp_gpu_init_worker(int worker, int* device) {
+    if (device) *device = -1;
+    int n = 0, d = -1, rc = count_devices(&n);
+    if (rc == IMP_OK) rc = imp_gpu_worker_device(worker, n, getenv("IMP_GPU_DEVICES"), &d);
+    if (rc == IMP_OK) rc = imp_gpu_init(d);
+    if (rc == IMP_OK && device) *device = d;
+    return rc;
 }
 
 int imp_gpu_set_device(int device) {
@@ -1226,7 +1295,9 @@ int imp_gpu_farm_run_host_policy(int n, imp_gpu_plan* const* plans, const unsign
     if (n > 0 && (!plans || !srcs || !src_steps || !dsts || !dst_steps)) return IMP_ERROR_INVALID_ARGS;
     const int avail = imp_gpu_device_count();
     if (avail <= 0) return fail_msg("no CUDA device available; libimp_gpu has no CPU fallback");
-    if (n_gpus > avail || n_gpus > MAX_DEV) return fail_msg("imp_gpu_farm_run_host: more GPUs requested than present");
+    int devs[MAX_DEV], n_devs = 0;                      // GPU g of the assignment runs on device devs[g]
+    if (int rc = device_list(getenv("IMP_GPU_DEVICES"), avail, devs, &n_devs)) return rc;
+    if (n_gpus > n_devs) return fail_msg("imp_gpu_farm_run_host: more GPUs requested than present");
     std::vector<std::vector<ImpHostJob>> share(n_gpus);
     try {
         const std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps, dsts, dst_steps);
@@ -1242,7 +1313,7 @@ int imp_gpu_farm_run_host_policy(int n, imp_gpu_plan* const* plans, const unsign
     const int caller_dev = t_dev;
     for (int g = 0; g < n_gpus; g++) {
         th.emplace_back([&, g]() {
-            int rc = imp_gpu_set_device(g);
+            int rc = imp_gpu_set_device(devs[g]);
             if (rc == IMP_OK && !share[g].empty()) {
                 try { rc = run_host_chunked(share[g], ImpResult::Frame, n_streams); } catch (const std::bad_alloc&) { rc = IMP_ERROR_MALLOC_FAILED; }
             }
@@ -1252,7 +1323,7 @@ int imp_gpu_farm_run_host_policy(int n, imp_gpu_plan* const* plans, const unsign
     }
     for (auto& t : th) t.join();
     if (caller_dev >= 0) { t_dev = caller_dev; cudaSetDevice(caller_dev); }
-    for (int g = 0; g < n_gpus; g++) if (rcs[g]) { snprintf(t_err, sizeof t_err, "gpu %d: %s", g, errs[g].c_str()); return rcs[g]; }
+    for (int g = 0; g < n_gpus; g++) if (rcs[g]) { snprintf(t_err, sizeof t_err, "gpu %d: %s", devs[g], errs[g].c_str()); return rcs[g]; }
     return IMP_OK;
 }
 

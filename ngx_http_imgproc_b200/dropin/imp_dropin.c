@@ -15,6 +15,8 @@
  * exactly like the one it replaces (same IMP_* code, image untouched on error), records the operation and fixes the
  * IplImage header up; imp_FlushAlbum runs what was recorded for all frames as fused GPU passes.
  */
+#include <ngx_config.h>
+#include <ngx_core.h>
 #include "required.h"
 #include "bridge.h"
 #include "filters.h"
@@ -46,8 +48,22 @@ static void imp_config_from(const Config* c, imp_gpu_config* g, imp_gpu_watermar
     }
 }
 
-/* module.c:100-107 calls these per worker process, i.e. after fork: the CUDA context is created here */
-void OnEnvStart()   { imp_gpu_init(0); imp_ops_set_image_allocator(imp_create, imp_release); }
+/* The worker's index (nginx's ngx_process_cycle.c sets it before the worker's init_process handlers run). Weak: inside
+ * nginx its own definition is the one linked, and a host built without nginx (the reference's RunJob linked against
+ * stand-in headers for testing) still links, as worker 0 unless it sets the symbol. */
+ngx_uint_t ngx_worker __attribute__((weak));
+
+/* module.c:100-107 calls these per worker process, i.e. after fork: the CUDA context is created here, on the device the
+ * worker's index selects (IMP_GPU_DEVICES, imp_gpu.h), so that worker_processes spreads the workers over every GPU of the
+ * box. Without a device every request answers IMP_ERROR_GPU; the startup log says why. */
+void OnEnvStart() {
+    int dev = -1;
+    if (imp_gpu_init_worker((int)ngx_worker, &dev) == IMP_OK)
+        ngx_log_error(NGX_LOG_NOTICE, ngx_cycle->log, 0, "imgproc: worker %d on GPU %d", (int)ngx_worker, dev);
+    else
+        ngx_log_error(NGX_LOG_EMERG, ngx_cycle->log, 0, "imgproc: worker %d has no GPU: %s", (int)ngx_worker, imp_gpu_last_error());
+    imp_ops_set_image_allocator(imp_create, imp_release);
+}
 void OnEnvDestroy() { imp_gpu_shutdown(); }
 
 int Crop(IplImage** pointer, char* args, char* gravity) { return imp_Crop(pointer, args, gravity); }

@@ -285,6 +285,21 @@ int  imp_gpu_gif_expand_host(const imp_gpu_gif_frame* frames, int n, int canvas_
 int  imp_gpu_gif_album_run_host(const imp_gpu_gif_frame* frames, int n, int canvas_w, int canvas_h, int destructive,
                                 imp_gpu_plan* const* plans, unsigned char* const* dsts, const int* dst_steps,
                                 int n_streams);
+/* Many GIF requests in one call: each album is what imp_gpu_gif_album_run_host takes. */
+typedef struct imp_gpu_gif_album {
+    const imp_gpu_gif_frame* pages; int n_pages;          /* as imp_gpu_gif_album_run_host takes them */
+    int canvas_w, canvas_h, destructive;
+    imp_gpu_plan* const* plans;                           /* n_pages entries; NULL = page only replayed (a `page` request) */
+    unsigned char* const* dsts; const int* dst_steps;     /* n_pages entries, used where plans[f] != NULL */
+} imp_gpu_gif_album;
+/* Runs every album: each album's results are byte-identical to what imp_gpu_gif_album_run_host gives for that album
+ * alone, whatever the neighbouring albums, their order or n_streams. Consecutive albums whose canvases fit 256 MB together
+ * form a round (an album above that is a round alone): one upload of all their pages, one expansion launch, and one
+ * chunked frame loop whose grouped launches span albums; rounds run one after another. Every album is checked before any
+ * work (page and palette pointers, page geometry, each plan's source a canvas_w x canvas_h 4-channel canvas, destination
+ * steps): one bad album returns IMP_ERROR_INVALID_ARGS and no destination of any album is written. n_albums == 0 returns
+ * IMP_OK. Synchronous, on the current device. */
+int  imp_gpu_gif_albums_run_host(const imp_gpu_gif_album* albums, int n_albums, int n_streams);
 
 /* ---- memory helpers so a C host needs no CUDA headers --------------------------------------------- */
 int  imp_gpu_malloc(void** d_ptr, size_t bytes);

@@ -37,6 +37,11 @@ class CGifFrame(C.Structure):
                 ("dispose", C.c_int), ("transparency_key", C.c_int), ("palette", C.c_void_p)]
 
 
+class CGifAlbum(C.Structure):
+    _fields_ = [("pages", C.c_void_p), ("n_pages", C.c_int), ("canvas_w", C.c_int), ("canvas_h", C.c_int), ("destructive", C.c_int),
+                ("plans", C.c_void_p), ("dsts", C.c_void_p), ("dst_steps", C.c_void_p)]
+
+
 class CConfig(C.Structure):
     _fields_ = [("max_target_w", C.c_uint), ("max_target_h", C.c_uint), ("max_filters", C.c_int),
                 ("allow_experiments", C.c_int), ("watermark", C.POINTER(CWatermark))]
@@ -225,6 +230,11 @@ class Library:
     def gif_album(self, frames, cw: int, ch: int, destructive: bool, plan: "Plan", outs=None, n_streams: int = 4):
         """imp_gpu_gif_album_run_host: pages up as indices, canvases expanded on the device, `plan` over every frame."""
         return GifAlbumJob(self, frames, cw, ch, destructive, plan, outs).run(self, n_streams)
+
+    def gif_albums(self, albums, n_streams: int = 4):
+        """imp_gpu_gif_albums_run_host: many GIF requests in one call. Each album is (pages as gif_album takes them, cw, ch,
+        destructive, a plan or a per-page plan list[, outs]); returns the result frames per album (None for a replay-only page)."""
+        return GifAlbumsJob(self, albums).run(self, n_streams)
 
     def gif_expand(self, frames, cw: int, ch: int, destructive: bool):
         """LoadGIF's canvas expansion (advancedio.c:195-248) on the device; frames as for gif_pages."""
@@ -417,6 +427,22 @@ class GifAlbumJob:
         cw, ch, d = self.geom
         lib.check(lib.lib.imp_gpu_gif_album_run_host(self.arr, self.n, cw, ch, d, self.P, self.D, self.DS, n_streams))
         return self.outs
+
+
+class GifAlbumsJob:
+    """imp_gpu_gif_albums_run_host with its argument arrays built once: one GifAlbumJob per album, their arrays gathered
+    into the imp_gpu_gif_album list."""
+
+    def __init__(self, lib: Library, albums):
+        self.jobs = [GifAlbumJob(lib, *a) for a in albums]
+        self.n = len(self.jobs)
+        self.arr = (CGifAlbum * max(self.n, 1))(*[CGifAlbum(C.addressof(j.arr), j.n, *j.geom, C.addressof(j.P), C.addressof(j.D), C.addressof(j.DS))
+                                                  for j in self.jobs])
+        lib.lib.imp_gpu_gif_albums_run_host.argtypes = [C.c_void_p, C.c_int, C.c_int]
+
+    def run(self, lib: Library, n_streams=4):
+        lib.check(lib.lib.imp_gpu_gif_albums_run_host(self.arr, self.n, n_streams))
+        return [j.outs for j in self.jobs]
 
 
 def farm_assign(lib: Library, plans: List[Plan], n_gpus: int, policy=FARM_ROUND_ROBIN) -> List[int]:

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libimp_gpu.so")
 SOURCES = ["imp_kernels.cu", "imp_k_strip.cu", "imp_k_blur.cu", "imp_k_cubic.cu", "imp_k_gather.cu", "imp_gpu.cu", "imp_transfer.cpp", "imp_planner.cpp", "imp_ops.cpp"]
-HEADERS = ["imp_plan.h", "imp_pixel.cuh", "imp_gather.cuh", "imp_internal.h", "imp_tiles.cuh", "imp_blur.cuh", "imp_cubic.cuh", "imp_gathertile.cuh",
+HEADERS = ["imp_plan.h", "imp_pixel.cuh", "imp_gather.cuh", "imp_internal.h", "imp_tiles.cuh", "imp_blur.cuh", "imp_cubic.cuh", "imp_gathertile.cuh", "imp_gif.cuh",
            os.path.join("..", "..", "include", "imp_gpu.h"), os.path.join("..", "..", "include", "imp_ops.h")]
 
 NVCC_FLAGS = [

@@ -1047,7 +1047,7 @@ const char* imp_gpu_last_error(void) { return t_err; }
 unsigned imp_gpu_debug_flags(void) {
     if (bind() != IMP_OK) return 0;
     cudaDeviceSynchronize();
-    return imp_debug_flags_strip() | imp_debug_flags_blur() | imp_debug_flags_cubic() | imp_debug_flags_gather();
+    return imp_debug_flags_kernels() | imp_debug_flags_strip() | imp_debug_flags_blur() | imp_debug_flags_cubic() | imp_debug_flags_gather();
 }
 unsigned long long imp_gpu_launch_count(void) { return imp_launches(); }
 
@@ -1423,34 +1423,24 @@ int imp_gpu_ascii_host(const unsigned char* img, int step, int w, int h, int c, 
 }
 
 // ---- "next" row §8f-2: GIF canvas expansion ------------------------------------------------------------------
-// Packed page block of a GIF: [ImpGifFrame n][palettes n*1024][index planes], device pointers already resolved against d_buf.
-static int gif_validate(const imp_gpu_gif_frame* frames, int n, size_t* meta_bytes, size_t* total) {
-    size_t idx_bytes = 0;
-    for (int f = 0; f < n; f++) {
+// The checks every GIF entry point makes on a GIF's pages.
+static int gif_check_pages(const imp_gpu_gif_frame* frames, int n) {
+    if (!frames || n <= 0) return IMP_ERROR_INVALID_ARGS;
+    for (int f = 0; f < n; f++)
         if (!frames[f].indices || !frames[f].palette || frames[f].width <= 0 || frames[f].height <= 0 || frames[f].pitch < frames[f].width) return IMP_ERROR_INVALID_ARGS;
-        idx_bytes += ((size_t)frames[f].pitch * frames[f].height + 15) & ~size_t(15);
-    }
-    *meta_bytes = (((size_t)n * sizeof(ImpGifFrame)) + 15) & ~size_t(15);
-    *total = *meta_bytes + (size_t)n * 1024 + idx_bytes;
     return IMP_OK;
 }
-static void gif_pack(const imp_gpu_gif_frame* frames, int n, size_t meta_bytes, uint8_t* h_buf, const uint8_t* d_buf) {
-    ImpGifFrame* meta = reinterpret_cast<ImpGifFrame*>(h_buf);
-    std::vector<size_t> offs((size_t)n);
-    size_t off = meta_bytes + (size_t)n * 1024;
-    for (int f = 0; f < n; f++) { offs[f] = off; off += ((size_t)frames[f].pitch * frames[f].height + 15) & ~size_t(15); }
-    auto pack = [&](int f0, int f1) {
-        for (int f = f0; f < f1; f++) {
-            const imp_gpu_gif_frame& g = frames[f];
-            memcpy(h_buf + meta_bytes + (size_t)f * 1024, g.palette, 1024);
-            copy_stream(h_buf + offs[f], g.indices, (size_t)g.pitch * g.height);
-            meta[f].indices = d_buf + offs[f]; meta[f].palette = d_buf + meta_bytes + (size_t)f * 1024;
-            meta[f].pitch = g.pitch; meta[f].w = g.width; meta[f].h = g.height; meta[f].left = g.left; meta[f].top = g.top;
-            meta[f].dispose = g.dispose; meta[f].key = g.transparency_key; meta[f].pad_ = 0;
-        }
-    };
-    // the pages are pageable host memory: a long animation (tens of MB) is packed by several cores (run_parts)
-    run_parts(n, stage_parts(off, n), pack);
+// Packs a round into h_buf, uploads it to d_buf as one copy and launches its one expansion into d_arena. The pages are
+// pageable host memory: a long animation (tens of MB) is packed by several cores (run_parts).
+static cudaError_t gif_round_expand(const ImpGifRound& r, uint8_t* h_buf, uint8_t* d_buf, uint8_t* d_arena, cudaStream_t st) {
+    const int np = (int)r.pages.size();
+    run_parts(np, stage_parts(r.pack_bytes, np), [&r, h_buf, d_buf](int k0, int k1) {
+        for (int k = k0; k < k1; k++) imp_gif_pack_page(r, k, h_buf, d_buf, copy_stream);
+    });
+    cudaError_t e = cudaMemcpyAsync(d_buf, h_buf, r.pack_bytes, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = imp_launch_gif_expand(reinterpret_cast<const ImpGifAlbum*>(d_buf), (int)r.albums.size(),
+                                                    reinterpret_cast<const ImpGifFrame*>(d_buf + r.page_off), r.blocks, d_arena, r.arena_bytes, st);
+    return e;
 }
 
 int imp_gpu_gif_expand_device(const imp_gpu_gif_frame* frames, int n, int canvas_w, int canvas_h, int destructive,
@@ -1458,16 +1448,16 @@ int imp_gpu_gif_expand_device(const imp_gpu_gif_frame* frames, int n, int canvas
     int rc = bind(); if (rc) return rc;
     if (!frames || n <= 0 || canvas_w <= 0 || canvas_h <= 0 || !d_canvases || canvas_pitch < canvas_w * 4 || canvas_pitch % 4) return IMP_ERROR_INVALID_ARGS;
     cudaStream_t st = pick_stream(stream);
-    size_t meta_bytes = 0, total = 0;
-    if ((rc = gif_validate(frames, n, &meta_bytes, &total))) return rc;
+    if ((rc = gif_check_pages(frames, n))) return rc;
+    const imp_gpu_gif_album album{frames, n, canvas_w, canvas_h, destructive, nullptr, nullptr, nullptr};
+    ImpGifRound r;
+    try { r = imp_gif_round_layout(&album, 1, canvas_pitch); } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
     uint8_t* h_buf = nullptr; uint8_t* d_buf = nullptr;
-    CK(cudaHostAlloc((void**)&h_buf, total, cudaHostAllocDefault));
-    cudaError_t e = cudaMallocAsync((void**)&d_buf, total, st);
+    CK(cudaHostAlloc((void**)&h_buf, r.pack_bytes, cudaHostAllocDefault));
+    cudaError_t e = cudaMallocAsync((void**)&d_buf, r.pack_bytes, st);
     if (e != cudaSuccess) { cudaFreeHost(h_buf); return fail(e, "cudaMallocAsync", __LINE__); }
-    try { gif_pack(frames, n, meta_bytes, h_buf, d_buf); }
+    try { e = gif_round_expand(r, h_buf, d_buf, (uint8_t*)d_canvases, st); }
     catch (const std::bad_alloc&) { cudaFreeAsync(d_buf, st); cudaFreeHost(h_buf); return IMP_ERROR_MALLOC_FAILED; }
-    e = cudaMemcpyAsync(d_buf, h_buf, total, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = imp_launch_gif_expand(reinterpret_cast<const ImpGifFrame*>(d_buf), n, canvas_w, canvas_h, destructive ? 1 : 0, (uint8_t*)d_canvases, canvas_pitch, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);          // h_buf / d_buf are released below
     cudaFreeAsync(d_buf, st);
     cudaFreeHost(h_buf);
@@ -1480,37 +1470,64 @@ int imp_gpu_gif_expand_device(const imp_gpu_gif_frame* frames, int n, int canvas
 // (bridge.c:576-656) without leaving it: grouped launches over all frames, results D2H as in imp_gpu_batch_run_host.
 int imp_gpu_gif_album_run_host(const imp_gpu_gif_frame* frames, int n, int canvas_w, int canvas_h, int destructive,
                                imp_gpu_plan* const* plans, unsigned char* const* dsts, const int* dst_steps, int n_streams) {
+    const imp_gpu_gif_album album{frames, n, canvas_w, canvas_h, destructive, plans, dsts, dst_steps};
+    return imp_gpu_gif_albums_run_host(&album, 1, n_streams);
+}
+
+// Many GIF requests: per round (imp_gif_round_bounds) one pack of all its albums' pages, one upload, one expansion launch
+// and one chunked frame loop over all its albums' frames, so that chunks and grouped launches span requests.
+int imp_gpu_gif_albums_run_host(const imp_gpu_gif_album* albums, int n_albums, int n_streams) {
     int rc = bind(); if (rc) return rc;
-    if (!frames || n <= 0 || canvas_w <= 0 || canvas_h <= 0 || !plans || !dsts || !dst_steps) return IMP_ERROR_INVALID_ARGS;
-    for (int f = 0; f < n; f++) {
-        const imp_gpu_plan* p = plans[f];                             // null: replayed for the pages after it, no result wanted
-        if (p && (p->src_w != canvas_w || p->src_h != canvas_h || p->src_c != 4)) return IMP_ERROR_INVALID_ARGS;
-    }
-    size_t meta_bytes = 0, total = 0;
-    if ((rc = gif_validate(frames, n, &meta_bytes, &total))) return rc;
-    const int pitch = align16(canvas_w * 4);
-    const size_t canvas_bytes = (size_t)pitch * canvas_h;
-    // a frame's source is its page's canvas; the page stands in for it until the canvases are allocated, so that a bad job
-    // is refused before any buffer grows
+    if (n_albums < 0 || (n_albums > 0 && !albums)) return IMP_ERROR_INVALID_ARGS;
+    if (n_albums == 0) return IMP_OK;
+    // a frame's source is its page's canvas; the page stands in for it until the canvases are placed, so that a bad job
+    // of any album is refused before any buffer grows or any work starts
     std::vector<ImpHostJob> jobs;
+    std::vector<int> job0((size_t)n_albums + 1);                     // album a's jobs: [job0[a], job0[a + 1])
+    std::vector<int> rounds;
+    std::vector<ImpGifRound> lay;
+    size_t pack_max = 0, arena_max = 0;
     try {
-        for (int f = 0; f < n; f++)
-            if (plans[f]) jobs.push_back(ImpHostJob{plans[f], frames[f].indices, pitch, dsts[f], dst_steps[f], false});
+        for (int a = 0; a < n_albums; a++) {
+            const imp_gpu_gif_album& al = albums[a];
+            if (al.canvas_w <= 0 || al.canvas_h <= 0 || !al.plans || !al.dsts || !al.dst_steps) return IMP_ERROR_INVALID_ARGS;
+            if ((rc = gif_check_pages(al.pages, al.n_pages))) return rc;
+            job0[a] = (int)jobs.size();
+            for (int f = 0; f < al.n_pages; f++) {
+                imp_gpu_plan* p = al.plans[f];                        // null: replayed for the pages after it, no result wanted
+                if (!p) continue;
+                if (p->src_w != al.canvas_w || p->src_h != al.canvas_h || p->src_c != 4) return IMP_ERROR_INVALID_ARGS;
+                jobs.push_back(ImpHostJob{p, al.pages[f].indices, align16(al.canvas_w * 4), al.dsts[f], al.dst_steps[f], false});
+            }
+        }
+        job0[n_albums] = (int)jobs.size();
+        if ((rc = check_host_jobs(ImpResult::Frame, jobs))) return rc;
+        rounds = imp_gif_round_bounds(albums, n_albums);
+        for (size_t r = 0; r + 1 < rounds.size(); r++) {
+            lay.push_back(imp_gif_round_layout(albums + rounds[r], rounds[r + 1] - rounds[r]));
+            pack_max = std::max(pack_max, lay.back().pack_bytes);
+            arena_max = std::max(arena_max, lay.back().arena_bytes);
+        }
     } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
-    if ((rc = check_host_jobs(ImpResult::Frame, jobs))) return rc;
     DevCtx& ctx = g_dev[t_dev];
     std::lock_guard<std::mutex> run_lk(ctx.run_mu);
-    if ((rc = ctx.h_gif.grow(total, true)) || (rc = ctx.d_gif.grow(total, false)) || (rc = ctx.d_canvas.grow(canvas_bytes * n, false))) return rc;
+    if ((rc = ctx.h_gif.grow(pack_max, true)) || (rc = ctx.d_gif.grow(pack_max, false)) || (rc = ctx.d_canvas.grow(arena_max, false))) return rc;
     if (!ctx.gif_ev) CK(cudaEventCreateWithFlags(&ctx.gif_ev, cudaEventDisableTiming));
-    for (int f = 0, k = 0; f < n; f++)
-        if (plans[f]) jobs[k++].src = ctx.d_canvas.p + (size_t)f * canvas_bytes;
     try {                                                             // the C caller cannot unwind: bad_alloc ends as a code
-    gif_pack(frames, n, meta_bytes, ctx.h_gif.p, ctx.d_gif.p);
-    CK(cudaMemcpyAsync(ctx.d_gif.p, ctx.h_gif.p, total, cudaMemcpyHostToDevice, ctx.stream));
-    CK(imp_launch_gif_expand(reinterpret_cast<const ImpGifFrame*>(ctx.d_gif.p), n, canvas_w, canvas_h, destructive ? 1 : 0, ctx.d_canvas.p, pitch, ctx.stream));
-    CK(cudaEventRecord(ctx.gif_ev, ctx.stream));
-    if (jobs.empty()) { CK(cudaStreamSynchronize(ctx.stream)); return IMP_OK; }
-    rc = run_host_chunked_locked(jobs.data(), (int)jobs.size(), ImpResult::Frame, n_streams, true, ctx.gif_ev);
+    for (size_t r = 0; r < lay.size() && rc == IMP_OK; r++) {         // one after another: the pack and the arena are reused
+        const ImpGifRound& R = lay[r];
+        const int a0 = rounds[r], a1 = rounds[r + 1];
+        for (int a = a0; a < a1; a++) {
+            const ImpGifAlbum& A = R.albums[a - a0];
+            for (int f = 0, k = job0[a]; f < A.n; f++)
+                if (albums[a].plans[f]) jobs[k++].src = ctx.d_canvas.p + A.canvas_off + (size_t)f * A.pitch * A.ch;
+        }
+        CK(gif_round_expand(R, ctx.h_gif.p, ctx.d_gif.p, ctx.d_canvas.p, ctx.stream));
+        CK(cudaEventRecord(ctx.gif_ev, ctx.stream));
+        const int j0 = job0[a0], j1 = job0[a1];
+        if (j0 == j1) CK(cudaStreamSynchronize(ctx.stream));
+        else rc = run_host_chunked_locked(jobs.data() + j0, j1 - j0, ImpResult::Frame, n_streams, true, ctx.gif_ev);
+    }
     } catch (const std::bad_alloc&) { rc = IMP_ERROR_MALLOC_FAILED; }
     if (rc != IMP_OK) cudaStreamSynchronize(ctx.stream);           // the staging buffers are reused by the next call
     return rc;

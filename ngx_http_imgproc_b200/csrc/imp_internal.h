@@ -107,6 +107,30 @@ constexpr size_t IMP_CHUNK_BYTES = 128u << 20;       // the most crop-window + r
 // The chunk boundaries [0, e1, ..., n] of n jobs over n_streams lanes (clamped to 1..8).
 std::vector<int> imp_chunk_bounds(const ImpHostJob* jobs, int n, int n_streams);
 
+// ---- GIF albums (imp_transfer.cpp): rounds and the packed page block of a round -----------------------------------
+constexpr size_t IMP_GIF_ROUND_BYTES = 256u << 20;  // the most canvas bytes a round holds (one album may exceed it)
+// The device bytes of an album's canvases: every page, replay-only pages included, at pitch align16(4 * canvas_w),
+// rounded up to 256 so that the next album's canvases start aligned.
+size_t imp_gif_canvas_bytes(const imp_gpu_gif_album& a);
+// The round boundaries [0, e1, ..., n] of n albums: consecutive albums while their canvas bytes stay within
+// IMP_GIF_ROUND_BYTES; an album above it forms a round alone. No albums: {0}, no round.
+std::vector<int> imp_gif_round_bounds(const imp_gpu_gif_album* albums, int n);
+// Where everything of a round lives. Pack (pinned, copied to the device as one block):
+// [album table][page table][palettes, 1024 bytes each][index planes, pitch * height each, 16-byte aligned];
+// arena: each album's canvases, imp_gif_canvas_bytes apart. `albums` holds every entry but the pack offsets of the pages.
+struct ImpGifRound {
+    std::vector<ImpGifAlbum> albums;
+    std::vector<const imp_gpu_gif_frame*> pages;   // the round's pages in page-table order
+    std::vector<size_t> idx_off;                   // page k's index plane in the pack
+    size_t page_off = 0, pal_off = 0, pack_bytes = 0, arena_bytes = 0;
+    long long blocks = 0;                          // expansion grid
+};
+// The layout of albums [0, n) as one round, page f of album a stored at canvas `pitch` (0: align16(4 * canvas_w)).
+ImpGifRound imp_gif_round_layout(const imp_gpu_gif_album* albums, int n, int pitch = 0);
+// Writes page k of the round into the pack at h_buf: its page-table entry (pointers resolved against d_buf, where the pack
+// lands on the device), palette and index plane, the plane through `copy`. The album table is written with page 0.
+void imp_gif_pack_page(const ImpGifRound& r, int k, uint8_t* h_buf, const uint8_t* d_buf, void (*copy)(uint8_t*, const uint8_t*, size_t));
+
 // How a job's source reaches the device and its result the host.
 enum class ImpRoute : uint8_t {
     Resident,        // source: already on this device (GIF canvases), nothing to upload
@@ -188,7 +212,10 @@ cudaError_t imp_launch_cubic_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs,
 cudaError_t imp_launch_gather_tile(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st);  // imp_k_gather.cu
 // rows of `row_bytes` bytes from (src, sp) to (dst, dp); dst and dp are multiples of 4 (the library's own pitched buffers)
 cudaError_t imp_launch_repitch(const uint8_t* d_src, int sp, uint8_t* d_dst, int dp, int row_bytes, int rows, cudaStream_t st);
-cudaError_t imp_launch_gif_expand(const ImpGifFrame* d_frames, int n, int cw, int ch, int destructive, uint8_t* d_canvases, int cpitch, cudaStream_t st);
+// Expands every album of a round's device tables (ImpGifRound) into the canvases of d_arena: `blocks` = ImpGifRound::blocks.
+cudaError_t imp_launch_gif_expand(const ImpGifAlbum* d_albums, int n_albums, const ImpGifFrame* d_pages, long long blocks,
+                                  uint8_t* d_arena, size_t arena_bytes, cudaStream_t st);
+unsigned imp_debug_flags_kernels();
 // One frame of a brightness or ASCII launch: a result on the device and where its answer goes.
 struct ImpInfoJob {
     const uint8_t* img;          // rows of w*c bytes (c in {1,3,4}), `pitch` apart

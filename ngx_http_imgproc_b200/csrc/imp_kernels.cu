@@ -8,6 +8,7 @@
 #include "imp_internal.h"
 #include <algorithm>
 #include "imp_gather.cuh"
+#include "imp_gif.cuh"
 
 #include <atomic>
 static std::atomic<unsigned long long> g_imp_launches{0};
@@ -224,45 +225,23 @@ cudaError_t imp_launch_repitch(const uint8_t* d_src, int sp, uint8_t* d_dst, int
     return cudaGetLastError();                 // a copy, not a pixel stage: not counted by imp_gpu_launch_count()
 }
 
-// GIF canvas expansion (SURVEY 8f-2; advancedio.c:195-248): every canvas pixel walks the frames in order, carrying the
-// reference's `master` index for the disposal replay in a register, and writes one BGRA pixel per frame. Frames travel
-// over PCIe as 8-bit indices (4x fewer bytes than the BGRA canvases the CPU path builds).
-__global__ void __launch_bounds__(256) imp_gif_expand_kernel(const ImpGifFrame* __restrict__ frames, int n, int cw, int ch, int destructive,
-                                                             uint8_t* __restrict__ canvases, int cpitch) {
-    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-    if (x >= cw || y >= ch) return;
-    int master = 0;
-    for (int f = 0; f < n; f++) {
-        const ImpGifFrame fr = frames[f];
-        const int rowidx = fr.h + fr.top - y - 1;
-        int idx;
-        // advancedio.c:203 tests `x > left + w`, so the column right of the frame reads row[w]: a pad byte of the
-        // scanline or the first index of the next one. Reproduced while that byte is inside the page's pixel block.
-        const int col = x - fr.left;
-        if (rowidx < 0 || rowidx >= fr.h || col < 0 || col > fr.w || rowidx * fr.pitch + col >= fr.h * fr.pitch) idx = fr.key;
-        else idx = __ldg(fr.indices + (size_t)rowidx * fr.pitch + col);
-        if (destructive) {
-            if (fr.dispose == 2) {                       // GIF_DISPOSAL_BACKGROUND
-                if (idx == fr.key) idx = 0; else master = idx;
-            } else {                                     // LEAVE / PREVIOUS / UNSPECIFIED
-                if (idx == fr.key && f > 0) idx = master; else master = idx;
-            }
-        }
-        // idx is 0..255 or -1 (a page without a transparent colour). palette[-1] aliases FreeImage's biClrImportant == 256,
-        // i.e. the bytes {0,1,0,0} (advancedio.c:232 with FreeImage_GetTransparentIndex == -1).
-        uchar4 q = make_uchar4(0, 1, 0, 0);
-        if (idx >= 0 && idx < 256) q = __ldg(reinterpret_cast<const uchar4*>(fr.palette) + idx);
-        const uchar4 px = make_uchar4(q.x, q.y, q.z, idx == fr.key ? 0 : 255);
-        *reinterpret_cast<uchar4*>(canvases + ((size_t)f * ch + y) * cpitch + (size_t)x * 4) = px;
-    }
+// GIF canvas expansion (SURVEY 8f-2; advancedio.c:195-248) of every album of a round in one launch: each thread owns one
+// canvas pixel of one album, walks that album's pages in order and writes one BGRA pixel per page (imp_gif.cuh). Pages
+// travel over PCIe as 8-bit indices (4x fewer bytes than the BGRA canvases the CPU path builds).
+__global__ void __launch_bounds__(IMP_GIF_THREADS) imp_gif_expand_kernel(const ImpGifAlbum* __restrict__ albums, int n_albums,
+                                                                         const ImpGifFrame* __restrict__ pages,
+                                                                         uint8_t* __restrict__ arena, size_t arena_bytes) {
+    imp_gif_expand_thread(albums, n_albums, pages, arena, arena_bytes, (long long)blockIdx.x, (int)threadIdx.x);
 }
 
-cudaError_t imp_launch_gif_expand(const ImpGifFrame* d_frames, int n, int cw, int ch, int destructive, uint8_t* d_canvases, int cpitch, cudaStream_t st) {
-    dim3 grid((cw + 255) / 256, ch);
-    imp_gif_expand_kernel<<<grid, 256, 0, st>>>(d_frames, n, cw, ch, destructive, d_canvases, cpitch);
+cudaError_t imp_launch_gif_expand(const ImpGifAlbum* d_albums, int n_albums, const ImpGifFrame* d_pages, long long blocks,
+                                  uint8_t* d_arena, size_t arena_bytes, cudaStream_t st) {
+    imp_gif_expand_kernel<<<(unsigned)blocks, IMP_GIF_THREADS, 0, st>>>(d_albums, n_albums, d_pages, d_arena, arena_bytes);
     g_imp_launches++;
     return cudaGetLastError();
 }
+
+unsigned imp_debug_flags_kernels() { return imp_debug_flags_tu(); }
 
 namespace {
 

@@ -38,6 +38,25 @@ static __device__ unsigned g_imp_recip31[256];
 static __device__ int2 g_imp_hsv[256];
 #endif
 
+// ---- debug build (-DIMP_DEBUG_BOUNDS; ngx_http_imgproc_b200/build.py --debug -> libimp_gpu_dbg.so) -----------------------
+// compute-sanitizer is not available on the GPU pool, so the tile kernels and the GIF expansion carry their own bounds
+// assertions on every staged-tile, lookup-table, out-stage, index-plane, canvas and destination address they form; a
+// violated one sets a bit of the translation unit's flag word that imp_gpu_debug_flags() reads back (tests/test_gpu_host_path.py
+// runs the request fuzz over the debug build). Bits: 0-1 blur (border fill, out stage), 2-3 cubic, 4-6 gather tile, 8-11 strip
+// kernels (tile reads, taps, destination), 12-13 GIF expansion (index plane, canvas). Host code (the test harness) checks nothing.
+#if defined(IMP_DEBUG_BOUNDS) && defined(__CUDACC__)
+static __device__ unsigned g_imp_dbg_flags;
+#if defined(__CUDA_ARCH__)
+#define IMP_DBG(cond, bit) do { if (!(cond)) atomicOr(&g_imp_dbg_flags, 1u << (bit)); } while (0)
+#else
+#define IMP_DBG(cond, bit) do { } while (0)
+#endif
+static inline unsigned imp_debug_flags_tu() { unsigned v = 0; cudaMemcpyFromSymbol(&v, g_imp_dbg_flags, sizeof v); return v; }
+#else
+#define IMP_DBG(cond, bit) do { } while (0)
+static inline unsigned imp_debug_flags_tu() { return 0; }
+#endif
+
 #if defined(__CUDA_ARCH__)
 #define IMP_FMUL(a, b) __fmul_rn((a), (b))
 #define IMP_FADD(a, b) __fadd_rn((a), (b))

@@ -167,3 +167,14 @@ struct ImpGifFrame {
     const uint8_t* palette;   // device pointer, 256 * 4 bytes
     int pitch, w, h, left, top, dispose, key, pad_;
 };
+
+// Threads of one GIF expansion block. Every album's pixels start on a block edge, so a block serves exactly one album.
+#define IMP_GIF_THREADS 256
+
+// One album of a round of GIF albums, as the expansion kernel reads it from the device table (imp_gif.cuh).
+struct ImpGifAlbum {
+    unsigned long long canvas_off;   // the album's first canvas in the arena (page f at canvas_off + f * pitch * ch)
+    long long blk0;                  // the album's first block of the expansion grid
+    int first, n;                    // pages [first, first + n) of the round's page table
+    int cw, ch, pitch, destructive;
+};

@@ -6,21 +6,7 @@
 // footprint); these are selected per job when the source rows are 16-byte addressable
 // (pick_launch, imp_gpu.cu) and the footprint fits the shared-memory budget.
 #pragma once
-#include "imp_gather.cuh"
-
-// ---- debug build (-DIMP_DEBUG_BOUNDS; ngx_http_imgproc_b200/build.py --debug -> libimp_gpu_dbg.so) -----------------------
-// compute-sanitizer is not available on the GPU pool, so the tile kernels carry their own bounds assertions on every
-// staged-tile, lookup-table, out-stage and destination address they form; a violated one sets a bit that
-// imp_gpu_debug_flags() reads back (tests/test_gpu_host_path.py runs the request fuzz over the debug build). Bits:
-// 0-1 blur (border fill, out stage), 2-3 cubic, 4-6 gather tile, 8-11 strip kernels (tile reads, taps, destination).
-#if defined(IMP_DEBUG_BOUNDS)
-static __device__ unsigned g_imp_dbg_flags;
-#define IMP_DBG(cond, bit) do { if (!(cond)) atomicOr(&g_imp_dbg_flags, 1u << (bit)); } while (0)
-static inline unsigned imp_debug_flags_tu() { unsigned v = 0; cudaMemcpyFromSymbol(&v, g_imp_dbg_flags, sizeof v); return v; }
-#else
-#define IMP_DBG(cond, bit) do { } while (0)
-static inline unsigned imp_debug_flags_tu() { return 0; }
-#endif
+#include "imp_gather.cuh"      // imp_pixel.cuh: IMP_DBG, the bounds assertions of the debug build
 
 namespace imp_tiles {
 

@@ -1,7 +1,9 @@
 // imp_transfer.cpp — how the chunked host path moves a batch over the link: where the batch is cut into chunks, and
-// how each job's source reaches the device and its result comes back. Pure host logic (no CUDA call): the caller says
-// which buffers are page-locked, so tests/test_transfer_plan.py pins every decision on the CPU.
+// how each job's source reaches the device and its result comes back; for GIF albums, where the album list is cut into
+// rounds and how a round's pages are packed for their one upload. Pure host logic (no CUDA call): the caller says which
+// buffers are page-locked, so tests/test_transfer_plan.py and tests/test_gif_albums.py pin every decision on the CPU.
 #include "imp_internal.h"
+#include <string.h>
 #include <algorithm>
 
 // The size of an ASCII answer (include/imp_gpu.h). Defined here because it is a rule of the layout below (an ASCII job's
@@ -91,4 +93,67 @@ ImpChunkLayout imp_chunk_layout(const ImpHostJob* jobs, int m, ImpResult kind, b
         }
     }
     return c;
+}
+
+// ---- GIF albums ------------------------------------------------------------------------------------------------------
+namespace {
+size_t a16(size_t v) { return (v + 15) & ~size_t(15); }
+}  // namespace
+
+size_t imp_gif_canvas_bytes(const imp_gpu_gif_album& a) {
+    return align256((size_t)align16(a.canvas_w * 4) * a.canvas_h * a.n_pages);
+}
+
+// A round's canvases stay resident until its last frame has run, and the next round reuses them: the budget bounds the
+// device memory a call holds whatever the number of albums, while a round of thumbnails still holds hundreds of albums.
+std::vector<int> imp_gif_round_bounds(const imp_gpu_gif_album* albums, int n) {
+    std::vector<int> bounds{0};
+    for (int i = 0; i < n;) {
+        int e = i; size_t bytes = 0;
+        while (e < n) {
+            const size_t need = imp_gif_canvas_bytes(albums[e]);
+            if (e > i && bytes + need > IMP_GIF_ROUND_BYTES) break;
+            bytes += need; e++;
+        }
+        bounds.push_back(e);
+        i = e;
+    }
+    return bounds;
+}
+
+ImpGifRound imp_gif_round_layout(const imp_gpu_gif_album* albums, int n, int pitch) {
+    ImpGifRound r;
+    r.albums.resize(n);
+    size_t canvas = 0;
+    long long blk = 0;
+    for (int a = 0; a < n; a++) {
+        const imp_gpu_gif_album& al = albums[a];
+        const int pt = pitch ? pitch : align16(al.canvas_w * 4);
+        r.albums[a] = ImpGifAlbum{canvas, blk, (int)r.pages.size(), al.n_pages, al.canvas_w, al.canvas_h, pt, al.destructive ? 1 : 0};
+        canvas += pitch ? (size_t)pt * al.canvas_h * al.n_pages : imp_gif_canvas_bytes(al);
+        blk += ((long long)al.canvas_w * al.canvas_h + IMP_GIF_THREADS - 1) / IMP_GIF_THREADS;
+        for (int f = 0; f < al.n_pages; f++) r.pages.push_back(&al.pages[f]);
+    }
+    const size_t np = r.pages.size();
+    r.arena_bytes = canvas;
+    r.blocks = blk;
+    r.page_off = a16((size_t)n * sizeof(ImpGifAlbum));
+    r.pal_off = r.page_off + a16(np * sizeof(ImpGifFrame));
+    size_t off = r.pal_off + np * 1024;
+    r.idx_off.resize(np);
+    for (size_t k = 0; k < np; k++) { r.idx_off[k] = off; off += a16((size_t)r.pages[k]->pitch * r.pages[k]->height); }
+    r.pack_bytes = off;
+    return r;
+}
+
+void imp_gif_pack_page(const ImpGifRound& r, int k, uint8_t* h_buf, const uint8_t* d_buf, void (*copy)(uint8_t*, const uint8_t*, size_t)) {
+    if (k == 0) memcpy(h_buf, r.albums.data(), r.albums.size() * sizeof(ImpGifAlbum));
+    const imp_gpu_gif_frame& g = *r.pages[k];
+    const size_t pal = r.pal_off + (size_t)k * 1024;
+    memcpy(h_buf + pal, g.palette, 1024);
+    copy(h_buf + r.idx_off[k], g.indices, (size_t)g.pitch * g.height);
+    ImpGifFrame& m = reinterpret_cast<ImpGifFrame*>(h_buf + r.page_off)[k];
+    m.indices = d_buf + r.idx_off[k]; m.palette = d_buf + pal;
+    m.pitch = g.pitch; m.w = g.width; m.h = g.height; m.left = g.left; m.top = g.top;
+    m.dispose = g.dispose; m.key = g.transparency_key; m.pad_ = 0;
 }

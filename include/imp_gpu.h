@@ -203,7 +203,10 @@ int  imp_gpu_batch_run_host(int n, imp_gpu_plan* const* plans, const unsigned ch
 /* Asynchronous form (SURVEY 8b-4 submit/wait): checks every job (a bad one: IMP_ERROR_INVALID_ARGS, no ticket), then
  * returns at once with a ticket; a helper thread drives the batch on the caller's current device. The argument arrays
  * are copied, the pixel buffers must stay valid until imp_gpu_batch_wait, which blocks, returns the batch's code and
- * frees the ticket. imp_gpu_batch_poll: 1 when finished, 0 while running. */
+ * frees the ticket. imp_gpu_batch_poll: 1 when finished, 0 while running. Every plan holds a reference until the wait,
+ * so imp_gpu_plan_destroy right after the submit is safe. On any failure *ticket = NULL and nothing is written; n == 0
+ * gives a ticket whose wait returns IMP_OK. imp_gpu_batch_brightness_submit_host, imp_gpu_batch_ascii_submit_host and
+ * imp_gpu_gif_albums_submit_host (below) are the same for their calls, and poll and wait serve every kind of ticket. */
 int  imp_gpu_batch_submit_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs,
                                const int* src_steps, unsigned char* const* dsts, const int* dst_steps,
                                int n_streams, imp_gpu_ticket** ticket);
@@ -239,6 +242,15 @@ int  imp_gpu_batch_brightness_host(int n, imp_gpu_plan* const* plans, const unsi
                                    float* brightness, int n_streams);
 int  imp_gpu_batch_ascii_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                               const char* const* args, unsigned char* const* texts, const long* text_caps, int n_streams);
+/* Asynchronous forms of the two calls above, as imp_gpu_batch_submit_host is of imp_gpu_batch_run_host: every check of the
+ * synchronous call runs at the submit (a packed answer or a text_caps[i] smaller than the text: IMP_ERROR_INVALID_ARGS,
+ * no ticket, nothing written). The argument arrays are copied, each ASCII job's ramp is taken from args[i] at the submit;
+ * the sources and the brightness / texts buffers must stay valid until imp_gpu_batch_wait. */
+int  imp_gpu_batch_brightness_submit_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs,
+                                          const int* src_steps, float* brightness, int n_streams, imp_gpu_ticket** ticket);
+int  imp_gpu_batch_ascii_submit_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                                     const char* const* args, unsigned char* const* texts, const long* text_caps,
+                                     int n_streams, imp_gpu_ticket** ticket);
 
 /* One frame already decoded: what Info() (bridge.c:283-300) prints as round(brightness*100). The reference accumulates
  * float32 in column-major order; the device sums in double (the same reduction as the batch call, so a frame gives the same
@@ -300,6 +312,10 @@ typedef struct imp_gpu_gif_album {
  * steps): one bad album returns IMP_ERROR_INVALID_ARGS and no destination of any album is written. n_albums == 0 returns
  * IMP_OK. Synchronous, on the current device. */
 int  imp_gpu_gif_albums_run_host(const imp_gpu_gif_album* albums, int n_albums, int n_streams);
+/* Asynchronous form, as imp_gpu_batch_submit_host is of imp_gpu_batch_run_host: every album is checked at the submit (one
+ * bad album: IMP_ERROR_INVALID_ARGS, no ticket, nothing written). The album descriptors and their pages, plans, dsts and
+ * dst_steps arrays are copied; the index planes, palettes and destinations must stay valid until imp_gpu_batch_wait. */
+int  imp_gpu_gif_albums_submit_host(const imp_gpu_gif_album* albums, int n_albums, int n_streams, imp_gpu_ticket** ticket);
 
 /* ---- memory helpers so a C host needs no CUDA headers --------------------------------------------- */
 int  imp_gpu_malloc(void** d_ptr, size_t bytes);

@@ -153,6 +153,11 @@ class Library:
         L.imp_gpu_ascii_length.argtypes = [C.c_int, C.c_int]
         L.imp_gpu_batch_brightness_host.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.imp_gpu_batch_ascii_host.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
+        L.imp_gpu_batch_brightness_submit_host.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]
+        L.imp_gpu_batch_ascii_submit_host.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                      C.POINTER(C.c_void_p)]
+        L.imp_gpu_gif_albums_submit_host.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        self.in_flight = {}          # ticket -> what its buffers live in, kept until HostJobs.wait
 
     # ---- lifetime ---------------------------------------------------------------------------------
     def last_error(self) -> str:
@@ -263,16 +268,40 @@ class Library:
 
     def batch_ascii(self, plans: List["Plan"], srcs: List[np.ndarray], args=None, n_streams: int = 4) -> List[bytes]:
         """imp_gpu_batch_ascii_host: ASCII of each result. `args`: one value for every job or a list (None: 10-level ramp)."""
+        a = self._ascii_arrays(plans, srcs, args)
+        self.check(self.lib.imp_gpu_batch_ascii_host(len(plans), *a[:6], n_streams))
+        return [b.tobytes() for b in a[6]]
+
+    def _ascii_arrays(self, plans, srcs, args):
+        """The ASCII calls' arguments: plans, sources, steps, args, text pointers, capacities, then the texts (numpy arrays
+        of exactly each text's length)."""
         n = len(plans)
-        P, S, SS = _job_arrays(plans, srcs)
         args = list(args) if isinstance(args, (list, tuple)) else [args] * n
         A = (C.c_char_p * max(n, 1))(*[None if a is None else a.encode() for a in args])
         lens = [self.lib.imp_gpu_ascii_length(p.out_w, p.out_h) for p in plans]
-        bufs = [C.create_string_buffer(max(k, 1)) for k in lens]
-        T = (C.c_void_p * max(n, 1))(*[C.addressof(b) for b in bufs])
+        texts = [np.zeros(k, np.uint8) for k in lens]
+        T = (C.c_void_p * max(n, 1))(*[t.ctypes.data for t in texts])
         caps = (C.c_long * max(n, 1))(*lens)
-        self.check(self.lib.imp_gpu_batch_ascii_host(n, P, S, SS, A, T, caps, n_streams))
-        return [b.raw[:k] for b, k in zip(bufs, lens)]
+        return _job_arrays(plans, srcs) + (A, T, caps, texts)
+
+    # The submits return at once with a ticket for HostJobs.poll / HostJobs.wait; the arrays they fill are returned beside it
+    # and, with the sources, kept alive by the library handle until the wait.
+    def batch_brightness_submit(self, plans: List["Plan"], srcs: List[np.ndarray], n_streams: int = 4):
+        """imp_gpu_batch_brightness_submit_host: (ticket, float32 array the brightnesses land in)."""
+        P, S, SS = _job_arrays(plans, srcs)
+        out = np.zeros(len(plans), np.float32)
+        t = C.c_void_p()
+        self.check(self.lib.imp_gpu_batch_brightness_submit_host(len(plans), P, S, SS, out.ctypes.data, n_streams, C.byref(t)))
+        self.in_flight[t.value] = (srcs, out)
+        return t, out
+
+    def batch_ascii_submit(self, plans: List["Plan"], srcs: List[np.ndarray], args=None, n_streams: int = 4):
+        """imp_gpu_batch_ascii_submit_host: (ticket, one uint8 array per job that its text lands in; .tobytes() after the wait)."""
+        a = self._ascii_arrays(plans, srcs, args)
+        t = C.c_void_p()
+        self.check(self.lib.imp_gpu_batch_ascii_submit_host(len(plans), *a[:6], n_streams, C.byref(t)))
+        self.in_flight[t.value] = (srcs, a[6])
+        return t, a[6]
 
     # ---- plans --------------------------------------------------------------------------------------
     def plan(self, w, h, c, cfg: Optional[Config] = None, **req) -> "Plan":
@@ -392,15 +421,19 @@ class HostJobs:
         """imp_gpu_batch_submit_host: returns a ticket for wait()."""
         t = C.c_void_p()
         lib.check(lib.lib.imp_gpu_batch_submit_host(self.n, self.P, self.S, self.SS, self.D, self.DS, n_streams, C.byref(t)))
+        lib.in_flight[t.value] = self
         return t
 
+    # poll and wait take a ticket of any submit
     @staticmethod
     def poll(lib: Library, ticket) -> bool:
         return bool(lib.lib.imp_gpu_batch_poll(ticket))
 
     @staticmethod
     def wait(lib: Library, ticket):
+        keep = lib.in_flight.pop(ticket.value, None)      # taken before the wait frees the ticket (its address may be reused)
         lib.check(lib.lib.imp_gpu_batch_wait(ticket))
+        del keep
 
 
 class GifAlbumJob:
@@ -442,6 +475,17 @@ class GifAlbumsJob:
 
     def run(self, lib: Library, n_streams=4):
         lib.check(lib.lib.imp_gpu_gif_albums_run_host(self.arr, self.n, n_streams))
+        return self.outs
+
+    def submit(self, lib: Library, n_streams=4):
+        """imp_gpu_gif_albums_submit_host: returns a ticket for HostJobs.wait(); the results land in `outs`."""
+        t = C.c_void_p()
+        lib.check(lib.lib.imp_gpu_gif_albums_submit_host(self.arr, self.n, n_streams, C.byref(t)))
+        lib.in_flight[t.value] = self
+        return t
+
+    @property
+    def outs(self):
         return [j.outs for j in self.jobs]
 
 

@@ -841,6 +841,7 @@ int run_host_chunked_locked(const ImpHostJob* jobs, int n, ImpResult kind, int n
     return result;
 }
 int run_host_chunked(const std::vector<ImpHostJob>& jobs, ImpResult kind, int n_streams) {
+    if (jobs.empty()) return IMP_OK;
     std::lock_guard<std::mutex> run_lk(g_dev[t_dev].run_mu);
     return run_host_chunked_locked(jobs.data(), (int)jobs.size(), kind, n_streams, false, nullptr);
 }
@@ -865,6 +866,35 @@ std::vector<ImpHostJob> host_jobs(int n, imp_gpu_plan* const* plans, const unsig
     std::vector<ImpHostJob> v(n);
     for (int i = 0; i < n; i++) v[i] = ImpHostJob{plans[i], srcs[i], src_steps[i], dsts ? dsts[i] : nullptr, dst_steps ? dst_steps[i] : 0, false};
     return v;
+}
+
+// The "build and check" halves of the frame, brightness and ASCII calls: the job list the run takes (empty when n <= 0), or
+// the code the call refuses with. The synchronous call and its submit both take their jobs from here.
+int frame_jobs(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+               unsigned char* const* dsts, const int* dst_steps, std::vector<ImpHostJob>& jobs) {
+    if (n <= 0) return IMP_OK;
+    if (!plans || !srcs || !src_steps || !dsts || !dst_steps) return IMP_ERROR_INVALID_ARGS;
+    jobs = host_jobs(n, plans, srcs, src_steps, dsts, dst_steps);
+    return check_host_jobs(ImpResult::Frame, jobs);
+}
+int brightness_jobs(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps, float* brightness,
+                    std::vector<ImpHostJob>& jobs) {
+    if (n <= 0) return IMP_OK;
+    if (!plans || !srcs || !src_steps || !brightness) return IMP_ERROR_INVALID_ARGS;
+    jobs = host_jobs(n, plans, srcs, src_steps);
+    for (int i = 0; i < n; i++) jobs[i].dst = reinterpret_cast<uint8_t*>(brightness + i);
+    return check_host_jobs(ImpResult::Brightness, jobs);
+}
+int ascii_jobs(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps, const char* const* args,
+               unsigned char* const* texts, const long* text_caps, std::vector<ImpHostJob>& jobs) {
+    if (n <= 0) return IMP_OK;
+    if (!plans || !srcs || !src_steps || !args || !texts || !text_caps) return IMP_ERROR_INVALID_ARGS;
+    jobs = host_jobs(n, plans, srcs, src_steps);
+    for (int i = 0; i < n; i++) {
+        jobs[i].dst = texts[i];
+        jobs[i].wide = args[i] && strcmp(args[i], "wide") == 0;                  // filters.c:490-494
+    }
+    return check_host_jobs(ImpResult::Ascii, jobs, text_caps);
 }
 
 // The checks imp_gpu_run_device and imp_gpu_batch_add make on a device job.
@@ -931,12 +961,52 @@ int device_list(const char* spec, int n_devices, int* list, int* len) {
 
 }  // namespace
 
+// A host call in flight: what its "build and check" half captured, and its "run" half, which a helper thread applies to
+// that on the device the caller had current at the submit.
 struct imp_gpu_ticket {
     std::thread th;
     int rc = IMP_OK; std::string err;
     std::atomic<bool> done{false};
-    std::vector<ImpHostJob> jobs;
+    std::vector<ImpHostJob> jobs;                        // each plan holds one more reference until the wait
+    std::function<int(std::vector<ImpHostJob>&)> run;
 };
+
+namespace {
+
+// Every submit ends here once its call's checks have passed: the ticket takes the job list and the run, and the helper
+// thread starts. Nothing throws out of it; an allocation that fails leaves no ticket and no extra plan reference.
+int start_ticket(std::vector<ImpHostJob> jobs, std::function<int(std::vector<ImpHostJob>&)> run, imp_gpu_ticket** ticket) {
+    imp_gpu_ticket* t = nullptr;
+    bool held = false;
+    try {
+        t = new imp_gpu_ticket();
+        t->jobs = std::move(jobs); t->run = std::move(run);
+        for (const ImpHostJob& j : t->jobs) j.plan->refs.fetch_add(1);       // the call keeps its plans alive
+        held = true;
+        const int dev = t_dev;
+        t->th = std::thread([t, dev]() {
+            int r = imp_gpu_set_device(dev);
+            if (r == IMP_OK) {
+                try { r = t->run(t->jobs); } catch (const std::bad_alloc&) { r = IMP_ERROR_MALLOC_FAILED; }
+            }
+            t->rc = r;
+            if (r) t->err = t_err;
+            t->done.store(true, std::memory_order_release);
+        });
+    } catch (...) {
+        if (t) { if (held) for (const ImpHostJob& j : t->jobs) plan_release(j.plan); delete t; }
+        return IMP_ERROR_MALLOC_FAILED;
+    }
+    *ticket = t;
+    return IMP_OK;
+}
+
+// The "run" half of the frame, brightness and ASCII calls.
+std::function<int(std::vector<ImpHostJob>&)> chunked_run(ImpResult kind, int n_streams) {
+    return [kind, n_streams](std::vector<ImpHostJob>& jobs) { return run_host_chunked(jobs, kind, n_streams); };
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -1211,11 +1281,9 @@ int imp_gpu_run_host(imp_gpu_plan* plan, const unsigned char* src, int src_step,
 int imp_gpu_batch_run_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                            unsigned char* const* dsts, const int* dst_steps, int n_streams) {
     int rc = bind(); if (rc) return rc;
-    if (n <= 0) return IMP_OK;
-    if (!plans || !srcs || !src_steps || !dsts || !dst_steps) return IMP_ERROR_INVALID_ARGS;
     try {
-        const std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps, dsts, dst_steps);
-        if ((rc = check_host_jobs(ImpResult::Frame, jobs))) return rc;
+        std::vector<ImpHostJob> jobs;
+        if ((rc = frame_jobs(n, plans, srcs, src_steps, dsts, dst_steps, jobs))) return rc;
         return run_host_chunked(jobs, ImpResult::Frame, n_streams);
     } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
@@ -1228,29 +1296,12 @@ int imp_gpu_batch_submit_host(int n, imp_gpu_plan* const* plans, const unsigned 
     if (!ticket) return IMP_ERROR_INVALID_ARGS;
     *ticket = nullptr;
     int rc = bind(); if (rc) return rc;
-    if (n < 0 || (n > 0 && (!plans || !srcs || !src_steps || !dsts || !dst_steps))) return IMP_ERROR_INVALID_ARGS;
-    imp_gpu_ticket* t = nullptr;
+    if (n < 0) return IMP_ERROR_INVALID_ARGS;
     try {
-        t = new imp_gpu_ticket();
-        t->jobs = host_jobs(n, plans, srcs, src_steps, dsts, dst_steps);
-        if ((rc = check_host_jobs(ImpResult::Frame, t->jobs))) { delete t; return rc; }
-        for (const ImpHostJob& j : t->jobs) j.plan->refs.fetch_add(1);       // the batch keeps its plans alive
-        const int dev = t_dev;
-        t->th = std::thread([t, dev, n_streams]() {
-            int r = imp_gpu_set_device(dev);
-            if (r == IMP_OK && !t->jobs.empty()) {
-                try { r = run_host_chunked(t->jobs, ImpResult::Frame, n_streams); } catch (const std::bad_alloc&) { r = IMP_ERROR_MALLOC_FAILED; }
-            }
-            t->rc = r;
-            if (r) t->err = t_err;
-            t->done.store(true, std::memory_order_release);
-        });
-    } catch (...) {
-        if (t) { for (const ImpHostJob& j : t->jobs) plan_release(j.plan); delete t; }
-        return IMP_ERROR_MALLOC_FAILED;
-    }
-    *ticket = t;
-    return IMP_OK;
+        std::vector<ImpHostJob> jobs;
+        if ((rc = frame_jobs(n, plans, srcs, src_steps, dsts, dst_steps, jobs))) return rc;
+        return start_ticket(std::move(jobs), chunked_run(ImpResult::Frame, n_streams), ticket);
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
 
 int imp_gpu_batch_poll(const imp_gpu_ticket* ticket) { return ticket && ticket->done.load(std::memory_order_acquire) ? 1 : 0; }
@@ -1336,12 +1387,9 @@ int imp_gpu_farm_run_host(int n, imp_gpu_plan* const* plans, const unsigned char
 int imp_gpu_batch_brightness_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                                   float* brightness, int n_streams) {
     int rc = bind(); if (rc) return rc;
-    if (n <= 0) return IMP_OK;
-    if (!plans || !srcs || !src_steps || !brightness) return IMP_ERROR_INVALID_ARGS;
     try {
-        std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps);
-        for (int i = 0; i < n; i++) jobs[i].dst = reinterpret_cast<uint8_t*>(brightness + i);
-        if ((rc = check_host_jobs(ImpResult::Brightness, jobs))) return rc;
+        std::vector<ImpHostJob> jobs;
+        if ((rc = brightness_jobs(n, plans, srcs, src_steps, brightness, jobs))) return rc;
         return run_host_chunked(jobs, ImpResult::Brightness, n_streams);
     } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
@@ -1349,16 +1397,36 @@ int imp_gpu_batch_brightness_host(int n, imp_gpu_plan* const* plans, const unsig
 int imp_gpu_batch_ascii_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
                              const char* const* args, unsigned char* const* texts, const long* text_caps, int n_streams) {
     int rc = bind(); if (rc) return rc;
-    if (n <= 0) return IMP_OK;
-    if (!plans || !srcs || !src_steps || !args || !texts || !text_caps) return IMP_ERROR_INVALID_ARGS;
     try {
-        std::vector<ImpHostJob> jobs = host_jobs(n, plans, srcs, src_steps);
-        for (int i = 0; i < n; i++) {
-            jobs[i].dst = texts[i];
-            jobs[i].wide = args[i] && strcmp(args[i], "wide") == 0;                  // filters.c:490-494
-        }
-        if ((rc = check_host_jobs(ImpResult::Ascii, jobs, text_caps))) return rc;
+        std::vector<ImpHostJob> jobs;
+        if ((rc = ascii_jobs(n, plans, srcs, src_steps, args, texts, text_caps, jobs))) return rc;
         return run_host_chunked(jobs, ImpResult::Ascii, n_streams);
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+}
+
+// Asynchronous forms of the two above (imp_gpu_batch_submit_host's contract): each ASCII job's ramp is taken at the submit.
+int imp_gpu_batch_brightness_submit_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                                         float* brightness, int n_streams, imp_gpu_ticket** ticket) {
+    if (!ticket) return IMP_ERROR_INVALID_ARGS;
+    *ticket = nullptr;
+    int rc = bind(); if (rc) return rc;
+    try {
+        std::vector<ImpHostJob> jobs;
+        if ((rc = brightness_jobs(n, plans, srcs, src_steps, brightness, jobs))) return rc;
+        return start_ticket(std::move(jobs), chunked_run(ImpResult::Brightness, n_streams), ticket);
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+}
+
+int imp_gpu_batch_ascii_submit_host(int n, imp_gpu_plan* const* plans, const unsigned char* const* srcs, const int* src_steps,
+                                    const char* const* args, unsigned char* const* texts, const long* text_caps, int n_streams,
+                                    imp_gpu_ticket** ticket) {
+    if (!ticket) return IMP_ERROR_INVALID_ARGS;
+    *ticket = nullptr;
+    int rc = bind(); if (rc) return rc;
+    try {
+        std::vector<ImpHostJob> jobs;
+        if ((rc = ascii_jobs(n, plans, srcs, src_steps, args, texts, text_caps, jobs))) return rc;
+        return start_ticket(std::move(jobs), chunked_run(ImpResult::Ascii, n_streams), ticket);
     } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
 
@@ -1474,63 +1542,95 @@ int imp_gpu_gif_album_run_host(const imp_gpu_gif_frame* frames, int n, int canva
     return imp_gpu_gif_albums_run_host(&album, 1, n_streams);
 }
 
-// Many GIF requests: per round (imp_gif_round_bounds) one pack of all its albums' pages, one upload, one expansion launch
-// and one chunked frame loop over all its albums' frames, so that chunks and grouped launches span requests.
-int imp_gpu_gif_albums_run_host(const imp_gpu_gif_album* albums, int n_albums, int n_streams) {
-    int rc = bind(); if (rc) return rc;
-    if (n_albums < 0 || (n_albums > 0 && !albums)) return IMP_ERROR_INVALID_ARGS;
-    if (n_albums == 0) return IMP_OK;
-    // a frame's source is its page's canvas; the page stands in for it until the canvases are placed, so that a bad job
-    // of any album is refused before any buffer grows or any work starts
-    std::vector<ImpHostJob> jobs;
-    std::vector<int> job0((size_t)n_albums + 1);                     // album a's jobs: [job0[a], job0[a + 1])
-    std::vector<int> rounds;
+// What the run of an albums call needs besides its job list, all of it the library's own: a submit keeps it until the wait.
+struct GifRounds {
+    std::vector<imp_gpu_gif_frame> pages;    // every album's page descriptors, copied; `lay` points into them
+    std::vector<int> page;                   // job k runs on page page[k] of its album
+    std::vector<int> job0;                   // album a's jobs: [job0[a], job0[a + 1])
+    std::vector<int> rounds;                 // imp_gif_round_bounds
     std::vector<ImpGifRound> lay;
     size_t pack_max = 0, arena_max = 0;
-    try {
-        for (int a = 0; a < n_albums; a++) {
-            const imp_gpu_gif_album& al = albums[a];
-            if (al.canvas_w <= 0 || al.canvas_h <= 0 || !al.plans || !al.dsts || !al.dst_steps) return IMP_ERROR_INVALID_ARGS;
-            if ((rc = gif_check_pages(al.pages, al.n_pages))) return rc;
-            job0[a] = (int)jobs.size();
-            for (int f = 0; f < al.n_pages; f++) {
-                imp_gpu_plan* p = al.plans[f];                        // null: replayed for the pages after it, no result wanted
-                if (!p) continue;
-                if (p->src_w != al.canvas_w || p->src_h != al.canvas_h || p->src_c != 4) return IMP_ERROR_INVALID_ARGS;
-                jobs.push_back(ImpHostJob{p, al.pages[f].indices, align16(al.canvas_w * 4), al.dsts[f], al.dst_steps[f], false});
-            }
+};
+
+// The "build and check" half of imp_gpu_gif_albums_run_host. A frame's source is its page's canvas; the page stands in for
+// it until the canvases are placed, so that a bad job of any album is refused before any buffer grows or any work starts.
+static int gif_albums_build(const imp_gpu_gif_album* albums, int n_albums, std::vector<ImpHostJob>& jobs, GifRounds& g) {
+    if (n_albums < 0 || (n_albums > 0 && !albums)) return IMP_ERROR_INVALID_ARGS;
+    std::vector<imp_gpu_gif_album> own(albums, albums + n_albums);   // their `pages` are pointed at g.pages below
+    g.job0.assign((size_t)n_albums + 1, 0);
+    for (int a = 0; a < n_albums; a++) {
+        const imp_gpu_gif_album& al = albums[a];
+        if (al.canvas_w <= 0 || al.canvas_h <= 0 || !al.plans || !al.dsts || !al.dst_steps) return IMP_ERROR_INVALID_ARGS;
+        if (int rc = gif_check_pages(al.pages, al.n_pages)) return rc;
+        g.job0[a] = (int)jobs.size();
+        for (int f = 0; f < al.n_pages; f++) {
+            imp_gpu_plan* p = al.plans[f];                            // null: replayed for the pages after it, no result wanted
+            if (!p) continue;
+            if (p->src_w != al.canvas_w || p->src_h != al.canvas_h || p->src_c != 4) return IMP_ERROR_INVALID_ARGS;
+            jobs.push_back(ImpHostJob{p, al.pages[f].indices, align16(al.canvas_w * 4), al.dsts[f], al.dst_steps[f], false});
+            g.page.push_back(f);
         }
-        job0[n_albums] = (int)jobs.size();
-        if ((rc = check_host_jobs(ImpResult::Frame, jobs))) return rc;
-        rounds = imp_gif_round_bounds(albums, n_albums);
-        for (size_t r = 0; r + 1 < rounds.size(); r++) {
-            lay.push_back(imp_gif_round_layout(albums + rounds[r], rounds[r + 1] - rounds[r]));
-            pack_max = std::max(pack_max, lay.back().pack_bytes);
-            arena_max = std::max(arena_max, lay.back().arena_bytes);
-        }
-    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+        g.pages.insert(g.pages.end(), al.pages, al.pages + al.n_pages);
+    }
+    g.job0[n_albums] = (int)jobs.size();
+    if (int rc = check_host_jobs(ImpResult::Frame, jobs)) return rc;
+    for (int a = 0, f0 = 0; a < n_albums; f0 += own[a].n_pages, a++) own[a].pages = g.pages.data() + f0;
+    g.rounds = imp_gif_round_bounds(own.data(), n_albums);
+    for (size_t r = 0; r + 1 < g.rounds.size(); r++) {
+        g.lay.push_back(imp_gif_round_layout(own.data() + g.rounds[r], g.rounds[r + 1] - g.rounds[r]));
+        g.pack_max = std::max(g.pack_max, g.lay.back().pack_bytes);
+        g.arena_max = std::max(g.arena_max, g.lay.back().arena_bytes);
+    }
+    return IMP_OK;
+}
+
+// The "run" half: per round one pack of all its albums' pages, one upload, one expansion launch and one chunked frame loop
+// over all its albums' frames, so that chunks and grouped launches span requests.
+static int gif_albums_run(const GifRounds& g, std::vector<ImpHostJob>& jobs, int n_streams) {
+    if (g.lay.empty()) return IMP_OK;
     DevCtx& ctx = g_dev[t_dev];
     std::lock_guard<std::mutex> run_lk(ctx.run_mu);
-    if ((rc = ctx.h_gif.grow(pack_max, true)) || (rc = ctx.d_gif.grow(pack_max, false)) || (rc = ctx.d_canvas.grow(arena_max, false))) return rc;
+    int rc;
+    if ((rc = ctx.h_gif.grow(g.pack_max, true)) || (rc = ctx.d_gif.grow(g.pack_max, false)) || (rc = ctx.d_canvas.grow(g.arena_max, false))) return rc;
     if (!ctx.gif_ev) CK(cudaEventCreateWithFlags(&ctx.gif_ev, cudaEventDisableTiming));
     try {                                                             // the C caller cannot unwind: bad_alloc ends as a code
-    for (size_t r = 0; r < lay.size() && rc == IMP_OK; r++) {         // one after another: the pack and the arena are reused
-        const ImpGifRound& R = lay[r];
-        const int a0 = rounds[r], a1 = rounds[r + 1];
+    for (size_t r = 0; r < g.lay.size() && rc == IMP_OK; r++) {       // one after another: the pack and the arena are reused
+        const ImpGifRound& R = g.lay[r];
+        const int a0 = g.rounds[r], a1 = g.rounds[r + 1];
         for (int a = a0; a < a1; a++) {
             const ImpGifAlbum& A = R.albums[a - a0];
-            for (int f = 0, k = job0[a]; f < A.n; f++)
-                if (albums[a].plans[f]) jobs[k++].src = ctx.d_canvas.p + A.canvas_off + (size_t)f * A.pitch * A.ch;
+            for (int k = g.job0[a]; k < g.job0[a + 1]; k++) jobs[k].src = ctx.d_canvas.p + A.canvas_off + (size_t)g.page[k] * A.pitch * A.ch;
         }
         CK(gif_round_expand(R, ctx.h_gif.p, ctx.d_gif.p, ctx.d_canvas.p, ctx.stream));
         CK(cudaEventRecord(ctx.gif_ev, ctx.stream));
-        const int j0 = job0[a0], j1 = job0[a1];
+        const int j0 = g.job0[a0], j1 = g.job0[a1];
         if (j0 == j1) CK(cudaStreamSynchronize(ctx.stream));
         else rc = run_host_chunked_locked(jobs.data() + j0, j1 - j0, ImpResult::Frame, n_streams, true, ctx.gif_ev);
     }
     } catch (const std::bad_alloc&) { rc = IMP_ERROR_MALLOC_FAILED; }
     if (rc != IMP_OK) cudaStreamSynchronize(ctx.stream);           // the staging buffers are reused by the next call
     return rc;
+}
+
+int imp_gpu_gif_albums_run_host(const imp_gpu_gif_album* albums, int n_albums, int n_streams) {
+    int rc = bind(); if (rc) return rc;
+    std::vector<ImpHostJob> jobs;
+    GifRounds g;
+    try { if ((rc = gif_albums_build(albums, n_albums, jobs, g))) return rc; }
+    catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
+    return gif_albums_run(g, jobs, n_streams);
+}
+
+int imp_gpu_gif_albums_submit_host(const imp_gpu_gif_album* albums, int n_albums, int n_streams, imp_gpu_ticket** ticket) {
+    if (!ticket) return IMP_ERROR_INVALID_ARGS;
+    *ticket = nullptr;
+    int rc = bind(); if (rc) return rc;
+    try {
+        std::vector<ImpHostJob> jobs;
+        auto g = std::make_shared<GifRounds>();
+        if ((rc = gif_albums_build(albums, n_albums, jobs, *g))) return rc;
+        return start_ticket(std::move(jobs), [g, n_streams](std::vector<ImpHostJob>& j) { return gif_albums_run(*g, j, n_streams); }, ticket);
+    } catch (const std::bad_alloc&) { return IMP_ERROR_MALLOC_FAILED; }
 }
 
 int imp_gpu_gif_expand_host(const imp_gpu_gif_frame* frames, int n, int canvas_w, int canvas_h, int destructive,

@@ -403,7 +403,7 @@ ImpJob make_job(const imp_gpu_plan* p, int d, size_t k, const uint8_t* src, int 
 }
 
 // Turns `items` into launch steps and the jobs they cover (in device-table order), pass by pass. Within a pass the jobs are
-// grouped by (kind, sc, kernel, param, flavour, ctas_per_sm), one launch per group in that order; a generic blur is a step
+// grouped by (kind, exact integer AREA taps, sc, kernel, param, flavour, ctas_per_sm), one launch per group in that order; a generic blur is a step
 // of its own. alloc(bytes, &p): where the items' scratch lives (plan_scratch_layout, item after item).
 template <class Alloc>
 int build_steps(const std::vector<imp_gpu_batch::Item>& items, Alloc alloc, imp_gpu_batch::TmCache* tmaps,
@@ -420,7 +420,7 @@ int build_steps(const std::vector<imp_gpu_batch::Item>& items, Alloc alloc, imp_
     if (int rc = alloc(bytes, &scratch)) return rc;
     struct Pending {
         const ImpPass* hdr; ImpLaunch l; ImpJob job; uint16_t* plane;
-        auto key() const { return std::make_tuple(hdr->kind, hdr->sc, l.kernel, l.param, l.flavour, l.ctas_per_sm); }
+        auto key() const { return std::make_tuple(hdr->kind, hdr->area_d != 0, hdr->sc, l.kernel, l.param, l.flavour, l.ctas_per_sm); }
     };
     std::vector<Pending> pend;
     for (size_t k = 0; k < max_passes; k++) {
@@ -439,7 +439,8 @@ int build_steps(const std::vector<imp_gpu_batch::Item>& items, Alloc alloc, imp_
             const bool generic = pend[s].l.kernel == ImpKernel::BlurGeneric;
             for (e = s + 1; e < pend.size() && !generic && pend[e].key() == pend[s].key(); e++) {}
             imp_gpu_batch::Step st{};
-            st.g = ImpLaunchGroup{pend[s].hdr->kind, pend[s].hdr->sc, pend[s].l.kernel, pend[s].l.param, pend[s].l.flavour, (int)jobs.size(), (int)(e - s), 0, 0};
+            st.g = ImpLaunchGroup{pend[s].hdr->kind, pend[s].hdr->sc, pend[s].l.kernel, pend[s].l.param, pend[s].l.flavour, (int)jobs.size(), (int)(e - s), 0, 0,
+                                  pend[s].hdr->area_d != 0};
             if (generic) { st.hdr = *pend[s].hdr; st.plane = pend[s].plane; }
             for (size_t j = s; j < e; j++) {
                 st.g.ctas = std::max(st.g.ctas, pend[j].l.ctas_per_job);

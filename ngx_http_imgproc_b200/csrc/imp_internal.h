@@ -173,6 +173,7 @@ struct ImpLaunchGroup {
     int first, count;            // jobs [first, first+count) of the device job table
     int ctas;                    // grid.x: the largest ctas_per_job of the group
     int smem_bytes;              // the largest smem_bytes of the group
+    int area_exact;              // AREA_FRAC: the jobs' passes take exact integer taps (ImpPass::area_d != 0)
 };
 // d_jobs == nullptr: a single job passed by value (`one`), no device job table needed.
 cudaError_t imp_launch_group(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st);

@@ -1,4 +1,4 @@
-// imp_k_strip.cu — translation unit of the persistent TMA strip kernels (imp_tiles.cuh): INTER_AREA fractional / integer.
+// imp_k_strip.cu — translation unit of the persistent TMA strip kernels (imp_tiles.cuh): INTER_AREA fractional / integer, INTER_LINEAR.
 #include "imp_internal.h"
 #include "imp_tiles.cuh"
 
@@ -26,10 +26,11 @@ static cudaError_t launch_strip_sc(const ImpLaunchGroup& g, const ImpJob* d_jobs
     return cudaErrorInvalidValue;
 }
 
-// strip kernel modes (imp_tiles.cuh): 0 fractional INTER_AREA, 1 integer INTER_AREA, 3 INTER_LINEAR
+// strip kernel modes (imp_tiles.cuh): 0 fractional INTER_AREA, 1 integer INTER_AREA, 2 fractional INTER_AREA with exact
+// integer taps, 3 INTER_LINEAR
 cudaError_t imp_launch_strip(const ImpLaunchGroup& g, const ImpJob* d_jobs, const ImpJob* one, cudaStream_t st) {
     switch (g.kind) {
-        case IMP_G_AREA_FRAC: return launch_strip_sc<0>(g, d_jobs, one, st);
+        case IMP_G_AREA_FRAC: return g.area_exact ? launch_strip_sc<2>(g, d_jobs, one, st) : launch_strip_sc<0>(g, d_jobs, one, st);
         case IMP_G_AREA_INT:  return launch_strip_sc<1>(g, d_jobs, one, st);
         case IMP_G_LINEAR:    return launch_strip_sc<3>(g, d_jobs, one, st);
     }

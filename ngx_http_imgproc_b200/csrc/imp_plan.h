@@ -60,6 +60,9 @@ struct ImpOp {                // 64 bytes
 
 #define IMP_MAX_OPS 48
 
+// An INTER_AREA tap with its exact integer weight (ImpPass::area_d): source index (pixels, window-relative) and k.
+struct ImpAreaKTap { int si, k; };
+
 // One pass, as the kernels see it. Lives at offset 0 of the pass blob in device memory; every *_off
 // is a byte offset into that blob (0 = absent).
 struct ImpPass {
@@ -81,6 +84,11 @@ struct ImpPass {
     int taph_off, tapv_off;   // BLUR tile kernel: the same taps as u8 dot-product words: u32 taph[4][NWH] (dp4a, four byte
                               // alignments), u32 tapv[2][NWV] (dp2a, two parities); ImpBlurDims<R> below
     int max_xtaps, max_ytaps; // AREA_FRAC: largest tap count per output column / row
+    // AREA_FRAC with exact integer taps (imp_planner.cpp, area_exact): every weight is k/p per axis and the output is
+    // (N + area_bias) / area_d with N = sum k_y * k_x * S. area_d = p_x * p_y (odd, <= 257); 0 = float taps only.
+    int area_d, area_bias;    // D, (D - 1) / 2
+    unsigned area_magic;      // ceil(2^32 / D): (N + bias) / D == umulhi(N + bias, magic) for N + bias < 2^17
+    int ixcoef_off, iycoef_off; // ImpAreaKTap {si, k}[taps]: the xcoef / ycoef tables with the integer weights
     int tile_rs, tile_rows;   // tile kernels: shared-memory row stride (bytes) and max source rows per 32x8 tile
     int tile_smem;            // tile kernels: source-tile bytes (tile_rs*tile_rows); 0 = no tile kernel for this pass
     int xtile_off, ytile_off; // tile kernels: int2 per tile column {first px, last px}; int4 per tile row {first src row, rows, first y tap, y taps}

@@ -211,6 +211,54 @@ void area_table(int ssize, int dsize, double scale, std::vector<Range>& ranges, 
     }
 }
 
+// Exact integer taps for a fractional INTER_AREA pass (the strip kernel's integer mode, imp_tiles.cuh). With the scale
+// cw/rw = p_x/q_x in lowest terms every weight area_table makes is k/p_x for an integer k (a whole source pixel q_x, a
+// partial one 0 < k < q_x), and likewise in y, so an output pixel is exactly N/D with N = sum_j k_yj sum_i k_xi S_ij and
+// D = p_x p_y. For odd D, N/D is never a half-integer: it lies at least 1/(2D) from every rounding boundary. The float
+// path (imp_gather_area_frac: OpenCV's rounded products and sums, then cvRound) differs from N/D by rounding error alone;
+// while that error E is below 1/(2D), cvRound of the float sum is round(N/D) = (N + (D-1)/2) / D: the same bits.
+//
+// The bound, with u = 2^-24, g(n) = n u / (1 - n u), float weights a (x) and b (y), S <= 255:
+//   float vs R = sum_j b_j sum_i a_i S_ij: a row sum of n_x rounded products and n_x - 1 rounded additions is within
+//     g(n_x) of its exact value relative to sum_i a_i S_i <= 255 A; the n_y rounded products with b and n_y - 1 additions
+//     add g(n_y) relative to sum_j b_j h_j <= 255 A B (1 + g(n_x)). So |float - R| <= 255 (g(n_x) + g(n_y)) A B (1 + g(n_x)).
+//   R vs N/D: b a - (k_y/p_y)(k_x/p_x) = b (a - k_x/p_x) + (k_x/p_x)(b - k_y/p_y), so |R - N/D| <= 255 (B da + K db).
+// A and B are the largest column and row sums of a and b, K = max(A, 1) bounds the column sums of a and of k_x/p_x (the
+// latter are exactly 1: checked), and da, db the largest per-column and per-row sums of |a - k/p|. The pass qualifies when
+// E = the sum of both <= 1/(4D), a factor 2 of margin. D <= 257 keeps 255 D < 2^16, so the kernel's packed u16 channel
+// pairs cannot carry into each other, and every k <= 255 fits the byte lanes of its dp4a weight words.
+bool area_exact(int cw, int rw, int ch, int rh, const std::vector<Range>& xr, const std::vector<AreaTap>& xt, int nx,
+                const std::vector<Range>& yr, const std::vector<AreaTap>& yt, int ny, std::vector<ImpAreaKTap>& kx,
+                std::vector<ImpAreaKTap>& ky, int& D) {
+    auto gcd = [](int a, int b) { while (b) { int t = a % b; a = b; b = t; } return a; };
+    const int px = cw / gcd(cw, rw), py = ch / gcd(ch, rh);
+    D = px * py;
+    if (D <= 1 || D % 2 == 0 || D > 257) return false;
+    // integer weights per axis: the largest weight sum and the largest |a - k/p| sum over its columns (rows)
+    auto axis = [](int p, const std::vector<Range>& r, const std::vector<AreaTap>& t, std::vector<ImpAreaKTap>& k, double& amax, double& dmax) {
+        k.resize(t.size()); amax = 0; dmax = 0;
+        for (const Range& g : r) {
+            double asum = 0, dsum = 0;
+            int ksum = 0;
+            for (int i = g.first; i < g.first + g.count; i++) {
+                const long q = lrint((double)t[i].a * p);
+                if (q < 1 || q > 255 || fabs((double)t[i].a - (double)q / p) > 1e-6) return false;
+                k[i] = ImpAreaKTap{t[i].si, (int)q};
+                asum += t[i].a; dsum += fabs((double)t[i].a - (double)q / p); ksum += (int)q;
+            }
+            if (ksum != p) return false;
+            amax = std::max(amax, asum); dmax = std::max(dmax, dsum);
+        }
+        return true;
+    };
+    double A, B, da, db;
+    if (!axis(px, xr, xt, kx, A, da) || !axis(py, yr, yt, ky, B, db)) return false;
+    const double u = ldexp(1.0, -24);
+    auto g = [u](int n) { return n * u / (1 - n * u); };
+    const double E = 255 * ((g(nx) + g(ny)) * A * B * (1 + g(nx)) + B * da + std::max(A, 1.0) * db);
+    return E <= 1.0 / (4.0 * D);
+}
+
 short sat_i16(float v) { long r = lrintf(v); return (short)std::max(-32768L, std::min(32767L, r)); }
 
 // SURVEY App. A.4: offsets + 11-bit coefficients for INTER_LINEAR / INTER_CUBIC.
@@ -846,6 +894,14 @@ int imp_build_plan(const imp_gpu_request* req, const imp_gpu_config* cfg, int w,
                 P.xcoef_off = L.bb.add(xt.data(), xt.size() * sizeof(AreaTap));
                 P.yofs_off = L.bb.add(yr.data(), yr.size() * sizeof(Range));
                 P.ycoef_off = L.bb.add(yt.data(), yt.size() * sizeof(AreaTap));
+                std::vector<ImpAreaKTap> kx, ky;
+                int D = 0;
+                if (!fast && area_exact(cw, rw, ch, rh, xr, xt, P.max_xtaps, yr, yt, P.max_ytaps, kx, ky, D)) {
+                    P.area_d = D; P.area_bias = (D - 1) / 2;
+                    P.area_magic = (unsigned)(((1ull << 32) + D - 1) / D);
+                    P.ixcoef_off = L.bb.add(kx.data(), kx.size() * sizeof(ImpAreaKTap));
+                    P.iycoef_off = L.bb.add(ky.data(), ky.size() * sizeof(ImpAreaKTap));
+                }
             }
         } else {
             bool cubic = (mode == 2);

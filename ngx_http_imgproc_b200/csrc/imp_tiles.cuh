@@ -308,6 +308,114 @@ __device__ __forceinline__ void area_strip_consume(const ImpJob& job, const ImpP
     }
 }
 
+// Fractional INTER_AREA with exact integer taps (MODE 2; ImpPass::area_d, imp_planner.cpp area_exact): the ring, staged
+// y taps, row descriptors, epilogue and store map of MODE 0 with integer sums in place of the float tap loop. The planner
+// admits a pass only where round((sum k_y sum k_x S) / D) provably equals the float path's cvRound, so the bits are the
+// same. 4 channels: a pixel splits into its {B,R} and {G,A} u16 pairs (2 PRMT), each pair takes one IMAD by the tap's
+// k_x and each row sum one IMAD by k_y; a lane never exceeds 255 D < 2^16, so the pairs cannot carry into each other.
+// 1 / 3 channels: dp4a of each loaded word with a weight word per channel that holds k_x at that channel's byte positions.
+// Zero-weight padded taps (k = 0) keep the tap loop free of branches, as in the float consumer. A mode of its own so that
+// the float instantiations keep their register allocation.
+template <int SC, int NT, int FL>
+__device__ __forceinline__ void area_exact_strip_consume(const ImpJob& job, const ImpPass* __restrict__ P, const uint8_t* __restrict__ blob,
+                                                         const uint8_t* tile0, int stage_bytes, uint64_t* full, uint64_t* empty,
+                                                         const uint8_t* s_ops, int nops, int bx0, int col_off, int tiles_y, int NSTAGE) {
+    const ImpRange* __restrict__ xr = reinterpret_cast<const ImpRange*>(blob + P->xofs_off);
+    const ImpAreaKTap* __restrict__ xt = reinterpret_cast<const ImpAreaKTap*>(blob + P->ixcoef_off);
+    const int bw = P->bw, bh = P->bh, rs = P->tile_rs;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const bool in_x = bx0 + lane < bw;
+    const int bx = min(bx0 + lane, bw - 1);
+    const int2 rxv = __ldg(reinterpret_cast<const int2*>(xr + bx));
+    IMP_DBG(rxv.x >= 0 && rxv.y >= 1 && rxv.y <= NT, 14);
+    constexpr int NW = (NT * SC + 3) / 4;                  // words of one row's taps (1 / 3 channels)
+    constexpr int NA = SC == 4 ? 2 : SC;                   // accumulators: two u16 pairs, or one per channel
+    unsigned kx[NT];                                       // 4 channels: k_x per tap
+    unsigned wk[SC][NW];                                   // 1 / 3 channels: k_x at the byte positions of channel c
+#pragma unroll
+    for (int k = 0; k < NT; k++) kx[k] = (k < rxv.y) ? (unsigned)__ldg(reinterpret_cast<const int2*>(xt + rxv.x + k)).y : 0u;
+    if constexpr (SC != 4) {
+#pragma unroll
+        for (int c = 0; c < SC; c++) {
+#pragma unroll
+            for (int wi = 0; wi < NW; wi++) {
+                unsigned m = 0;
+#pragma unroll
+                for (int bpos = 0; bpos < 4; bpos++) {
+                    const int pos = wi * 4 + bpos;
+                    if (pos < NT * SC && pos % SC == c) m |= kx[pos / SC] << (8 * bpos);
+                }
+                wk[c][wi] = m;
+            }
+        }
+    }
+    const unsigned bias = (unsigned)P->area_bias, magic = P->area_magic;
+    const int my_off = col_off + __ldg(reinterpret_cast<const int*>(xt + rxv.x)) * SC;   // byte offset of my first tap in a tile row
+
+    const int box_bytes = rs * P->tile_rows;
+    const int ytap_bytes = (P->tile_ytaps * 8 + 15) & ~15;
+    const int oc = P->oc, dc = P->dc;
+    const StripStore st = strip_store_line(P->out, job.dst, job.dst_pitch, dc, bx);
+    const StripOpsRows orows = strip_ops_rows(s_ops, nops, bx);
+    int stage = 0, phase = 0;
+    const uint32_t full_a = smem_u32(full), empty_a = smem_u32(empty);
+    for (int t = 0; t < tiles_y; t++) {
+        const int by = min(t * TH + warp, bh - 1);
+        const bool in_y = t * TH + warp < bh;
+        mbar_wait_a(full_a + stage * 8, phase);
+        const uint8_t* sbase = tile0 + stage * stage_bytes;
+        // {byte offset of my first source row in the tile, taps, first tap}, as in MODE 0
+        const int4 yrow = reinterpret_cast<const int4*>(sbase + box_bytes + ytap_bytes)[by - t * TH];
+        IMP_DBG(my_off >= 0 && yrow.x >= 0 && yrow.x + (yrow.y - 1) * rs + my_off + NT * SC + (SC == 4 ? 0 : 4) <= box_bytes + (SC == 4 ? 0 : 4) && my_off + NT * SC <= rs + 4, 8);
+        IMP_DBG(yrow.z >= 0 && (yrow.z + yrow.y) * 8 <= ytap_bytes, 9);
+        const ImpAreaKTap* yt = reinterpret_cast<const ImpAreaKTap*>(sbase + box_bytes) + yrow.z;   // the row's staged y taps
+        const uint8_t* row = sbase + my_off + yrow.x;
+        unsigned acc[NA];
+#pragma unroll
+        for (int c = 0; c < NA; c++) acc[c] = 0;
+        for (int j = 0; j < yrow.y; j++, row += rs) {
+            const unsigned ky = (unsigned)yt[j].k;
+            if constexpr (SC == 4) {
+                unsigned lo = 0, hi = 0;                   // the row's {B,R} and {G,A} as u16 pairs
+#pragma unroll
+                for (int k = 0; k < NT; k++) {
+                    const uint32_t w = *reinterpret_cast<const uint32_t*>(row + k * 4);
+                    lo += __byte_perm(w, 0, 0x4240) * kx[k];
+                    hi += __byte_perm(w, 0, 0x4341) * kx[k];
+                }
+                acc[0] += lo * ky;
+                acc[1] += hi * ky;
+            } else {
+                uint32_t seg[NW];
+                load_bytes<NT * SC>(row, seg);
+#pragma unroll
+                for (int c = 0; c < SC; c++) {
+                    unsigned h = 0;
+#pragma unroll
+                    for (int wi = 0; wi < NW; wi++) h = __dp4a(seg[wi], wk[c][wi], h);
+                    acc[c] += h * ky;
+                }
+            }
+        }
+        unsigned n[SC];
+        if constexpr (SC == 4) { n[0] = acc[0] & 0xFFFF; n[2] = acc[0] >> 16; n[1] = acc[1] & 0xFFFF; n[3] = acc[1] >> 16; }
+        else {
+#pragma unroll
+            for (int c = 0; c < SC; c++) n[c] = acc[c];
+        }
+        int v[SC];
+#pragma unroll
+        for (int c = 0; c < SC; c++) {
+            IMP_DBG(n[c] <= 255u * (unsigned)P->area_d, 15);
+            v[c] = min((int)__umulhi(n[c] + bias, magic), 255);
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive_a(empty_a + stage * 8);             // this warp is done with the stage
+        if (in_x && in_y) strip_epilogue<SC, FL>(job, oc, dc, st, orows, s_ops, nops, bx, by, v);
+        if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
+    }
+}
+
 // Integer-scale consumer (INTER_AREA NxM): no tap tables at all — output row y reads source rows y*ny .. y*ny+ny-1 and
 // output column x reads source pixels x*nx .. — and the store map is hoisted (registers are plentiful here).
 // Kept separate from the fractional consumer: sharing one body cost that one 4 % (register allocation).
@@ -403,8 +511,10 @@ __device__ __forceinline__ void linear_strip_consume(const ImpJob& job, const Im
 // LIGHT: the pass has no ops or only fused tables (ImpPass::light — every plain resize): the instantiation without the general
 // op interpreter fits 56 registers, so four CTAs share an SM instead of three.
 // FL 2: compositing ops and fused tables only ("resize + watermark", cfg2 / cfg5): the interpreter without the HSV code.
+// MODE: 0 fractional INTER_AREA (float taps), 1 integer-scale INTER_AREA, 2 fractional INTER_AREA with exact integer taps,
+// 3 INTER_LINEAR. Modes 0 and 2 stage the same bytes per ring stage and run at the same occupancy.
 template <int SC, int MODE, int FL>
-__global__ void __launch_bounds__(STRIP_THREADS, (FL == 1 && MODE != 0) ? 4 : 3)      // the fractional mode keeps 12 x weights in registers: 72
+__global__ void __launch_bounds__(STRIP_THREADS, (FL == 1 && (MODE == 1 || MODE == 3)) ? 4 : 3)      // the fractional modes keep 12 x weights in registers: 72
 imp_strip_kernel(const ImpJob* __restrict__ jobs, int first, int count, const __grid_constant__ ImpJob one, const int NSTAGE) {
     extern __shared__ __align__(128) uint8_t smem[];
     const int jn = blockIdx.y + blockIdx.z * 65535;
@@ -427,8 +537,9 @@ imp_strip_kernel(const ImpJob* __restrict__ jobs, int first, int count, const __
     uint8_t* tile0 = s_ops + ((ops_bytes + 127) & ~127);              // 128-byte aligned
     const int rs = P->tile_rs;
     // stage = [pixel box][y taps of the tile][y ranges of its 8 output rows] (the last two only in fractional mode)
-    const int ytap_bytes = (MODE == 0) ? ((P->tile_ytaps * 8 + 15) & ~15) : 0;
-    const int stage_bytes = (rs * P->tile_rows + ytap_bytes + (MODE == 0 ? 128 : 0) + 127) & ~127;
+    constexpr bool FRAC = MODE == 0 || MODE == 2;
+    const int ytap_bytes = FRAC ? ((P->tile_ytaps * 8 + 15) & ~15) : 0;
+    const int stage_bytes = (rs * P->tile_rows + ytap_bytes + (FRAC ? 128 : 0) + 127) & ~127;
     const int tid = threadIdx.x;
     if (tid == 0) {
         for (int i = 0; i < NSTAGE; i++) { mbar_init(full + i, 1); mbar_init(empty + i, TH); }
@@ -448,7 +559,7 @@ imp_strip_kernel(const ImpJob* __restrict__ jobs, int first, int count, const __
         // ---- TMA producer: one elected thread, one instruction per tile ----
         if (tid == STRIP_CONSUMERS) {
             const int4* __restrict__ ytile = reinterpret_cast<const int4*>(blob + P->ytile_off);
-            const uint8_t* __restrict__ g_yt = blob + P->ycoef_off;
+            const uint8_t* __restrict__ g_yt = blob + (MODE == 2 ? P->iycoef_off : P->ycoef_off);     // 8-byte taps either way
             const uint8_t* __restrict__ g_yr = blob + P->yrow4_off;
             const uint32_t box_bytes = (uint32_t)(rs * P->tile_rows);
             int stage = 0, phase = 0;
@@ -456,7 +567,7 @@ imp_strip_kernel(const ImpJob* __restrict__ jobs, int first, int count, const __
                 const int4 yt4 = __ldg(ytile + t);                       // {first source row, rows, first y tap, y taps}
                 mbar_wait(empty + stage, phase ^ 1);
                 uint8_t* sdst = tile0 + stage * stage_bytes;
-                if (MODE == 0) {
+                if (FRAC) {
                     // the tile's y taps and row ranges ride along as two small bulk copies, so the consumers' inner
                     // loops never leave shared memory
                     const int tapbase = yt4.z & ~1;
@@ -493,6 +604,21 @@ imp_strip_kernel(const ImpJob* __restrict__ jobs, int first, int count, const __
         case 10: area_strip_consume<SC, 10, 0, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
         case 11: area_strip_consume<SC, 11, 0, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
         default: area_strip_consume<SC, 12, 0, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        }
+    } else if constexpr (MODE == 2) {
+        switch (P->max_xtaps) {                                       // uniform over the pass
+        case 1: area_exact_strip_consume<SC, 1, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 2: area_exact_strip_consume<SC, 2, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 3: area_exact_strip_consume<SC, 3, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 4: area_exact_strip_consume<SC, 4, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 5: area_exact_strip_consume<SC, 5, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 6: area_exact_strip_consume<SC, 6, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 7: area_exact_strip_consume<SC, 7, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 8: area_exact_strip_consume<SC, 8, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 9: area_exact_strip_consume<SC, 9, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 10: area_exact_strip_consume<SC, 10, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        case 11: area_exact_strip_consume<SC, 11, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
+        default: area_exact_strip_consume<SC, 12, FL>(job, P, blob, tile0, stage_bytes, full, empty, s_ops, nops, bx0, col_off, tiles_y, NSTAGE); break;
         }
     } else {
         switch (P->nx) {
